@@ -2,7 +2,7 @@
 """Headline benchmark: equivalent-resistance solve of a 16M-node resistor grid (config C5a).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--grid 4096]
-                    [--precond amg|jacobi]
+                    [--precond amg|jacobi] [--dump-outputs DIR]
 
 One "step" is one pass of the hot path over the workload: (N > 1: select the rank's components
 on the device ->) stamp the component table -> build the CSR -> AMG-preconditioned CG (default;
@@ -16,6 +16,15 @@ runs on every GPU count (rows partitioned over the ranks).
   cpu_baseline : the unmodified reference (baseline/_ref; oracle port if absent) on a bounded
           sample of the same workload; same_size_pair: that sample through this repo as well
 Prints ONE JSON line on rank 0.
+
+--dump-outputs DIR writes, after the timed steps, what the last timed step computed as float64 .npy files,
+so that two builds can be compared output for output (the workload is deterministic for given arguments):
+  R                       e(1) - e(g) of the value leg
+  potentials_sample       the solved node potentials at a fixed, seeded sample of 2^20 rows (all rows of
+                          a smaller system): the whole vector of the 4096 grid would be 134 MB
+  potentials_sample_rows  the row index of each sampled potential
+  R_e2e                   R of the e2e leg (public API)
+--impl reference writes R only.
 """
 import argparse
 import json
@@ -45,6 +54,33 @@ def ncu_traffic(kernel, N):
 
 
 KNIGHT_LIMIT = 4 / np.pi - 0.5       # infinite-grid knight's-move resistance
+DUMP_ROWS = 1 << 20                  # potentials written by --dump-outputs: 8 MB, plus 8 MB of row indices
+
+
+def sample_rows(n):
+    """The sorted rows of the solution that --dump-outputs writes: a fixed, seeded sample."""
+    if n <= DUMP_ROWS:
+        return np.arange(n, dtype=np.int64)
+    return np.sort(np.random.default_rng(0).choice(n, DUMP_ROWS, replace=False))
+
+
+def gather_rows(x_local, row0, rows, world):
+    """x[rows] of a solution of which this rank holds rows row0 .. row0 + len(x_local), on every rank."""
+    import torch
+    idx = torch.from_numpy(rows).to(x_local.device)
+    mine = (idx >= row0) & (idx < row0 + x_local.numel())
+    out = torch.zeros(len(rows), dtype=torch.float64, device=x_local.device)
+    out[mine] = x_local[idx[mine] - row0]
+    if world > 1:
+        import torch.distributed as dist
+        dist.all_reduce(out)                 # each row has one owner; the other ranks add exact zeros
+    return out.cpu().numpy()
+
+
+def write_outputs(directory, arrays):
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, f"{name}.npy"), np.asarray(a, dtype=np.float64))
 
 
 # --------------------------------------------------------------------------- reference arm
@@ -161,6 +197,8 @@ def run_reference(args):
         "e2e": {"value": value, "unit": "unknowns/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
         "host_cpus": os.cpu_count(), "R": r,
     }
+    if args.dump_outputs:
+        write_outputs(args.dump_outputs, {"R": [r]})
     print(json.dumps(line), flush=True)
 
 
@@ -261,12 +299,14 @@ def run_ours(args):
     torch.cuda.synchronize()
 
     def step_device():
+        """(R, info, the rank's rows of the solution)"""
         if runner is not None:
-            return runner.step(dtab)
+            r, info = runner.step(dtab)
+            return r, info, runner.x_local
         csr, rhs = dev.assemble_csr(table, dtab=dtab)
         x, info = dev.pcg(csr, rhs, rtol=RTOL)
         info["nnz"] = csr.nnz
-        return float(x[row_1]), info                          # e(1) - e(g), ground is 0 V
+        return float(x[row_1]), info, x                       # e(1) - e(g), ground is 0 V
 
     def barrier():
         if world > 1:
@@ -274,7 +314,7 @@ def run_ours(args):
         torch.cuda.synchronize()
 
     for _ in range(args.warmup):
-        r, info = step_device()
+        r, info, x_local = step_device()
     barrier()
     sampler = ClockSampler(local) if rank == 0 else None
     launches0 = lib.nodal_launch_count()
@@ -282,7 +322,7 @@ def run_ours(args):
     ev0.record()
     iters, infos = [], []
     for _ in range(args.steps):
-        r, info = step_device()
+        r, info, x_local = step_device()
         iters.append(info["iterations"])
         infos.append(info)
     ev1.record()
@@ -290,6 +330,11 @@ def run_ours(args):
     ms = ev0.elapsed_time(ev1)
     launches = lib.nodal_launch_count() - launches0
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs:
+        rows = sample_rows(n_unknowns)
+        row0 = int(runner.bounds[rank]) if runner is not None else 0
+        dump = {"R": [r], "potentials_sample": gather_rows(x_local, row0, rows, world),
+                "potentials_sample_rows": rows}
     if world > 1:
         t = torch.tensor([ms], device="cuda", dtype=torch.float64)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -341,6 +386,9 @@ def run_ours(args):
         if world > 1:
             dist.destroy_process_group()
         return
+    if args.dump_outputs:
+        dump["R_e2e"] = [r_e2e]
+        write_outputs(args.dump_outputs, dump)
 
     # ---- roofline of the dominant kernel, per-launch time from CUDA events (rank 0, one GPU's share)
     peak, peak_src = load_peaks()
@@ -467,7 +515,11 @@ def main():
     ap.add_argument("--gather-below", type=int, default=0,
                     help="AMG: levels with at most this many rows are replicated on every rank (0 = library default)")
     ap.add_argument("--no-side", action="store_true", help="skip the side measurement of the other preconditioner")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed to DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
     else:
