@@ -198,6 +198,45 @@ int nodal_connected_components(nodal_ctx* ctx, int64_t ncomp, const int32_t* a, 
                                int32_t kcl, int32_t* labels, int32_t* ncomponents_h,
                                int32_t* reached_h, void* stream);
 
+/* ---------------------------------------------------------------- voltage-source elimination
+ * csrc/sources.cu.  For an R / A / E table whose E rows form a forest (no loop of sources, every
+ * branch owned by exactly one E row), the MNA system the reference hands to spsolve
+ * (nodal/nodal.py:325) is reduced to an R / A table over one unknown per tree of sources (an SPD
+ * weighted Laplacian), solved with the SPD solvers, and expanded back.  Nodes are 0..kcl-1 plus
+ * ground = node kcl.
+ *
+ * nodal_source_forest: erow (be) receives the table rows of the E sources in table order;
+ * adj_ptr (kcl + 2) / adj_row (2 be) every node's incident sources ordered by the other node;
+ * per node (kcl + 1): rep_row (reduced row of its tree, NODAL_GROUND for ground's tree), offset
+ * (potential relative to the tree's root), parent_edge (table row of the source to its parent, -1
+ * at a root), depth; roots (kcl) the root node of each reduced row.  info_h (host, 8): [0] E rows,
+ * [1] loops of the source graph, [2] branches not owned by exactly one E row, [3] trees, [4] trees
+ * without ground, [5] nodes in ground's tree, [6] reduced rows, [7] depth of the forest.  When
+ * [1] or [2] is non-zero the per-node outputs are not written. */
+int nodal_source_forest(nodal_ctx* ctx, int64_t ncomp, const uint8_t* type, const double* value,
+                        const int32_t* a, const int32_t* b, const int32_t* branch, int32_t kcl, int32_t be,
+                        int32_t* erow, int32_t* adj_ptr, int32_t* adj_row, int32_t* rep_row, double* offset,
+                        int32_t* parent_edge, int32_t* depth, int32_t* roots, int64_t* info_h, void* stream);
+/* The reduced table (kcl = reduced rows, be = 0) in component order: pos (ncomp) receives each
+ * component's first output row, *count_h the number of rows; then nodal_source_reduce_table writes
+ * them (csrc/sources_core.cuh src_reduce_component gives the rule). */
+int nodal_source_reduce_scan(nodal_ctx* ctx, int64_t ncomp, const uint8_t* type, const int32_t* a,
+                             const int32_t* b, int32_t kcl, const int32_t* rep_row, const double* offset,
+                             uint32_t* pos, int64_t* count_h, void* stream);
+int nodal_source_reduce_table(nodal_ctx* ctx, int64_t ncomp, const uint8_t* type, const double* value,
+                              const int32_t* a, const int32_t* b, int32_t kcl, const int32_t* rep_row,
+                              const double* offset, const uint32_t* pos, uint8_t* out_type, double* out_value,
+                              int32_t* out_a, int32_t* out_b, void* stream);
+/* x (n) = potentials from the reduced solution y, then the source currents from the KCL residual
+ * rhs - G [e; 0] of the full MNA system (indptr / indices / data, n rows) summed over the subtree each
+ * source cuts off, deepest level first.  *relres_h = ||rhs - G x|| / ||rhs||. */
+int nodal_source_expand(nodal_ctx* ctx, int32_t kcl, int32_t n, int32_t nsrc, const int32_t* erow,
+                        const int32_t* a, const int32_t* b, const int32_t* branch, const int32_t* adj_ptr,
+                        const int32_t* adj_row, const int32_t* rep_row, const double* offset,
+                        const int32_t* depth, int32_t max_depth, const double* y, const double* rhs,
+                        int64_t nnz, const int32_t* indptr, const int32_t* indices, const double* data,
+                        double* x, double* relres_h, void* stream);
+
 /* ---------------------------------------------------------------- dense kernels
  * Blocked FP64 LU with partial pivoting + triangular solves.  Replaces
  * numpy.linalg.solve (LAPACK dgesv) at nodal/nodal.py:327.  G (n x n row-major)

@@ -50,6 +50,13 @@ SIGNATURES = {
                                 C.POINTER(_f64), _vp]),
     "nodal_connected_components": (C.c_int, [_vp, _i64, _vp, _vp, _i32, _vp, C.POINTER(_i32),
                                              C.POINTER(_i32), _vp]),
+    "nodal_source_forest": (C.c_int, [_vp, _i64, _vp, _vp, _vp, _vp, _vp, _i32, _i32] + [_vp] * 8
+                            + [C.POINTER(_i64), _vp]),
+    "nodal_source_reduce_scan": (C.c_int, [_vp, _i64, _vp, _vp, _vp, _i32, _vp, _vp, _vp, C.POINTER(_i64), _vp]),
+    "nodal_source_reduce_table": (C.c_int, [_vp, _i64, _vp, _vp, _vp, _vp, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp,
+                                            _vp]),
+    "nodal_source_expand": (C.c_int, [_vp, _i32, _i32, _i32] + [_vp] * 9 + [_i32, _vp, _vp, _i64, _vp, _vp, _vp, _vp,
+                                                                             C.POINTER(_f64), _vp]),
     "nodal_lu_solve": (C.c_int, [_vp, _i32, _vp, _vp, _vp, C.POINTER(_i32), _vp]),
     "nodal_dgemm_sub_profile": (C.c_int, [_vp, _vp, _vp, _vp, _i32, _i32, _i32, _i32, _i32, C.POINTER(_f64), _vp]),
     "nodal_lu_batched": (C.c_int, [_vp, _i64, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp,

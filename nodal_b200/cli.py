@@ -19,6 +19,9 @@ def make_parser(description, file_help):
     parser.add_argument("--check-connected", action="store_true",
                         help="with -s: fail on floating sub-circuits instead of printing what the "
                              "iterative solver returned")
+    parser.add_argument("--eliminate-sources", choices=("auto", "on", "off"), default="auto",
+                        help="with -s: solve R / A / E netlists by eliminating the voltage sources and running "
+                             "the AMG-PCG on the reduced system (auto: above the dense-LU fallback size)")
     return parser
 
 
@@ -29,6 +32,9 @@ def circuit_options(options):
         kw["precond"] = options.precond
     if options.sparse and options.check_connected:
         kw["check_connected"] = True
+    mode = getattr(options, "eliminate_sources", "auto")
+    if options.sparse and mode != "auto":
+        kw["eliminate_sources"] = mode == "on"
     return kw
 
 

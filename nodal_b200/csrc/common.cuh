@@ -158,4 +158,6 @@ size_t scan_scratch_bytes(int64_t count);
 int radix_sort_pairs(nodal_ctx* ctx, u64* keys, u64* vals, u64* keys_alt, u64* vals_alt,
                      int64_t count, int bits, bool* result_in_alt, cudaStream_t st);
 size_t radix_sort_scratch_bytes(int64_t count);
-int radix_sort_check(nodal_ctx* ctx);   // after a stream sync: NODAL_CUDA_ERROR if a sort pass gave up
+int radix_sort_check(nodal_ctx* ctx);
+int cc_union_find(nodal_ctx* ctx, int64_t nedges, const int32_t* rows, const int32_t* a, const int32_t* b,
+                  int32_t kcl, int32_t* parent, int32_t* labels, cudaStream_t st);   // csrc/graph.cu   // after a stream sync: NODAL_CUDA_ERROR if a sort pass gave up

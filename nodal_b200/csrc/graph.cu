@@ -34,10 +34,11 @@ cc_init_kernel(int32_t nodes, int32_t* __restrict__ parent) {
 }
 
 __global__ void __launch_bounds__(GT)
-cc_hook_kernel(int64_t ncomp, const int32_t* __restrict__ a, const int32_t* __restrict__ b,
-               int32_t kcl, int32_t* parent) {
-    for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < ncomp;
-         e += (int64_t)gridDim.x * blockDim.x) {
+cc_hook_kernel(int64_t ncomp, const int32_t* __restrict__ rows, const int32_t* __restrict__ a,
+               const int32_t* __restrict__ b, int32_t kcl, int32_t* parent) {
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < ncomp;
+         i += (int64_t)gridDim.x * blockDim.x) {
+        const int64_t e = rows ? rows[i] : i;
         int32_t u = a[e], v = b[e];
         if (u < 0) u = kcl;              // ground lead
         if (v < 0) v = kcl;
@@ -85,6 +86,28 @@ cc_count_kernel(int32_t nodes, const int32_t* __restrict__ labels, int32_t* __re
     }
 }
 
+static int cc_grid(nodal_ctx* ctx, int64_t work) {
+    int64_t g = (work + GT - 1) / GT;
+    const int64_t cap = (int64_t)ctx->num_sms * 16;
+    return (int)(g < 1 ? 1 : g < cap ? g : cap);
+}
+
+// labels[v] = smallest node of v's component over the edges a[e] - b[e], e = rows[i] for i < nedges
+// (rows == nullptr: e = i).  `parent` is scratch of kcl + 1 entries.  Shared with csrc/sources.cu.
+int cc_union_find(nodal_ctx* ctx, int64_t nedges, const int32_t* rows, const int32_t* a, const int32_t* b,
+                  int32_t kcl, int32_t* parent, int32_t* labels, cudaStream_t st) {
+    const int32_t nodes = kcl + 1;
+    cc_init_kernel<<<cc_grid(ctx, nodes), GT, 0, st>>>(nodes, parent);
+    KERNEL_CHECK();
+    if (nedges > 0) {
+        cc_hook_kernel<<<cc_grid(ctx, nedges), GT, 0, st>>>(nedges, rows, a, b, kcl, parent);
+        KERNEL_CHECK();
+    }
+    cc_label_kernel<<<cc_grid(ctx, nodes), GT, 0, st>>>(nodes, parent, labels);
+    KERNEL_CHECK();
+    return NODAL_OK;
+}
+
 extern "C" int nodal_connected_components(nodal_ctx* ctx, int64_t ncomp, const int32_t* a,
                                           const int32_t* b, int32_t kcl, int32_t* labels,
                                           int32_t* ncomponents_h, int32_t* reached_h, void* stream) {
@@ -109,22 +132,10 @@ extern "C" int nodal_connected_components(nodal_ctx* ctx, int64_t ncomp, const i
         nodal_set_error("nodal_connected_components: out of device memory");
         return NODAL_CUDA_ERROR;
     }
-    auto grid = [&](int64_t work) {
-        int64_t g = (work + GT - 1) / GT;
-        const int64_t cap = (int64_t)ctx->num_sms * 16;
-        return (int)(g < 1 ? 1 : g < cap ? g : cap);
-    };
     auto run = [&]() -> int {
         CUDA_TRY(cudaMemsetAsync(counts, 0, 2 * sizeof(int32_t), st));
-        cc_init_kernel<<<grid(nodes), GT, 0, st>>>(nodes, parent);
-        KERNEL_CHECK();
-        if (ncomp > 0) {
-            cc_hook_kernel<<<grid(ncomp), GT, 0, st>>>(ncomp, a, b, kcl, parent);
-            KERNEL_CHECK();
-        }
-        cc_label_kernel<<<grid(nodes), GT, 0, st>>>(nodes, parent, labels);
-        KERNEL_CHECK();
-        cc_count_kernel<<<grid(nodes), GT, 0, st>>>(nodes, labels, counts);
+        NODAL_TRY(cc_union_find(ctx, ncomp, nullptr, a, b, kcl, parent, labels, st));
+        cc_count_kernel<<<cc_grid(ctx, nodes), GT, 0, st>>>(nodes, labels, counts);
         KERNEL_CHECK();
         int32_t* host = reinterpret_cast<int32_t*>(ctx->pinned);
         CUDA_TRY(cudaMemcpyAsync(host, counts, 2 * sizeof(int32_t), cudaMemcpyDeviceToHost, st));

@@ -367,6 +367,60 @@ class Device:
         _lib.check(st, "nodal_connected_components")
         return count.value, reached.value, labels
 
+    # ------------------------------------------------------------ voltage-source elimination
+    def source_forest(self, dtab, ncomp, kcl, be):
+        """Forest of the E rows of a device-resident R / A / E table (csrc/sources.cu).  Returns
+        (info dict, dict of device tensors); the tensors are only written when info["loops"] and
+        info["branch_conflicts"] are 0."""
+        torch = self.torch
+        i32 = lambda k: self.empty(max(1, k), torch.int32)             # noqa: E731
+        nodes = kcl + 1
+        out = dict(erow=i32(be), adj_ptr=i32(nodes + 1), adj_row=i32(2 * be), rep_row=i32(nodes),
+                   offset=self.empty(nodes, torch.float64), parent_edge=i32(nodes), depth=i32(nodes),
+                   roots=i32(kcl))
+        info = (C.c_int64 * 8)()
+        p = self.ptr
+        _lib.check(self.lib.nodal_source_forest(
+            self.ctx, ncomp, p(dtab["type"]), p(dtab["value"]), p(dtab["a"]), p(dtab["b"]), p(dtab["branch"]),
+            kcl, be, *[p(out[k]) for k in ("erow", "adj_ptr", "adj_row", "rep_row", "offset", "parent_edge",
+                                           "depth", "roots")], info, self.stream()), "nodal_source_forest")
+        keys = ("sources", "loops", "branch_conflicts", "trees", "floating_trees", "grounded_nodes", "rows", "depth")
+        return {k: int(info[i]) for i, k in enumerate(keys)}, out
+
+    def source_reduce(self, dtab, ncomp, kcl, forest):
+        """The reduced R / A table as device columns (`dtab` form) and its number of rows."""
+        torch = self.torch
+        pos = self.empty(max(1, ncomp), torch.int32)
+        count = C.c_int64(0)
+        p = self.ptr
+        args = (p(dtab["type"]), p(dtab["a"]), p(dtab["b"]), kcl, p(forest["rep_row"]), p(forest["offset"]))
+        _lib.check(self.lib.nodal_source_reduce_scan(self.ctx, ncomp, *args, p(pos), C.byref(count), self.stream()),
+                   "nodal_source_reduce_scan")
+        m = count.value
+        red = dict(type=self.empty(max(1, m), torch.uint8), value=self.empty(max(1, m), torch.float64),
+                   a=self.empty(max(1, m), torch.int32), b=self.empty(max(1, m), torch.int32),
+                   c=None, d=None, drv=None, branch=None)
+        _lib.check(self.lib.nodal_source_reduce_table(
+            self.ctx, ncomp, p(dtab["type"]), p(dtab["value"]), p(dtab["a"]), p(dtab["b"]), kcl,
+            p(forest["rep_row"]), p(forest["offset"]), p(pos), p(red["type"]), p(red["value"]), p(red["a"]),
+            p(red["b"]), self.stream()), "nodal_source_reduce_table")
+        return red, m
+
+    def source_expand(self, dtab, kcl, forest, info, y, csr: DeviceCSR, rhs):
+        """x = [potentials; source currents] of the full system from the reduced solution y, and
+        ||rhs - G x|| / ||rhs|| with the full MNA matrix `csr`."""
+        n = csr.n
+        x = self.empty(max(1, n), self.torch.float64)[:n]
+        relres = C.c_double(0.0)
+        p = self.ptr
+        f = forest
+        _lib.check(self.lib.nodal_source_expand(
+            self.ctx, kcl, n, info["sources"], p(f["erow"]), p(dtab["a"]), p(dtab["b"]), p(dtab["branch"]),
+            p(f["adj_ptr"]), p(f["adj_row"]), p(f["rep_row"]), p(f["offset"]), p(f["depth"]), info["depth"],
+            p(y), p(rhs), csr.nnz, p(csr.indptr), p(csr.indices), p(csr.data), p(x), C.byref(relres),
+            self.stream()), "nodal_source_expand")
+        return x, relres.value
+
     def amg(self, csr: DeviceCSR, **params):
         """Aggregation-AMG hierarchy for an SPD DeviceCSR (csrc/amg.cu); see DeviceAMG."""
         return DeviceAMG(self, csr, **params)

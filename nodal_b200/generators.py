@@ -196,6 +196,81 @@ def lattice3d(N, resistance=1.0):
     return _lattice((N, N, N), (h, h, h), (h + 2, h + 1, h), resistance)
 
 
+# --------------------------------------------------------------------------- power-delivery grid
+def power_grid(N, pitch, vdd=1.0, load=1e-4, seed=0, resistance=1.0):
+    """Resistive N x N mesh held by supply pads (IR-drop analysis): the resistors of grid2d's loop
+    order between nodes "n{x}_{y}", then one E source "v{k}" of `vdd` from every node with x and y
+    multiples of `pitch` to ground "g" (row-major), then a load "l{k}" on every node (row-major):
+    an A row from "g" to the node drawing a current uniform in [0, load) (seed).  Numbering,
+    anomnum and branch are those of the csv path (first appearance; branch k = pad k)."""
+    N, pitch = int(N), int(pitch)
+    if N < 2 or pitch < 1:
+        raise ValueError("power_grid needs N >= 2 and pitch >= 1")
+    rng = np.random.default_rng(seed)
+    sites = N * N
+    sid = np.arange(sites, dtype=np.int64)
+    x, y = sid // N, sid % N
+    has = np.stack([x + 1 < N, y + 1 < N], axis=1)
+    nb = np.stack([sid + N, sid + 1], axis=1)
+    ra = np.repeat(sid, 2).reshape(sites, 2)[has]
+    rb = nb[has]
+    gid = sites
+    pads = sid[(x % pitch == 0) & (y % pitch == 0)]
+    P = len(pads)
+    a_id = np.concatenate([ra, pads, np.full(sites, gid)])
+    b_id = np.concatenate([rb, np.full(P, gid), sid])
+    index, kcl = first_appearance_numbering(a_id, b_id, gid)
+    m_r = len(ra)
+    type_ = np.concatenate([np.full(m_r, K.T_R, np.uint8), np.full(P, K.T_E, np.uint8), np.full(sites, K.T_A, np.uint8)])
+    value = np.concatenate([np.full(m_r, float(resistance)), np.full(P, float(vdd)), rng.uniform(0.0, load, sites)])
+    branch = np.full(len(type_), -1, np.int32)
+    branch[m_r:m_r + P] = np.arange(P, dtype=np.int32)
+    table = ComponentTable(type_, value, index[a_id], index[b_id], branch=branch, kcl=kcl, be=P)
+
+    def encode(name):
+        if name == "g":
+            return gid
+        if not name.startswith("n"):
+            return None
+        try:
+            px, py = (int(t) for t in name[1:].split("_"))
+        except ValueError:
+            return None
+        return px * N + py if 0 <= px < N and 0 <= py < N else None
+
+    def decode(nid):
+        return "g" if nid == gid else f"n{nid // N}_{nid % N}"
+
+    def names(k):
+        k = int(k)
+        return f"r{k}" if k < m_r else f"v{k - m_r}" if k < m_r + P else f"l{k - m_r - P}"
+
+    net = TableNetlist(table, _LazyNodeMap(index, encode, decode, kcl), "g", names=names,
+                       anomnum=_PadNames(P))
+    net._currents = [f"v{k}" for k in range(P)]
+    return net
+
+
+class _PadNames(Mapping):
+    """anomnum of power_grid: "v{k}" -> k without materialising the names."""
+
+    def __init__(self, count):
+        self._count = count
+
+    def __getitem__(self, name):
+        if isinstance(name, str) and name.startswith("v") and name[1:].isdigit():
+            k = int(name[1:])
+            if k < self._count and name == f"v{k}":
+                return k
+        raise KeyError(name)
+
+    def __len__(self):
+        return self._count
+
+    def __iter__(self):
+        return (f"v{k}" for k in range(self._count))
+
+
 # --------------------------------------------------------------------------- sparse random networks
 def random_network(nodes, degree=8, seed=0, decades=2.0, locality=None):
     """Connected random resistive network (north star: "random-network netlists"): `nodes` nodes, a

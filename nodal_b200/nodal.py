@@ -24,6 +24,7 @@ import numpy as np
 
 from . import constants as c
 from . import models
+from . import sources
 from .table import ComponentTable
 
 logging.basicConfig(level=logging.ERROR)  # as the reference does at import (nodal.py:27)
@@ -250,7 +251,9 @@ class Circuit:
 
     ``sparse=False``: dense G, blocked FP64 LU with partial pivoting (replaces
     numpy.linalg.solve).  ``sparse=True``: CSR G, Jacobi-PCG for R/A-only
-    netlists, restarted GMRES otherwise (replaces scipy spsolve).
+    netlists, restarted GMRES otherwise (replaces scipy spsolve); R/A/E netlists
+    whose voltage sources form a forest are solved through the elimination of
+    the sources (``eliminate_sources``, see sources.py).
 
     Attributes as in the reference: netlist, sparse, G, A, currents.  G and A
     live in HBM; ``G`` is a torch tensor (dense) or a DeviceCSR, and
@@ -276,13 +279,19 @@ class Circuit:
         dev = Device.get(self.options.get("device"))
         self._dev = dev
         self._dist = None
+        self._dtab = None
         if self.options.get("distributed"):
             G, A = self._build_distributed(dev, table)
         elif self.sparse:
             # csr_order="first_touch": G's columns in the order the reference's G.tocsr() has before its
             # solve (nodal.py:396-397); the solve then works on the sorted form, as spsolve sorts in place
             order = self.options.get("csr_order", "sorted")
-            G, A = dev.assemble_csr(table, order=order)
+            # tables the source elimination will take keep their device columns for it (sources.py)
+            self._eliminate = sources.check_option(self.options, table)
+            limit = int(self.options.get("dense_fallback_max_rows", 32768))
+            if sources.skip_reason(table, self._eliminate, limit) == "":
+                self._dtab = dev.upload_table(table)
+            G, A = dev.assemble_csr(table, dtab=self._dtab, order=order)
             if order != "sorted":
                 self._G_sorted = dev.assemble_csr(table)[0]
         else:
@@ -360,39 +369,8 @@ class Circuit:
             if first:
                 info["fallback_from_amg"] = first
             return x, info
-        if kind == "amg" and amg is None and warm is None and self.options.get("precond", "auto") == "auto":
-            # "auto": which preconditioner pays depends on the graph, not on its size -- on a 4 M-node
-            # expander-like random network Jacobi-PCG needs 98 iterations (43 ms) and the AMG hierarchy
-            # 265 ms; on a banded random network of the same size it is 4 616 iterations (1.9 s)
-            # against 68 (156 ms); grids are the second kind.  A short Jacobi-PCG probe tells them
-            # apart: if 24 iterations gained two digits it will finish in ~100, otherwise its iterate
-            # is the initial guess of the AMG solve.
-            probe_its = int(self.options.get("auto_probe_iterations", 24))
-            if self.G.n >= self.options.get("auto_probe_min_rows", 50_000) and probe_its > 0:
-                x0, info0 = dev.pcg(self.G, rhs, rtol=rtol, maxit=probe_its, flags=self.options.get("pcg_flags", 0))
-                if info0["status"] == 0:
-                    info0["auto"] = "jacobi (converged inside the probe)"
-                    return x0, info0
-                if info0["status"] == 2 and info0["relres"] <= 1e-2:
-                    x, info = dev.pcg(self.G, rhs, rtol=rtol, maxit=self.options.get("maxit"), x0=x0,
-                                      flags=self.options.get("pcg_flags", 0))
-                    info["iterations"] += info0["iterations"]
-                    info["auto"] = f"jacobi (probe relres {info0['relres']:.1e})"
-                    if info["status"] == 0:
-                        return x, info
-                    x0 = x
-                elif info0["status"] != 2 or not np.isfinite(info0["relres"]):
-                    x0 = None                                  # breakdown in the probe: start AMG from zero
-                x, info = self._amg_solve(rhs, None, rtol, x0)
-                if x0 is not None:
-                    info["auto"] = f"amg (probe relres {info0['relres']:.1e})"
-                    info["iterations_probe"] = info0["iterations"]
-                return x, info
-        if kind == "amg":
-            return self._amg_solve(rhs, amg, rtol, warm)
-        if kind == "pcg":
-            return dev.pcg(self.G, rhs, rtol=rtol, maxit=self.options.get("maxit"),
-                           flags=self.options.get("pcg_flags", 0), x0=warm)
+        if kind in ("amg", "pcg"):
+            return self._spd_solve(self.G, rhs, kind, rtol, warm, amg)
         x, info = dev.gmres(self.G, rhs, rtol=self.options.get("rtol", 1e-12),
                             restart=self.options.get("restart", 60),
                             maxit=self.options.get("maxit") or 20000)
@@ -414,6 +392,43 @@ class Circuit:
                             f"{limit} rows (dense fallback limit)")
         return x, info
 
+    def _spd_solve(self, G, rhs, kind, rtol, warm, amg=None):
+        """x, info for an SPD DeviceCSR G (R / A netlists, or the reduced system of csrc/sources.cu) on
+        one GPU: "amg" (with the "auto" Jacobi probe and the Jacobi-PCG retry) or "pcg"."""
+        dev = self._dev
+        if kind == "amg" and amg is None and warm is None and self.options.get("precond", "auto") == "auto":
+            # "auto": which preconditioner pays depends on the graph, not on its size -- on a 4 M-node
+            # expander-like random network Jacobi-PCG needs 98 iterations (43 ms) and the AMG hierarchy
+            # 265 ms; on a banded random network of the same size it is 4 616 iterations (1.9 s)
+            # against 68 (156 ms); grids are the second kind.  A short Jacobi-PCG probe tells them
+            # apart: if 24 iterations gained two digits it will finish in ~100, otherwise its iterate
+            # is the initial guess of the AMG solve.
+            probe_its = int(self.options.get("auto_probe_iterations", 24))
+            if G.n >= self.options.get("auto_probe_min_rows", 50_000) and probe_its > 0:
+                x0, info0 = dev.pcg(G, rhs, rtol=rtol, maxit=probe_its, flags=self.options.get("pcg_flags", 0))
+                if info0["status"] == 0:
+                    info0["auto"] = "jacobi (converged inside the probe)"
+                    return x0, info0
+                if info0["status"] == 2 and info0["relres"] <= 1e-2:
+                    x, info = dev.pcg(G, rhs, rtol=rtol, maxit=self.options.get("maxit"), x0=x0,
+                                      flags=self.options.get("pcg_flags", 0))
+                    info["iterations"] += info0["iterations"]
+                    info["auto"] = f"jacobi (probe relres {info0['relres']:.1e})"
+                    if info["status"] == 0:
+                        return x, info
+                    x0 = x
+                elif info0["status"] != 2 or not np.isfinite(info0["relres"]):
+                    x0 = None                                  # breakdown in the probe: start AMG from zero
+                x, info = self._amg_solve(G, rhs, None, rtol, x0)
+                if x0 is not None:
+                    info["auto"] = f"amg (probe relres {info0['relres']:.1e})"
+                    info["iterations_probe"] = info0["iterations"]
+                return x, info
+        if kind == "amg":
+            return self._amg_solve(G, rhs, amg, rtol, warm)
+        return dev.pcg(G, rhs, rtol=rtol, maxit=self.options.get("maxit"),
+                      flags=self.options.get("pcg_flags", 0), x0=warm)
+
     def _warm_start(self):
         """Initial guess of the iterative solvers: Circuit(..., x0=array of n values) -- e.g. the
         previous solution of a parameter sweep (SURVEY.md section 5).  None: start from zero."""
@@ -425,24 +440,24 @@ class Circuit:
             raise ValueError(f"x0 must have {self.table.n} entries")
         return self._dev.to_device(arr)
 
-    def _amg_solve(self, rhs, amg, rtol, x0):
+    def _amg_solve(self, G, rhs, amg, rtol, x0):
         """AMG-preconditioned CG on one GPU; Jacobi-PCG retry unless precond="amg" was forced."""
         dev = self._dev
         from . import _lib
         try:
             if amg is not None:
                 x, info = amg.solve(rhs, rtol=rtol, maxit=self.options.get("maxit"), x0=x0)
-            elif self.G.n >= self.options.get("amg_graph_min_rows", 100_000):
+            elif G.n >= self.options.get("amg_graph_min_rows", 100_000):
                 # large systems: the graph-captured form (csrc/dist_amg.cu with one rank):
                 # one CUDA graph per iteration, no host round trip inside the iteration
                 from . import dist as ndist
-                g = self.G
+                g = G
                 bounds = np.array([0, g.n], dtype=np.int32)
                 x, info = ndist.single_solver(dev).solve_amg(
                     g.n, bounds, g.indptr, g.indices, g.data, rhs, rtol=rtol, maxit=self.options.get("maxit"),
                     x0=x0, **(self.options.get("amg") or {}))
             else:
-                x, info = dev.amg_pcg(self.G, rhs, rtol=rtol, maxit=self.options.get("maxit"), x0=x0,
+                x, info = dev.amg_pcg(G, rhs, rtol=rtol, maxit=self.options.get("maxit"), x0=x0,
                                       **(self.options.get("amg") or {}))
             if info["status"] == 0 or self.options.get("precond") == "amg":
                 return x, info
@@ -451,7 +466,7 @@ class Circuit:
             if self.options.get("precond") == "amg":
                 raise
             first = str(err)
-        x, info = dev.pcg(self.G, rhs, rtol=rtol, maxit=self.options.get("maxit"),
+        x, info = dev.pcg(G, rhs, rtol=rtol, maxit=self.options.get("maxit"),
                           flags=self.options.get("pcg_flags", 0))
         info["fallback_from_amg"] = first
         return x, info
@@ -472,7 +487,14 @@ class Circuit:
         if self.sparse and self.options.get("check_connected") and not self.is_connected():
             logging.error("Model error: unconnected circuit")
             raise UnconnectedCircuitError
-        x, info = self._device_solve(self.A)
+        # R / A / E netlists: through the elimination of the voltage sources when it applies
+        # (sources.py); otherwise `info` is the stats of why not, or None
+        x, info = sources.solve(self) if self.sparse and self._dist is None else (None, None)
+        if x is None:
+            skipped = info
+            x, info = self._device_solve(self.A)
+            if skipped is not None:
+                info["reduction"] = skipped
         if self.sparse:
             e = self._dist_gather(x) if self._dist is not None else x.cpu().numpy()
             if info["status"] != 0:
