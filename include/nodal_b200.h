@@ -306,6 +306,12 @@ int nodal_amg_pcg_multi(nodal_ctx* ctx, nodal_amg* amg, int32_t K, const double*
  * ms_out[0] q = A p with the p.q partial sums, [1] r = b - A x, [2] the damped-Jacobi sweep. */
 int nodal_amg_profile_sweeps(nodal_ctx* ctx, nodal_amg* h, int32_t reps, double* ms_out, void* stream);
 
+/* Measurement aid for benchmarks/amg_cycle.py: average per-launch time (ms, as above) of the
+ * level-0 kernels of the V-cycle, unfused and fused (needs at least two levels):
+ * ms_out[0] jacobi0, [1] residual sweep, [2] prolong, [3] damped-Jacobi sweep,
+ * [4] fused residual of the Jacobi start, [5] fused post-smoothing of the prolongated iterate. */
+int nodal_amg_profile_cycle(nodal_ctx* ctx, nodal_amg* h, int32_t reps, double* ms_out, void* stream);
+
 /* Row-partitioned assembly: a rank stamps the components that touch one of its rows [rb, re)
  * (the loop of nodal/nodal.py:357-390 restricted to them, order kept, so the rank's rows of G are
  * bit-identical to the single-GPU CSR).  _scan writes the exclusive scan of the selection flags to

@@ -72,6 +72,7 @@ SIGNATURES = {
     "nodal_amg_pcg_multi": (C.c_int, [_vp, _vp, _i32, _vp, _vp, _f64, _i32, C.POINTER(_i32), C.POINTER(_f64),
                                       C.POINTER(_i32), _vp]),
     "nodal_amg_profile_sweeps": (C.c_int, [_vp, _vp, _i32, C.POINTER(_f64), _vp]),
+    "nodal_amg_profile_cycle": (C.c_int, [_vp, _vp, _i32, C.POINTER(_f64), _vp]),
     "nodal_table_select_scan": (C.c_int, [_vp, _i64, _vp, _vp, _i32, _i32, _vp, C.POINTER(_i64), _vp]),
     "nodal_table_select_gather": (C.c_int, [_vp, _i64, _vp, _i32, _i32] + [_vp] * 16 + [_vp]),
     "nodal_dist_amg_pcg": (C.c_int, [_vp, _vp, _i32, _vp, _i64, _vp, _vp, _vp, _vp, _vp, C.POINTER(_f64), _f64,

@@ -327,16 +327,27 @@ int sell_sweep(const nodal_amg* h, const AmgLevel& V, const double* b, const dou
     return NODAL_OK;
 }
 
-// z = M b : one V(1,1) cycle from a zero initial guess
+// The fused sweeps of the cycle (amg_kernels.cuh): MODE 1 writes r = b - A x0 with x0 = omega D^-1 b,
+// MODE 2 writes y = x~ + omega D^-1 (b - A x~) with x~ = x0 + scale P xc.
+template <int MODE>
+int cycle_sweep(const nodal_amg* h, const AmgLevel& V, const double* b, const double* xc, double* y,
+                cudaStream_t st) {
+    const nodal_sell* m = V.sell;
+    amg_cycle_sweep_kernel<MODE><<<sell_grid(h->ctx, m->nslices), AT, 0, st>>>(
+        m->n, m->nslices, m->slice_w, m->cols, m->vals, m->dinv, b, h->omega, V.agg, xc, h->scale, y);
+    KERNEL_CHECK();
+    return NODAL_OK;
+}
+
+// z = M b : one V(1,1) cycle from a zero initial guess.  Neither the Jacobi start x0 nor the
+// prolongated iterate is stored: the sweeps form them where they gather (cycle_sweep).
 int cycle(const nodal_amg* h, const double* b0, double* z0, cudaStream_t st) {
     const nodal_ctx* ctx = h->ctx;
     const int last = (int)h->lv.size() - 1;
     for (int l = 0; l < last; ++l) {
         const AmgLevel& V = h->lv[l];
         const double* b = l == 0 ? b0 : V.b;
-        amg_jacobi0_kernel<<<rows_grid(ctx, V.n), AT, 0, st>>>(V.n, V.sell->dinv, b, h->omega, V.x);
-        KERNEL_CHECK();
-        NODAL_TRY(sell_sweep<1>(h, V, b, V.x, V.r, nullptr, st));
+        NODAL_TRY(cycle_sweep<1>(h, V, b, nullptr, V.r, st));
         amg_restrict_kernel<<<rows_grid(ctx, V.nc), AT, 0, st>>>(V.nc, V.pt_ptr, V.pt_idx, V.r,
                                                               h->lv[l + 1].b);
         KERNEL_CHECK();
@@ -352,11 +363,7 @@ int cycle(const nodal_amg* h, const double* b0, double* z0, cudaStream_t st) {
     for (int l = last - 1; l >= 0; --l) {
         const AmgLevel& V = h->lv[l];
         const double* b = l == 0 ? b0 : V.b;
-        double* xa = V.r;       // the residual is not needed any more
-        amg_prolong_kernel<<<rows_grid(ctx, V.n), AT, 0, st>>>(V.n, V.agg, h->lv[l + 1].x, h->scale,
-                                                             V.x, xa);
-        KERNEL_CHECK();
-        NODAL_TRY(sell_sweep<2>(h, V, b, xa, l == 0 ? z0 : V.x, nullptr, st));
+        NODAL_TRY(cycle_sweep<2>(h, V, b, h->lv[l + 1].x, l == 0 ? z0 : V.x, st));
     }
     return NODAL_OK;
 }
@@ -629,6 +636,53 @@ extern "C" int nodal_amg_profile_sweeps(nodal_ctx* ctx, nodal_amg* h, int32_t re
         float ms = 0.f;
         if (cudaEventSynchronize(e1) == cudaSuccess) cudaEventElapsedTime(&ms, e0, e1);
         ms_out[mode] = ms / reps;
+    }
+    cudaEventDestroy(e0);
+    cudaEventDestroy(e1);
+    return rc;
+}
+
+// Per-launch time of the level-0 kernels of the V-cycle, unfused and fused, for
+// benchmarks/amg_cycle.py: `reps` launches each (after two warm-up launches) on the hierarchy's own
+// level-0 operator, aggregates and work vectors, bracketed by CUDA events on `stream`.
+// ms_out: [0] jacobi0, [1] MODE 1 residual, [2] prolong, [3] MODE 2 Jacobi sweep,
+//         [4] fused residual of the Jacobi start, [5] fused post-smoothing.
+extern "C" int nodal_amg_profile_cycle(nodal_ctx* ctx, nodal_amg* h, int32_t reps, double* ms_out, void* stream) {
+    if (!ctx || !h || h->ctx != ctx || !ms_out || reps < 1 || h->lv.size() < 2) return NODAL_BAD_ARG;
+    cudaStream_t st = (cudaStream_t)stream;
+    CUDA_TRY(cudaSetDevice(ctx->device));
+    const AmgLevel& A = h->lv[0];
+    const AmgLevel& C = h->lv[1];
+    double* b = h->r;
+    CUDA_TRY(cudaMemsetAsync(b, 0, sizeof(double) * (size_t)A.n, st));
+    CUDA_TRY(cudaMemsetAsync(A.x, 0, sizeof(double) * (size_t)A.n, st));
+    CUDA_TRY(cudaMemsetAsync(C.x, 0, sizeof(double) * (size_t)C.n, st));
+    cudaEvent_t e0, e1;
+    CUDA_TRY(cudaEventCreate(&e0));
+    CUDA_TRY(cudaEventCreate(&e1));
+    int rc = NODAL_OK;
+    for (int k = 0; k < 6 && rc == NODAL_OK; ++k) {
+        for (int i = -2; i < reps && rc == NODAL_OK; ++i) {
+            if (i == 0) cudaEventRecord(e0, st);
+            switch (k) {
+                case 0:
+                    amg_jacobi0_kernel<<<rows_grid(ctx, A.n), AT, 0, st>>>(A.n, A.sell->dinv, b, h->omega, A.x);
+                    KERNEL_CHECK();
+                    break;
+                case 1: rc = sell_sweep<1>(h, A, b, A.x, A.r, nullptr, st); break;
+                case 2:
+                    amg_prolong_kernel<<<rows_grid(ctx, A.n), AT, 0, st>>>(A.n, A.agg, C.x, h->scale, A.x, A.r);
+                    KERNEL_CHECK();
+                    break;
+                case 3: rc = sell_sweep<2>(h, A, b, A.r, h->z, nullptr, st); break;
+                case 4: rc = cycle_sweep<1>(h, A, b, nullptr, A.r, st); break;
+                default: rc = cycle_sweep<2>(h, A, b, C.x, h->z, st); break;
+            }
+        }
+        cudaEventRecord(e1, st);
+        float ms = 0.f;
+        if (cudaEventSynchronize(e1) == cudaSuccess) cudaEventElapsedTime(&ms, e0, e1);
+        ms_out[k] = ms / reps;
     }
     cudaEventDestroy(e0);
     cudaEventDestroy(e1);

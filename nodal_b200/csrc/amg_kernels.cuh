@@ -129,7 +129,7 @@ amg_gemv_kernel(int32_t n, const double* __restrict__ inv, const double* __restr
 static __global__ void __launch_bounds__(AT)
 amg_jacobi0_kernel(int32_t n, const double* __restrict__ dinv, const double* __restrict__ b,
                    double omega, double* __restrict__ x) {
-    ROW_LOOP(i, n) x[i] = omega * dinv[i] * b[i];
+    ROW_LOOP(i, n) x[i] = amg_jacobi_start(omega, dinv[i], b[i]);
 }
 
 // SELL-32 sweep, one warp per slice.
@@ -155,8 +155,8 @@ amg_sell_kernel(int32_t n, int32_t nslices, const u32* __restrict__ slice_w,
         const int64_t r = s * 32 + lane;
         if (r < n) {
             if (MODE == 0) { y[r] = acc; dot = fma(x[r], acc, dot); }
-            if (MODE == 1) y[r] = b[r] - acc;
-            if (MODE == 2) y[r] = x[r] + omega * dinv[r] * (b[r] - acc);
+            if (MODE == 1) y[r] = amg_residual(b[r], acc);
+            if (MODE == 2) y[r] = amg_jacobi_update(omega, dinv[r], b[r], acc, x[r]);
         }
     }
     if (MODE == 0) {
@@ -180,7 +180,59 @@ amg_restrict_kernel(int32_t nc, const int32_t* __restrict__ pt_ptr, const int32_
 static __global__ void __launch_bounds__(AT)
 amg_prolong_kernel(int32_t n, const int32_t* __restrict__ agg, const double* __restrict__ xc,
                    double scale, const double* __restrict__ x, double* __restrict__ xa) {
-    ROW_LOOP(i, n) xa[i] = x[i] + scale * xc[agg[i]];
+    ROW_LOOP(i, n) xa[i] = amg_prolong_add(scale, xc[agg[i]], x[i]);
+}
+
+// The V-cycle's sweeps with the vector they multiply formed at every gathered column instead of
+// stored by a kernel of its own (jacobi0 before MODE 1, prolong before MODE 2); same rounding steps
+// (amg_cycle_core.cuh), so y is bit for bit what the unfused pair computes.
+//   MODE 1: y = b - A x0                          x0 = omega D^-1 b      (residual of the Jacobi start)
+//   MODE 2: y = x~ + omega D^-1 (b - A x~)        x~ = x0 + scale P xc   (post-smoothing)
+struct JacobiStartAt {
+    const double* __restrict__ dinv;
+    const double* __restrict__ b;
+    double omega;
+    __device__ __forceinline__ double operator()(int32_t c) const {
+        return amg_jacobi_start(omega, __ldg(&dinv[c]), __ldg(&b[c]));
+    }
+};
+
+struct ProlongatedAt {
+    JacobiStartAt x0;
+    const int32_t* __restrict__ agg;
+    const double* __restrict__ xc;
+    double scale;
+    __device__ __forceinline__ double operator()(int32_t c) const {
+        return amg_prolong_add(scale, __ldg(&xc[__ldg(&agg[c])]), x0(c));
+    }
+};
+
+template <int MODE>
+static __global__ void __launch_bounds__(AT, 5)
+amg_cycle_sweep_kernel(int32_t n, int32_t nslices, const u32* __restrict__ slice_w,
+                       const int32_t* __restrict__ cols, const double* __restrict__ vals,
+                       const double* __restrict__ dinv, const double* __restrict__ b, double omega,
+                       const int32_t* __restrict__ agg, const double* __restrict__ xc, double scale,
+                       double* __restrict__ y) {
+    const int lane = threadIdx.x & 31;
+    const int64_t warp = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    const int64_t nwarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
+    const JacobiStartAt x0{dinv, b, omega};
+    const ProlongatedAt xa{x0, agg, xc, scale};
+    for (int64_t s = warp; s < nslices; s += nwarps) {
+        const u32 w0 = slice_w[s];
+        const int w = (int)(slice_w[s + 1] - w0);
+        const int64_t base = (int64_t)w0 * 32 + lane;
+        const int64_t r = s * 32 + lane;
+        if (MODE == 1) {
+            const double acc = sell_row_gather(cols, vals, base, w, x0);
+            if (r < n) y[r] = amg_residual(b[r], acc);
+        }
+        if (MODE == 2) {
+            const double acc = sell_row_gather(cols, vals, base, w, xa);
+            if (r < n) y[r] = amg_jacobi_update(omega, dinv[r], b[r], acc, xa((int32_t)r));
+        }
+    }
 }
 
 // ------------------------------------------------------------------ CG vector kernels

@@ -840,18 +840,37 @@ int sweep(Solver& S, const DLevel& L, const double* b, const double* x, double* 
     return NODAL_OK;
 }
 
+// The fused sweeps of the cycle (amg_kernels.cuh), for one rank: the sweeps form x0 and the
+// prolongated iterate at every gathered column, which needs them at every column the rank's rows
+// touch -- all of them local when there are no halos.
+template <int MODE>
+int cycle_sweep(Solver& S, const DLevel& L, const double* b, const double* xc, double* y, cudaStream_t sx) {
+    const nodal_sell* m = L.sell;
+    amg_cycle_sweep_kernel<MODE><<<amg_sell_grid(S.ctx, m->nslices), AT, 0, sx>>>(
+        m->n, m->nslices, m->slice_w, m->cols, m->vals, m->dinv, b, S.omega, L.agg, xc, S.scale, y);
+    KERNEL_CHECK();
+    return NODAL_OK;
+}
+
 // u = M r : one V(1,1) cycle over the distributed levels, the replicated hierarchy below them.
 // r: [nloc] of level 0; u: the [owned | halo] vector of level 0 the CG's SpMV gathers from.
+// With several ranks x0 and the prolongated iterate are stored and their halos exchanged before
+// the sweep that gathers them; with one rank the fused sweeps form them in place.
 int cycle(Solver& S, const PcgDev* dev, const double* r0, double* u0, cudaStream_t sx) {
     nodal_ctx* ctx = S.ctx;
     const int ND = (int)S.lv.size() - 1;          // levels 0 .. ND-1 are smoothed here; lv[ND] is gathered
+    const bool fused = S.R == 1;
     for (int l = 0; l < ND; ++l) {
         DLevel& L = S.lv[l];
         const double* b = l == 0 ? r0 : L.b;
-        amg_jacobi0_kernel<<<amg_rows_grid(ctx, L.nloc), AT, 0, sx>>>(L.nloc, L.sell->dinv, b, S.omega, L.x);
-        KERNEL_CHECK();
-        NODAL_TRY(exchange(S, dev, 2 * l, L.halo, L.x_off, sx));
-        NODAL_TRY(sweep<1>(S, L, b, L.x, L.r, sx));
+        if (fused) {
+            NODAL_TRY(cycle_sweep<1>(S, L, b, nullptr, L.r, sx));
+        } else {
+            amg_jacobi0_kernel<<<amg_rows_grid(ctx, L.nloc), AT, 0, sx>>>(L.nloc, L.sell->dinv, b, S.omega, L.x);
+            KERNEL_CHECK();
+            NODAL_TRY(exchange(S, dev, 2 * l, L.halo, L.x_off, sx));
+            NODAL_TRY(sweep<1>(S, L, b, L.x, L.r, sx));
+        }
         amg_restrict_kernel<<<amg_rows_grid(ctx, L.nc), AT, 0, sx>>>(L.nc, L.pt_ptr, L.pt_idx, L.r, S.lv[l + 1].b);
         KERNEL_CHECK();
     }
@@ -889,10 +908,14 @@ int cycle(Solver& S, const PcgDev* dev, const double* r0, double* u0, cudaStream
         DLevel& L = S.lv[l];
         const double* b = l == 0 ? r0 : L.b;
         const double* xc = (l + 1 == ND) ? S.xfull + S.lv[ND].row0 : S.lv[l + 1].x;
-        amg_prolong_kernel<<<amg_rows_grid(ctx, L.nloc), AT, 0, sx>>>(L.nloc, L.agg, xc, S.scale, L.x, L.r);
-        KERNEL_CHECK();
-        NODAL_TRY(exchange(S, dev, 2 * l + 1, L.halo, L.r_off, sx));
-        NODAL_TRY(sweep<2>(S, L, b, L.r, l == 0 ? u0 : L.x, sx));
+        if (fused) {
+            NODAL_TRY(cycle_sweep<2>(S, L, b, xc, l == 0 ? u0 : L.x, sx));
+        } else {
+            amg_prolong_kernel<<<amg_rows_grid(ctx, L.nloc), AT, 0, sx>>>(L.nloc, L.agg, xc, S.scale, L.x, L.r);
+            KERNEL_CHECK();
+            NODAL_TRY(exchange(S, dev, 2 * l + 1, L.halo, L.r_off, sx));
+            NODAL_TRY(sweep<2>(S, L, b, L.r, l == 0 ? u0 : L.x, sx));
+        }
     }
     return NODAL_OK;
 }

@@ -34,14 +34,23 @@ int csr_spmv_launch(nodal_ctx* ctx, int32_t n, int64_t nnz, const int32_t* indpt
                     cudaStream_t st);
 
 #ifdef __CUDACC__
-// Dot product of one SELL row (lane) with x: entries k = 0..w-1 at base + 32k.  Straight-line
-// code per width -- all column/value loads first, then all gathers, then the FMA chain in CSR
-// order -- so the memory-level parallelism does not depend on how the compiler treats a
-// predicated unrolled loop (it silently fell back to a rolled, dependent loop in one kernel).
-template <int W>
+#include "amg_cycle_core.cuh"
+
+// The operand of a row product at column c: here a stored vector.  The fused V-cycle sweeps
+// (amg_kernels.cuh) pass functors that form the operand from other vectors instead.
+struct SellLoad {
+    const double* __restrict__ x;
+    __device__ __forceinline__ double operator()(int32_t c) const { return __ldg(&x[c]); }
+};
+
+// Dot product of one SELL row (lane) with the gathered operand: entries k = 0..w-1 at base + 32k.
+// Straight-line code per width -- all column/value loads first, then all gathers, then the FMA
+// chain in CSR order -- so the memory-level parallelism does not depend on how the compiler treats
+// a predicated unrolled loop (it silently fell back to a rolled, dependent loop in one kernel).
+template <int W, class G>
 __device__ __forceinline__ double sell_dot_fixed(const int32_t* __restrict__ cols,
                                                  const double* __restrict__ vals, int64_t base,
-                                                 const double* __restrict__ x, double acc) {
+                                                 const G& gather, double acc) {
     int32_t c[W];
     double v[W], xv[W];
 #pragma unroll
@@ -50,15 +59,16 @@ __device__ __forceinline__ double sell_dot_fixed(const int32_t* __restrict__ col
         v[i] = vals[base + (int64_t)i * 32];
     }
 #pragma unroll
-    for (int i = 0; i < W; ++i) xv[i] = __ldg(&x[c[i]]);
+    for (int i = 0; i < W; ++i) xv[i] = gather(c[i]);
 #pragma unroll
-    for (int i = 0; i < W; ++i) acc = fma(v[i], xv[i], acc);
+    for (int i = 0; i < W; ++i) acc = amg_dot_step(v[i], xv[i], acc);
     return acc;
 }
 
-__device__ __forceinline__ double sell_row_dot(const int32_t* __restrict__ cols,
-                                               const double* __restrict__ vals, int64_t base, int w,
-                                               const double* __restrict__ x) {
+template <class G>
+__device__ __forceinline__ double sell_row_gather(const int32_t* __restrict__ cols,
+                                                  const double* __restrict__ vals, int64_t base, int w,
+                                                  const G& x) {
     double acc = 0.0;
     int k = 0;
     for (; k + 8 <= w; k += 8) acc = sell_dot_fixed<8>(cols, vals, base + (int64_t)k * 32, x, acc);
@@ -74,5 +84,11 @@ __device__ __forceinline__ double sell_row_dot(const int32_t* __restrict__ cols,
         default: break;
     }
     return acc;
+}
+
+__device__ __forceinline__ double sell_row_dot(const int32_t* __restrict__ cols,
+                                               const double* __restrict__ vals, int64_t base, int w,
+                                               const double* __restrict__ x) {
+    return sell_row_gather(cols, vals, base, w, SellLoad{x});
 }
 #endif

@@ -150,6 +150,14 @@ class DeviceAMG:
                    "nodal_amg_profile_sweeps")
         return dict(spmv_dot=ms[0], residual=ms[1], jacobi=ms[2])
 
+    def profile_cycle(self, reps=64):
+        """Average ms per launch of the level-0 V-cycle kernels, unfused and fused (csrc/amg.cu,
+        nodal_amg_profile_cycle): dict(jacobi0, residual, prolong, jacobi, fused_residual, fused_post)."""
+        ms = (C.c_double * 6)()
+        _lib.check(self.dev.lib.nodal_amg_profile_cycle(self.dev.ctx, self.handle, int(reps), ms, self.dev.stream()),
+                   "nodal_amg_profile_cycle")
+        return dict(zip(("jacobi0", "residual", "prolong", "jacobi", "fused_residual", "fused_post"), list(ms)))
+
     def solve(self, rhs, rtol=1e-10, maxit=None, x0=None):
         dev, n = self.dev, self.csr.n
         x = dev.zeros(max(2, n), dev.torch.float64)[:n] if x0 is None else x0.clone()
