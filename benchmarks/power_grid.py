@@ -9,7 +9,14 @@ elimination (csrc/sources.cu) exists for.
 One JSON document (also printed): the card's name and power limit; per rep of the eliminated solve
 the split assemble (full MNA CSR), forest, reduce, reduced assembly, AMG setup, solve, expand, the
 iterations and relres_full; and the "before": the GMRES path (eliminate_sources=False) on the same
-generator at the smaller sizes with an explicit iteration cap -- time, iterations, status, relres."""
+generator at the smaller sizes with an explicit iteration cap -- time, iterations, status, relres.
+
+    python -m torch.distributed.run --nproc-per-node R benchmarks/power_grid.py --distributed [--n ...]
+
+The row-partitioned eliminated solve (Circuit(..., distributed=True), nodal_b200/dist_sources.py)
+instead: per rep and per rank the split share upload, full-row exchange and assembly, E gather and
+forest, reduction, reduced exchange and assembly, AMG setup and solve (iterations), expansion and
+relres_full; rank 0 writes the document."""
 import argparse
 import json
 import os
@@ -72,6 +79,37 @@ def eliminated(N, pitch, reps):
     return rows[1:]
 
 
+def distributed(N, pitch, reps):
+    import torch.distributed as dist
+    rank, world, local = (int(os.environ[k]) for k in ("RANK", "WORLD_SIZE", "LOCAL_RANK"))
+    torch.cuda.set_device(local)
+    dist.init_process_group("nccl", device_id=torch.device("cuda", local))
+    net = gen.power_grid(N, pitch, vdd=1.0, load=1e-4, seed=0)
+    table = net.table()
+    rows = []
+    for rep in range(reps + 1):                 # rep 0 warms every kernel, the allocator and NCCL up
+        dist.barrier()
+        circuit, build_ms = timed(lambda: n.Circuit(net, sparse=True, distributed=True))
+        sol, total_ms = timed(circuit.solve)
+        st, red = sol.stats, sol.stats["reduction"]
+        row = dict(rep=rep, rank=rank, world=world, unknowns=table.n, build_ms=build_ms, solve_total_ms=total_ms,
+                   upload_ms=red["upload_ms"], full_exchange_assemble_ms=red["full_assemble_ms"],
+                   e_gather_forest_ms=red["forest_ms"], reduce_ms=red["reduce_ms"],
+                   reduced_exchange_assemble_ms=red["assemble_ms"], amg_setup_ms=st.get("setup_ms"),
+                   amg_solve_ms=st.get("solve_ms"), reduced_solve_wall_ms=red["solve_ms"], iterations=st["iterations"],
+                   solver=st["solver"], status=st["status"], expand_ms=red["expand_ms"], relres_ms=red["relres_ms"],
+                   relres_full=red["relres_full"], reduced_rows=red["reduced_rows"],
+                   local_rows=int(circuit.G.shape[0]), local_nnz=circuit.G.nnz)
+        if rank == 0:
+            print(json.dumps(row), flush=True)
+        rows.append(row)
+        del circuit, sol
+    every = [None] * world
+    dist.all_gather_object(every, rows)
+    dist.destroy_process_group()
+    return rank, [r for per_rank in every for r in per_rank if r["rep"] > 0]
+
+
 def gmres_before(N, pitch, maxit):
     net = gen.power_grid(N, pitch, vdd=1.0, load=1e-4, seed=0)
     circuit = n.Circuit(net, sparse=True, eliminate_sources=False, maxit=maxit)
@@ -94,10 +132,19 @@ def main():
     ap.add_argument("--gmres-sizes", default="512,1024")
     ap.add_argument("--gmres-maxit", type=int, default=3000)
     ap.add_argument("--out", default=None)
+    ap.add_argument("--distributed", action="store_true", help="row-partitioned solve, run under torchrun")
     args = ap.parse_args()
     if not torch.cuda.is_available():
         sys.exit("power_grid.py measures the GPU path: no CUDA device")
     doc = dict(card=card(), n=args.n, pitch=args.pitch, load="uniform [0, 1e-4) A on every node, 1 ohm mesh, 1 V pads")
+    if args.distributed:
+        rank, doc["distributed"] = distributed(args.n, args.pitch, args.reps)
+        doc["world"] = doc["distributed"][0]["world"]
+        if rank == 0 and args.out:
+            os.makedirs(os.path.dirname(os.path.abspath(args.out)), exist_ok=True)
+            with open(args.out, "w") as fh:
+                json.dump(doc, fh, indent=1)
+        return
     doc["eliminated"] = eliminated(args.n, args.pitch, args.reps)
     doc["gmres_before"] = [gmres_before(int(s), args.pitch, args.gmres_maxit)
                            for s in args.gmres_sizes.split(",") if s]

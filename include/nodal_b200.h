@@ -236,6 +236,32 @@ int nodal_source_expand(nodal_ctx* ctx, int32_t kcl, int32_t n, int32_t nsrc, co
                         const int32_t* depth, int32_t max_depth, const double* y, const double* rhs,
                         int64_t nnz, const int32_t* indptr, const int32_t* indices, const double* data,
                         double* x, double* relres_h, void* stream);
+/* The stages of nodal_source_expand for the row-partitioned solve, where a rank holds rows [rb, re)
+ * of the full MNA matrix (n rows, nnz_full entries in all; indptr rebased to 0, global columns) and
+ * the forest of the E-only table (erow / a / b / branch index that table).  They launch the kernels
+ * of nodal_source_expand, and the row products take their lanes per row from (n, nnz_full), so the
+ * currents are bit-identical to the single-GPU expansion of the same y.
+ * nodal_source_potentials: x (n) = potentials from y (all nodes), 0 on the branch rows.
+ * nodal_source_tree_rows: for the rank's rows whose node has depth >= 1, in row order: the row, its
+ * rhs entry (rhs: the rank's re - rb entries) and (G x)[row]; out_*: re - rb entries capacity,
+ * *count_h the number written.
+ * nodal_source_currents: the source currents into x[kcl + branch] from the tree rows of all ranks
+ * (ntree entries, any order).
+ * nodal_source_residual: sums_h[0] = sum (rhs - G x)^2 and sums_h[1] = sum rhs^2 over the rank's
+ * rows (block partials added in a fixed order). */
+int nodal_source_potentials(nodal_ctx* ctx, int32_t kcl, int32_t n, const int32_t* rep_row, const double* offset,
+                            const double* y, double* x, void* stream);
+int nodal_source_tree_rows(nodal_ctx* ctx, int32_t kcl, int32_t n, int64_t nnz_full, int32_t rb, int32_t re,
+                           const int32_t* depth, const double* rhs, int64_t nnz, const int32_t* indptr,
+                           const int32_t* indices, const double* data, const double* x, int32_t* out_row,
+                           double* out_rhs, double* out_gx, int64_t* count_h, void* stream);
+int nodal_source_currents(nodal_ctx* ctx, int32_t kcl, int32_t nsrc, const int32_t* erow, const int32_t* a,
+                          const int32_t* b, const int32_t* branch, const int32_t* adj_ptr, const int32_t* adj_row,
+                          const int32_t* depth, int32_t max_depth, int64_t ntree, const int32_t* tree_row,
+                          const double* tree_rhs, const double* tree_gx, double* x, void* stream);
+int nodal_source_residual(nodal_ctx* ctx, int32_t n, int64_t nnz_full, int32_t rows, const double* rhs, int64_t nnz,
+                          const int32_t* indptr, const int32_t* indices, const double* data, const double* x,
+                          double* sums_h, void* stream);
 
 /* ---------------------------------------------------------------- dense kernels
  * Blocked FP64 LU with partial pivoting + triangular solves.  Replaces
@@ -326,6 +352,27 @@ int nodal_table_select_gather(nodal_ctx* ctx, int64_t ncomp, const uint32_t* pos
                               uint8_t* out_type, double* out_value, int32_t* out_a, int32_t* out_b,
                               int32_t* out_c, int32_t* out_d, int32_t* out_drv, int32_t* out_branch,
                               void* stream);
+/* The same selection for R / A / E tables (_mna_): a component is also selected when it is an E row
+ * whose branch row kcl + branch is in [rb, re) -- the rows it writes are its leads' and that one.
+ * type and branch must be given.  And by type (_type_): the components whose type is t (the E rows
+ * the source forest is built from). */
+int nodal_table_select_mna_scan(nodal_ctx* ctx, int64_t ncomp, const uint8_t* type, const int32_t* a,
+                                const int32_t* b, const int32_t* branch, int32_t kcl, int32_t rb, int32_t re,
+                                uint32_t* pos, int64_t* count_h, void* stream);
+int nodal_table_select_mna_gather(nodal_ctx* ctx, int64_t ncomp, const uint32_t* pos, int32_t kcl, int32_t rb,
+                                  int32_t re, const uint8_t* type, const double* value, const int32_t* a,
+                                  const int32_t* b, const int32_t* c, const int32_t* d, const int32_t* drv,
+                                  const int32_t* branch, uint8_t* out_type, double* out_value, int32_t* out_a,
+                                  int32_t* out_b, int32_t* out_c, int32_t* out_d, int32_t* out_drv,
+                                  int32_t* out_branch, void* stream);
+int nodal_table_select_type_scan(nodal_ctx* ctx, int64_t ncomp, const uint8_t* type, const int32_t* a,
+                                 const int32_t* b, int32_t t, uint32_t* pos, int64_t* count_h, void* stream);
+int nodal_table_select_type_gather(nodal_ctx* ctx, int64_t ncomp, const uint32_t* pos, int32_t t,
+                                   const uint8_t* type, const double* value, const int32_t* a, const int32_t* b,
+                                   const int32_t* c, const int32_t* d, const int32_t* drv, const int32_t* branch,
+                                   uint8_t* out_type, double* out_value, int32_t* out_a, int32_t* out_b,
+                                   int32_t* out_c, int32_t* out_d, int32_t* out_drv, int32_t* out_branch,
+                                   void* stream);
 
 /* Row-partitioned aggregation-AMG preconditioned CG (csrc/dist_amg.cu): same partition contract as
  * nodal_dist_pcg, same call it replaces (spsolve, nodal/nodal.py:325, for R / A netlists).  Aggregates

@@ -75,6 +75,16 @@ SIGNATURES = {
     "nodal_amg_profile_cycle": (C.c_int, [_vp, _vp, _i32, C.POINTER(_f64), _vp]),
     "nodal_table_select_scan": (C.c_int, [_vp, _i64, _vp, _vp, _i32, _i32, _vp, C.POINTER(_i64), _vp]),
     "nodal_table_select_gather": (C.c_int, [_vp, _i64, _vp, _i32, _i32] + [_vp] * 16 + [_vp]),
+    "nodal_table_select_mna_scan": (C.c_int, [_vp, _i64, _vp, _vp, _vp, _vp, _i32, _i32, _i32, _vp, C.POINTER(_i64),
+                                              _vp]),
+    "nodal_table_select_mna_gather": (C.c_int, [_vp, _i64, _vp, _i32, _i32, _i32] + [_vp] * 16 + [_vp]),
+    "nodal_table_select_type_scan": (C.c_int, [_vp, _i64, _vp, _vp, _vp, _i32, _vp, C.POINTER(_i64), _vp]),
+    "nodal_table_select_type_gather": (C.c_int, [_vp, _i64, _vp, _i32] + [_vp] * 16 + [_vp]),
+    "nodal_source_potentials": (C.c_int, [_vp, _i32, _i32, _vp, _vp, _vp, _vp, _vp]),
+    "nodal_source_tree_rows": (C.c_int, [_vp, _i32, _i32, _i64, _i32, _i32, _vp, _vp, _i64, _vp, _vp, _vp, _vp, _vp,
+                                         _vp, _vp, C.POINTER(_i64), _vp]),
+    "nodal_source_currents": (C.c_int, [_vp, _i32, _i32] + [_vp] * 7 + [_i32, _i64, _vp, _vp, _vp, _vp, _vp]),
+    "nodal_source_residual": (C.c_int, [_vp, _i32, _i64, _i32, _vp, _i64, _vp, _vp, _vp, _vp, C.POINTER(_f64), _vp]),
     "nodal_dist_amg_pcg": (C.c_int, [_vp, _vp, _i32, _vp, _i64, _vp, _vp, _vp, _vp, _vp, C.POINTER(_f64), _f64,
                                      _i32, C.POINTER(_i32), C.POINTER(_f64), C.POINTER(_f64), _vp]),
 }

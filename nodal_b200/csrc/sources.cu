@@ -15,6 +15,9 @@
 //   nodal_source_expand        potentials from the reduced solution, KCL residual with the full G,
 //                              subtree sums level by level from the deepest, source currents, and
 //                              the relative residual of the full system.
+//   nodal_source_potentials / _tree_rows / _currents / _residual
+//                              the same expansion in stages for a rank of the row-partitioned solve
+//                              (nodal_b200/dist_sources.py), launching the same kernels.
 //
 // Nothing accumulates floating-point values with atomics: results are bitwise reproducible.
 #include <algorithm>
@@ -446,6 +449,163 @@ extern "C" int nodal_source_expand(nodal_ctx* ctx, int32_t kcl, int32_t n, int32
         CUDA_TRY(cudaMemcpyAsync(host, part + 2 * parts, 2 * sizeof(double), cudaMemcpyDeviceToHost, st));
         CUDA_TRY(cudaStreamSynchronize(st));
         *relres_h = host[1] > 0.0 ? sqrt(host[0] / host[1]) : sqrt(host[0]);
+        return NODAL_OK;
+    };
+    const int rc = run();
+    ctx_pool_free(ctx, gx);
+    ctx_pool_free(ctx, part);
+    return rc;
+}
+
+// ---------------------------------------------------------------- expansion in stages (row-partitioned)
+// The stages of nodal_source_expand for a rank that holds rows [rb, re) of the full MNA matrix
+// (row pointer rebased to 0, global columns) and the replicated forest of the E-only table.  They
+// launch the kernels above; the row products take their lanes per row from the whole matrix's
+// shape, so every rank forms G x on its rows exactly as the single-GPU expansion does.
+__global__ void __launch_bounds__(ST)
+src_tree_flag_kernel(int32_t rows, int32_t rb, int32_t kcl, const int32_t* __restrict__ depth, u32* __restrict__ flag) {
+    GRID_STRIDE(i, rows) {
+        const int64_t v = rb + i;
+        flag[i] = (v < kcl && depth[v] >= 1) ? 1u : 0u;
+    }
+}
+
+__global__ void __launch_bounds__(ST)
+src_tree_place_kernel(int32_t rows, int32_t rb, int32_t kcl, const int32_t* __restrict__ depth,
+                      const u32* __restrict__ pos, const double* __restrict__ rhs, const double* __restrict__ gx,
+                      int32_t* __restrict__ o_row, double* __restrict__ o_rhs, double* __restrict__ o_gx) {
+    GRID_STRIDE(i, rows) {
+        const int64_t v = rb + i;
+        if (!(v < kcl && depth[v] >= 1)) continue;
+        const u32 p = pos[i];
+        o_row[p] = (int32_t)v;
+        o_rhs[p] = rhs[i];
+        o_gx[p] = gx[i];
+    }
+}
+
+__global__ void __launch_bounds__(ST)
+src_tree_scatter_kernel(int32_t count, const int32_t* __restrict__ row, const double* __restrict__ t_rhs,
+                        const double* __restrict__ t_gx, double* __restrict__ rhs, double* __restrict__ gx) {
+    GRID_STRIDE(k, count) {
+        rhs[row[k]] = t_rhs[k];
+        gx[row[k]] = t_gx[k];
+    }
+}
+
+extern "C" int nodal_source_potentials(nodal_ctx* ctx, int32_t kcl, int32_t n, const int32_t* rep_row,
+                                       const double* offset, const double* y, double* x, void* stream) {
+    if (!ctx || kcl < 0 || n < kcl) return NODAL_BAD_ARG;
+    if (n == 0) return NODAL_OK;
+    CUDA_TRY(cudaSetDevice(ctx->device));
+    src_potentials_kernel<<<src_grid(ctx, n), ST, 0, (cudaStream_t)stream>>>(kcl, n, rep_row, offset, y, x);
+    KERNEL_CHECK();
+    return NODAL_OK;
+}
+
+extern "C" int nodal_source_tree_rows(nodal_ctx* ctx, int32_t kcl, int32_t n, int64_t nnz_full, int32_t rb, int32_t re,
+                                      const int32_t* depth, const double* rhs, int64_t nnz, const int32_t* indptr,
+                                      const int32_t* indices, const double* data, const double* x, int32_t* out_row,
+                                      double* out_rhs, double* out_gx, int64_t* count_h, void* stream) {
+    if (!ctx || kcl < 0 || n < kcl || rb < 0 || re < rb || re > n || nnz < 0 || !count_h) return NODAL_BAD_ARG;
+    *count_h = 0;
+    const int32_t rows = re - rb;
+    if (rows == 0) return NODAL_OK;
+    NvtxRange nvtx_range("nodal_source_tree_rows");
+    CUDA_TRY(cudaSetDevice(ctx->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    NODAL_TRY(ctx_reserve(ctx, scan_scratch_bytes(rows) + 4096));
+    u32* total = carve<u32>(ctx, 16);
+    if (!total) return NODAL_CUDA_ERROR;
+    double* gx = static_cast<double*>(ctx_pool_alloc(ctx, sizeof(double) * (size_t)rows));
+    u32* pos = static_cast<u32*>(ctx_pool_alloc(ctx, sizeof(u32) * (size_t)rows));
+    auto run = [&]() -> int {
+        if (!gx || !pos) {
+            nodal_set_error("nodal_source_tree_rows: out of device memory");
+            return NODAL_CUDA_ERROR;
+        }
+        NODAL_TRY(csr_spmv_rows_launch(ctx, rows, indptr, indices, data, x, gx, n, nnz_full, st));
+        src_tree_flag_kernel<<<src_grid(ctx, rows), ST, 0, st>>>(rows, rb, kcl, depth, pos);
+        KERNEL_CHECK();
+        NODAL_TRY(scan_exclusive_u32(ctx, pos, pos, rows, total, st));
+        src_tree_place_kernel<<<src_grid(ctx, rows), ST, 0, st>>>(rows, rb, kcl, depth, pos, rhs, gx, out_row, out_rhs,
+                                                                  out_gx);
+        KERNEL_CHECK();
+        u32* total_h = reinterpret_cast<u32*>(ctx->pinned);
+        CUDA_TRY(cudaMemcpyAsync(total_h, total, sizeof(u32), cudaMemcpyDeviceToHost, st));
+        CUDA_TRY(cudaStreamSynchronize(st));
+        *count_h = total_h[0];
+        return NODAL_OK;
+    };
+    const int rc = run();
+    ctx_pool_free(ctx, gx);
+    ctx_pool_free(ctx, pos);
+    return rc;
+}
+
+extern "C" int nodal_source_currents(nodal_ctx* ctx, int32_t kcl, int32_t nsrc, const int32_t* erow, const int32_t* a,
+                                     const int32_t* b, const int32_t* branch, const int32_t* adj_ptr,
+                                     const int32_t* adj_row, const int32_t* depth, int32_t max_depth, int64_t ntree,
+                                     const int32_t* tree_row, const double* tree_rhs, const double* tree_gx, double* x,
+                                     void* stream) {
+    if (!ctx || kcl < 0 || nsrc < 0 || max_depth < 0 || ntree < 0 || ntree > kcl) return NODAL_BAD_ARG;
+    if (nsrc == 0 || max_depth == 0) return NODAL_OK;
+    NvtxRange nvtx_range("nodal_source_currents");
+    CUDA_TRY(cudaSetDevice(ctx->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    // node-indexed rhs and G x; only the nodes at depth >= 1 (the tree rows) are read
+    double* rhs = static_cast<double*>(ctx_pool_alloc(ctx, sizeof(double) * ((size_t)kcl + 1)));
+    double* gx = static_cast<double*>(ctx_pool_alloc(ctx, sizeof(double) * ((size_t)kcl + 1)));
+    auto run = [&]() -> int {
+        if (!rhs || !gx) {
+            nodal_set_error("nodal_source_currents: out of device memory");
+            return NODAL_CUDA_ERROR;
+        }
+        if (ntree > 0) {
+            src_tree_scatter_kernel<<<src_grid(ctx, ntree), ST, 0, st>>>((int32_t)ntree, tree_row, tree_rhs, tree_gx,
+                                                                         rhs, gx);
+            KERNEL_CHECK();
+        }
+        for (int32_t level = max_depth; level >= 1; --level) {
+            src_subtree_level_kernel<<<src_grid(ctx, nsrc), ST, 0, st>>>(nsrc, erow, a, b, branch, kcl, adj_ptr,
+                                                                         adj_row, depth, level, rhs, gx, x);
+            KERNEL_CHECK();
+        }
+        return NODAL_OK;
+    };
+    const int rc = run();
+    ctx_pool_free(ctx, rhs);
+    ctx_pool_free(ctx, gx);
+    return rc;
+}
+
+extern "C" int nodal_source_residual(nodal_ctx* ctx, int32_t n, int64_t nnz_full, int32_t rows, const double* rhs,
+                                     int64_t nnz, const int32_t* indptr, const int32_t* indices, const double* data,
+                                     const double* x, double* sums_h, void* stream) {
+    if (!ctx || rows < 0 || rows > n || nnz < 0 || !sums_h) return NODAL_BAD_ARG;
+    sums_h[0] = sums_h[1] = 0.0;
+    if (rows == 0) return NODAL_OK;
+    NvtxRange nvtx_range("nodal_source_residual");
+    CUDA_TRY(cudaSetDevice(ctx->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    const int parts = src_grid(ctx, rows);
+    double* gx = static_cast<double*>(ctx_pool_alloc(ctx, sizeof(double) * (size_t)rows));
+    double* part = static_cast<double*>(ctx_pool_alloc(ctx, sizeof(double) * (2 * (size_t)parts + 2)));
+    auto run = [&]() -> int {
+        if (!gx || !part) {
+            nodal_set_error("nodal_source_residual: out of device memory");
+            return NODAL_CUDA_ERROR;
+        }
+        NODAL_TRY(csr_spmv_rows_launch(ctx, rows, indptr, indices, data, x, gx, n, nnz_full, st));
+        src_residual_partials_kernel<<<parts, ST, 0, st>>>(rows, rhs, gx, part);
+        KERNEL_CHECK();
+        src_residual_final_kernel<<<1, ST, 0, st>>>(parts, part, part + 2 * parts);
+        KERNEL_CHECK();
+        double* host = reinterpret_cast<double*>(ctx->pinned);
+        CUDA_TRY(cudaMemcpyAsync(host, part + 2 * parts, 2 * sizeof(double), cudaMemcpyDeviceToHost, st));
+        CUDA_TRY(cudaStreamSynchronize(st));
+        sums_h[0] = host[0];
+        sums_h[1] = host[1];
         return NODAL_OK;
     };
     const int rc = run();

@@ -32,6 +32,11 @@ void sell_clear_l2_window(cudaStream_t st);
 int csr_spmv_launch(nodal_ctx* ctx, int32_t n, int64_t nnz, const int32_t* indptr,
                     const int32_t* indices, const double* data, const double* x, double* y,
                     cudaStream_t st);
+// The same for `rows` rows of a larger matrix (shape_n rows, shape_nnz entries): the lanes per row
+// follow the whole matrix's shape, so every row's sum is formed as csr_spmv_launch forms it there.
+int csr_spmv_rows_launch(nodal_ctx* ctx, int32_t rows, const int32_t* indptr, const int32_t* indices,
+                         const double* data, const double* x, double* y, int32_t shape_n, int64_t shape_nnz,
+                         cudaStream_t st);
 
 #ifdef __CUDACC__
 #include "amg_cycle_core.cuh"

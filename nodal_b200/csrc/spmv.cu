@@ -43,8 +43,14 @@ static int pick_tpr(int32_t n, int64_t nnz) {
 int csr_spmv_launch(nodal_ctx* ctx, int32_t n, int64_t nnz, const int32_t* indptr,
                     const int32_t* indices, const double* data, const double* x, double* y,
                     cudaStream_t st) {
+    return csr_spmv_rows_launch(ctx, n, indptr, indices, data, x, y, n, nnz, st);
+}
+
+int csr_spmv_rows_launch(nodal_ctx* ctx, int32_t n, const int32_t* indptr, const int32_t* indices,
+                         const double* data, const double* x, double* y, int32_t shape_n, int64_t shape_nnz,
+                         cudaStream_t st) {
     if (n == 0) return NODAL_OK;
-    const int tpr = pick_tpr(n, nnz);
+    const int tpr = pick_tpr(shape_n, shape_nnz);
     int64_t blocks = ((int64_t)n * tpr + SPMV_THREADS - 1) / SPMV_THREADS;
     const int64_t cap = (int64_t)ctx->num_sms * 8;
     const int grid = (int)(blocks < cap ? blocks : cap);

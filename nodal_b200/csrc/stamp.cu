@@ -90,19 +90,46 @@ extern "C" int nodal_stamp_coo(nodal_ctx* ctx, int64_t ncomp, const uint8_t* typ
 }
 
 // ---------------------------------------------------------------- row-partitioned assembly
-// A rank of the multi-GPU path stamps only the components with a lead on one of its rows
-// [rb, re) (global stamping order kept, so its rows of G are bit-identical to the single-GPU
-// CSR).  The selection runs on the device from the full resident table: flags -> exclusive scan
-// -> ordered gather of the eight columns.
+// A rank of the multi-GPU path stamps only the components that write one of its rows [rb, re)
+// (global stamping order kept, so its rows of G are bit-identical to the single-GPU CSR).  The
+// selection runs on the device: flags -> exclusive scan -> ordered gather of the eight columns.
+// A component is selected when a lead is on a row in [rb, re) -- the only rows an R / A component
+// writes -- or when the kernel's extra test holds:
+//   NoExtra        nothing more (R / A tables)
+//   OwnBranchRow   an E row whose branch row kcl + branch is in [rb, re) (R / A / E tables)
+//   TypeIs         components of one type, with an empty [rb, re) (the E rows of the source forest)
+struct NoExtra {
+    __device__ __forceinline__ bool operator()(int64_t, int32_t, int32_t) const { return false; }
+};
+
+struct OwnBranchRow {
+    const uint8_t* __restrict__ type;
+    const int32_t* __restrict__ branch;
+    int32_t kcl;
+    __device__ __forceinline__ bool operator()(int64_t i, int32_t rb, int32_t re) const {
+        if (type[i] != NODAL_T_E) return false;
+        const int32_t r = kcl + branch[i];
+        return r >= rb && r < re;
+    }
+};
+
+struct TypeIs {
+    const uint8_t* __restrict__ type;
+    int32_t t;
+    __device__ __forceinline__ bool operator()(int64_t i, int32_t, int32_t) const { return type[i] == t; }
+};
+
+template <class Extra>
 __global__ void __launch_bounds__(STAMP_THREADS)
 select_flag_kernel(int64_t ncomp, const int32_t* __restrict__ a, const int32_t* __restrict__ b, int32_t rb,
-                   int32_t re, u32* __restrict__ flag) {
+                   int32_t re, u32* __restrict__ flag, Extra extra) {
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < ncomp; i += (int64_t)gridDim.x * blockDim.x) {
         const int32_t x = a[i], y = b[i];
-        flag[i] = ((x >= rb && x < re) || (y >= rb && y < re)) ? 1u : 0u;
+        flag[i] = ((x >= rb && x < re) || (y >= rb && y < re) || extra(i, rb, re)) ? 1u : 0u;
     }
 }
 
+template <class Extra>
 __global__ void __launch_bounds__(STAMP_THREADS)
 select_gather_kernel(int64_t ncomp, const u32* __restrict__ pos, int32_t rb, int32_t re,
                      const uint8_t* __restrict__ type, const double* __restrict__ value,
@@ -110,10 +137,10 @@ select_gather_kernel(int64_t ncomp, const u32* __restrict__ pos, int32_t rb, int
                      const int32_t* __restrict__ d, const int32_t* __restrict__ drv, const int32_t* __restrict__ branch,
                      uint8_t* __restrict__ o_type, double* __restrict__ o_value, int32_t* __restrict__ o_a,
                      int32_t* __restrict__ o_b, int32_t* __restrict__ o_c, int32_t* __restrict__ o_d,
-                     int32_t* __restrict__ o_drv, int32_t* __restrict__ o_branch) {
+                     int32_t* __restrict__ o_drv, int32_t* __restrict__ o_branch, Extra extra) {
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < ncomp; i += (int64_t)gridDim.x * blockDim.x) {
         const int32_t x = a[i], y = b[i];
-        if (!((x >= rb && x < re) || (y >= rb && y < re))) continue;
+        if (!((x >= rb && x < re) || (y >= rb && y < re) || extra(i, rb, re))) continue;
         const u32 p = pos[i];
         o_type[p] = type[i]; o_value[p] = value[i]; o_a[p] = x; o_b[p] = y;
         if (c) o_c[p] = c[i];
@@ -123,8 +150,13 @@ select_gather_kernel(int64_t ncomp, const u32* __restrict__ pos, int32_t rb, int
     }
 }
 
-extern "C" int nodal_table_select_scan(nodal_ctx* ctx, int64_t ncomp, const int32_t* a, const int32_t* b,
-                                       int32_t rb, int32_t re, uint32_t* pos, int64_t* count_h, void* stream) {
+static int select_grid(nodal_ctx* ctx, int64_t ncomp) {
+    return (int)std::min<int64_t>((ncomp + STAMP_THREADS - 1) / STAMP_THREADS, (int64_t)ctx->num_sms * 16);
+}
+
+template <class Extra>
+static int select_scan(nodal_ctx* ctx, int64_t ncomp, const int32_t* a, const int32_t* b, int32_t rb, int32_t re,
+                       Extra extra, uint32_t* pos, int64_t* count_h, void* stream) {
     if (!ctx || ncomp < 0 || !count_h || ncomp >= ((int64_t)1 << 32)) return NODAL_BAD_ARG;
     *count_h = 0;
     if (ncomp == 0) return NODAL_OK;
@@ -133,8 +165,7 @@ extern "C" int nodal_table_select_scan(nodal_ctx* ctx, int64_t ncomp, const int3
     NODAL_TRY(ctx_reserve(ctx, scan_scratch_bytes(ncomp) + 4096));
     u32* total = carve<u32>(ctx, 16);
     if (!total) return NODAL_CUDA_ERROR;
-    const int grid = (int)std::min<int64_t>((ncomp + STAMP_THREADS - 1) / STAMP_THREADS, (int64_t)ctx->num_sms * 16);
-    select_flag_kernel<<<grid, STAMP_THREADS, 0, st>>>(ncomp, a, b, rb, re, pos);
+    select_flag_kernel<Extra><<<select_grid(ctx, ncomp), STAMP_THREADS, 0, st>>>(ncomp, a, b, rb, re, pos, extra);
     KERNEL_CHECK();
     NODAL_TRY(scan_exclusive_u32(ctx, pos, pos, ncomp, total, st));
     u32* total_h = reinterpret_cast<u32*>(ctx->pinned);
@@ -144,19 +175,70 @@ extern "C" int nodal_table_select_scan(nodal_ctx* ctx, int64_t ncomp, const int3
     return NODAL_OK;
 }
 
+template <class Extra>
+static int select_gather(nodal_ctx* ctx, int64_t ncomp, const uint32_t* pos, int32_t rb, int32_t re, Extra extra,
+                         const uint8_t* type,
+                         const double* value, const int32_t* a, const int32_t* b, const int32_t* c, const int32_t* d,
+                         const int32_t* drv, const int32_t* branch, uint8_t* o_type, double* o_value, int32_t* o_a,
+                         int32_t* o_b, int32_t* o_c, int32_t* o_d, int32_t* o_drv, int32_t* o_branch, void* stream) {
+    if (!ctx || ncomp < 0) return NODAL_BAD_ARG;
+    if (ncomp == 0) return NODAL_OK;
+    CUDA_TRY(cudaSetDevice(ctx->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    select_gather_kernel<Extra><<<select_grid(ctx, ncomp), STAMP_THREADS, 0, st>>>(
+        ncomp, pos, rb, re, type, value, a, b, c, d, drv, branch, o_type, o_value, o_a, o_b, o_c, o_d, o_drv, o_branch,
+        extra);
+    KERNEL_CHECK();
+    return NODAL_OK;
+}
+
+extern "C" int nodal_table_select_scan(nodal_ctx* ctx, int64_t ncomp, const int32_t* a, const int32_t* b,
+                                       int32_t rb, int32_t re, uint32_t* pos, int64_t* count_h, void* stream) {
+    return select_scan(ctx, ncomp, a, b, rb, re, NoExtra{}, pos, count_h, stream);
+}
+
 extern "C" int nodal_table_select_gather(nodal_ctx* ctx, int64_t ncomp, const uint32_t* pos, int32_t rb, int32_t re,
                                          const uint8_t* type, const double* value, const int32_t* a,
                                          const int32_t* b, const int32_t* c, const int32_t* d, const int32_t* drv,
                                          const int32_t* branch, uint8_t* o_type, double* o_value, int32_t* o_a,
                                          int32_t* o_b, int32_t* o_c, int32_t* o_d, int32_t* o_drv,
                                          int32_t* o_branch, void* stream) {
-    if (!ctx || ncomp < 0) return NODAL_BAD_ARG;
-    if (ncomp == 0) return NODAL_OK;
-    CUDA_TRY(cudaSetDevice(ctx->device));
-    cudaStream_t st = (cudaStream_t)stream;
-    const int grid = (int)std::min<int64_t>((ncomp + STAMP_THREADS - 1) / STAMP_THREADS, (int64_t)ctx->num_sms * 16);
-    select_gather_kernel<<<grid, STAMP_THREADS, 0, st>>>(ncomp, pos, rb, re, type, value, a, b, c, d, drv, branch,
-                                                        o_type, o_value, o_a, o_b, o_c, o_d, o_drv, o_branch);
-    KERNEL_CHECK();
-    return NODAL_OK;
+    return select_gather(ctx, ncomp, pos, rb, re, NoExtra{}, type, value, a, b, c, d, drv, branch, o_type, o_value,
+                         o_a, o_b, o_c, o_d, o_drv, o_branch, stream);
+}
+
+extern "C" int nodal_table_select_mna_scan(nodal_ctx* ctx, int64_t ncomp, const uint8_t* type, const int32_t* a,
+                                           const int32_t* b, const int32_t* branch, int32_t kcl, int32_t rb,
+                                           int32_t re, uint32_t* pos, int64_t* count_h, void* stream) {
+    if (ncomp > 0 && (!type || !branch)) return NODAL_BAD_ARG;
+    return select_scan(ctx, ncomp, a, b, rb, re, OwnBranchRow{type, branch, kcl}, pos, count_h, stream);
+}
+
+extern "C" int nodal_table_select_mna_gather(nodal_ctx* ctx, int64_t ncomp, const uint32_t* pos, int32_t kcl,
+                                             int32_t rb, int32_t re, const uint8_t* type, const double* value,
+                                             const int32_t* a, const int32_t* b, const int32_t* c, const int32_t* d,
+                                             const int32_t* drv, const int32_t* branch, uint8_t* o_type,
+                                             double* o_value, int32_t* o_a, int32_t* o_b, int32_t* o_c, int32_t* o_d,
+                                             int32_t* o_drv, int32_t* o_branch, void* stream) {
+    if (ncomp > 0 && (!type || !branch)) return NODAL_BAD_ARG;
+    return select_gather(ctx, ncomp, pos, rb, re, OwnBranchRow{type, branch, kcl}, type, value, a, b, c, d, drv,
+                         branch, o_type, o_value, o_a, o_b, o_c, o_d, o_drv, o_branch, stream);
+}
+
+extern "C" int nodal_table_select_type_scan(nodal_ctx* ctx, int64_t ncomp, const uint8_t* type, const int32_t* a,
+                                            const int32_t* b, int32_t t, uint32_t* pos, int64_t* count_h,
+                                            void* stream) {
+    if (ncomp > 0 && !type) return NODAL_BAD_ARG;
+    return select_scan(ctx, ncomp, a, b, 0, 0, TypeIs{type, t}, pos, count_h, stream);
+}
+
+extern "C" int nodal_table_select_type_gather(nodal_ctx* ctx, int64_t ncomp, const uint32_t* pos, int32_t t,
+                                              const uint8_t* type, const double* value, const int32_t* a,
+                                              const int32_t* b, const int32_t* c, const int32_t* d,
+                                              const int32_t* drv, const int32_t* branch, uint8_t* o_type,
+                                              double* o_value, int32_t* o_a, int32_t* o_b, int32_t* o_c,
+                                              int32_t* o_d, int32_t* o_drv, int32_t* o_branch, void* stream) {
+    if (ncomp > 0 && !type) return NODAL_BAD_ARG;
+    return select_gather(ctx, ncomp, pos, 0, 0, TypeIs{type, t}, type, value, a, b, c, d, drv, branch, o_type, o_value,
+                         o_a, o_b, o_c, o_d, o_drv, o_branch, stream);
 }

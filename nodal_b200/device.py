@@ -290,22 +290,40 @@ class Device:
         del keys, vals
         return DeviceCSR(n, indptr, indices, data), rhs
 
+    _COLUMNS = ("type", "value", "a", "b", "c", "d", "drv", "branch")
+
+    def _select(self, dtab, ncomp, scan, scan_args, gather, gather_args):
+        """Ordered flag / scan / gather of the rows of `dtab` that one selection of csrc/stamp.cu picks."""
+        pos = self.empty(max(1, ncomp), self.torch.int32)
+        count = C.c_int64(0)
+        p = self.ptr
+        _lib.check(getattr(self.lib, scan)(self.ctx, ncomp, *scan_args, p(pos), C.byref(count), self.stream()), scan)
+        m = count.value
+        out = {k: (self.empty(max(1, m), dtab[k].dtype) if dtab[k] is not None else None) for k in self._COLUMNS}
+        _lib.check(getattr(self.lib, gather)(self.ctx, ncomp, p(pos), *gather_args, *[p(dtab[k]) for k in self._COLUMNS],
+                                             *[p(out[k]) for k in self._COLUMNS], self.stream()), gather)
+        return out, m
+
     def select_local(self, dtab, ncomp, rb, re):
         """Columns of the components with a lead on a row in [rb, re), order kept, selected on the
         device from the resident table (row-partitioned assembly).  Returns (columns, count)."""
-        torch = self.torch
-        pos = self.empty(max(1, ncomp), torch.int32)
-        count = C.c_int64(0)
         p = self.ptr
-        _lib.check(self.lib.nodal_table_select_scan(self.ctx, ncomp, p(dtab["a"]), p(dtab["b"]), int(rb), int(re),
-                                                    p(pos), C.byref(count), self.stream()), "nodal_table_select_scan")
-        m = count.value
-        names = ("type", "value", "a", "b", "c", "d", "drv", "branch")
-        out = {k: (self.empty(max(1, m), dtab[k].dtype) if dtab[k] is not None else None) for k in names}
-        _lib.check(self.lib.nodal_table_select_gather(
-            self.ctx, ncomp, p(pos), int(rb), int(re), *[p(dtab[k]) for k in names], *[p(out[k]) for k in names],
-            self.stream()), "nodal_table_select_gather")
-        return out, m
+        return self._select(dtab, ncomp, "nodal_table_select_scan", (p(dtab["a"]), p(dtab["b"]), int(rb), int(re)),
+                            "nodal_table_select_gather", (int(rb), int(re)))
+
+    def select_mna_rows(self, dtab, ncomp, kcl, rb, re):
+        """The same for an R / A / E table: also the E rows whose branch row kcl + branch is in [rb, re)."""
+        p = self.ptr
+        return self._select(dtab, ncomp, "nodal_table_select_mna_scan",
+                            (p(dtab["type"]), p(dtab["a"]), p(dtab["b"]), p(dtab["branch"]), int(kcl), int(rb), int(re)),
+                            "nodal_table_select_mna_gather", (int(kcl), int(rb), int(re)))
+
+    def select_type(self, dtab, ncomp, t):
+        """Columns of the components of type `t`, order kept."""
+        p = self.ptr
+        return self._select(dtab, ncomp, "nodal_table_select_type_scan", (p(dtab["type"]), p(dtab["a"]), p(dtab["b"]),
+                                                                          int(t)),
+                            "nodal_table_select_type_gather", (int(t),))
 
     def csr_to_dense(self, csr: DeviceCSR):
         n = csr.n
@@ -428,6 +446,46 @@ class Device:
             p(y), p(rhs), csr.nnz, p(csr.indptr), p(csr.indices), p(csr.data), p(x), C.byref(relres),
             self.stream()), "nodal_source_expand")
         return x, relres.value
+
+    # the stages of source_expand for a rank's rows of the full MNA matrix (dist_sources.py)
+    def source_potentials(self, kcl, n, forest, y):
+        """x (n): the potentials of every node from the reduced solution y, 0 on the branch rows."""
+        x = self.empty(max(1, n), self.torch.float64)[:n]
+        p = self.ptr
+        _lib.check(self.lib.nodal_source_potentials(self.ctx, kcl, n, p(forest["rep_row"]), p(forest["offset"]), p(y),
+                                                    p(x), self.stream()), "nodal_source_potentials")
+        return x
+
+    def source_tree_rows(self, kcl, n, nnz_full, rb, re, forest, rows, rhs, x):
+        """(row, rhs, G x) of the rows in [rb, re) whose node hangs in a source tree (depth >= 1), in row
+        order; `rows` is the rank's LocalRows of the full matrix (n rows, nnz_full entries in all)."""
+        torch = self.torch
+        cap = max(1, re - rb)
+        row, o_rhs, o_gx = self.empty(cap, torch.int32), self.empty(cap, torch.float64), self.empty(cap, torch.float64)
+        count = C.c_int64(0)
+        p = self.ptr
+        _lib.check(self.lib.nodal_source_tree_rows(
+            self.ctx, kcl, n, nnz_full, rb, re, p(forest["depth"]), p(rhs), rows.nnz, p(rows.indptr), p(rows.indices),
+            p(rows.data), p(x), p(row), p(o_rhs), p(o_gx), C.byref(count), self.stream()), "nodal_source_tree_rows")
+        k = count.value
+        return row[:k], o_rhs[:k], o_gx[:k]
+
+    def source_currents(self, kcl, etab, forest, info, tree_row, tree_rhs, tree_gx, x):
+        """Source currents into x[kcl + branch] from the tree rows of all ranks (E-only table `etab`)."""
+        p, f = self.ptr, forest
+        _lib.check(self.lib.nodal_source_currents(
+            self.ctx, kcl, info["sources"], p(f["erow"]), p(etab["a"]), p(etab["b"]), p(etab["branch"]),
+            p(f["adj_ptr"]), p(f["adj_row"]), p(f["depth"]), info["depth"], int(tree_row.numel()), p(tree_row),
+            p(tree_rhs), p(tree_gx), p(x), self.stream()), "nodal_source_currents")
+
+    def source_residual(self, n, nnz_full, rows, rhs, x):
+        """(sum (rhs - G x)^2, sum rhs^2) over the rank's rows (LocalRows of the full matrix)."""
+        sums = (C.c_double * 2)()
+        p = self.ptr
+        _lib.check(self.lib.nodal_source_residual(self.ctx, n, nnz_full, int(rhs.numel()), p(rhs), rows.nnz,
+                                                  p(rows.indptr), p(rows.indices), p(rows.data), p(x), sums,
+                                                  self.stream()), "nodal_source_residual")
+        return sums[0], sums[1]
 
     def amg(self, csr: DeviceCSR, **params):
         """Aggregation-AMG hierarchy for an SPD DeviceCSR (csrc/amg.cu); see DeviceAMG."""

@@ -190,6 +190,52 @@ def single_solver(dev):
     return _SOLVERS[key]
 
 
+def upload_share(dev, table, names, rank, world):
+    """Rank `rank`'s contiguous 1/world share of the component table, components
+    [M rank / world, M (rank + 1) / world), as device columns (the columns not in `names` are None)."""
+    m = len(table)
+    lo, hi = m * rank // world, m * (rank + 1) // world
+    pinned = getattr(table, "_pinned", None)
+    if pinned:
+        share = {k: pinned[k][lo:hi].to(dev.dev, non_blocking=True) for k in names}
+    else:
+        share = {k: dev.to_device(getattr(table, k)[lo:hi]) for k in names}
+    for k in ("type", "value", "a", "b", "c", "d", "drv", "branch"):
+        share.setdefault(k, None)
+    return share
+
+
+def exchange_rows(dev, share, ncomp, bounds, rank, world, select):
+    """The components every rank stamps, from the ranks' shares: rank s selects on the device, for every
+    rank d, the components of its share that `select(columns, ncomp, rb, re)` picks for d's rows
+    [bounds[d], bounds[d + 1]), and the selections travel over NVLink (torch.distributed
+    all_to_all_single: plumbing).  Shares are contiguous in stamping order and are concatenated in rank
+    order, so every rank receives its components in global stamping order (bit-identical rows).
+    Returns (columns, count); columns that are None in `share` stay None."""
+    if world == 1:
+        return share, ncomp
+    import torch
+    import torch.distributed as dist
+    names = [k for k, v in share.items() if v is not None]
+    pieces, counts = [], []
+    for d in range(world):
+        sel, cnt = select(share, ncomp, int(bounds[d]), int(bounds[d + 1]))
+        pieces.append(sel)
+        counts.append(cnt)
+    send_counts = torch.tensor(counts, dtype=torch.int64, device=dev.dev)
+    recv_counts = torch.empty_like(send_counts)
+    dist.all_to_all_single(recv_counts, send_counts)
+    recv_split = [int(v) for v in recv_counts.tolist()]
+    total = sum(recv_split)
+    local = {k: None for k in share}
+    for k in names:
+        send = torch.cat([pieces[d][k][: counts[d]] for d in range(world)])
+        recv = torch.empty(max(1, total), dtype=send.dtype, device=dev.dev)[:total]
+        dist.all_to_all_single(recv, send, output_split_sizes=recv_split, input_split_sizes=counts)
+        local[k] = recv
+    return local, total
+
+
 class GridRunner:
     """One rank of the row-partitioned equivalent-resistance step used by bench.py and by
     Circuit(..., distributed=True): select the rank's components ON THE DEVICE from the full
@@ -246,41 +292,13 @@ class GridRunner:
         rank sees its components in global stamping order (bit-identical rows).  Uploading the whole
         table on every rank instead costs 24 ms of host-memory bandwidth at 8 ranks."""
         from .device import coo_stride
-        dev, torch, table = self.dev, self.dev.torch, self.table
+        dev, table = self.dev, self.table
         R, r, m = self.world, self.rank, len(table)
-        lo, hi = m * r // R, m * (r + 1) // R
-        names = ("type", "value", "a", "b") if table.is_spd_structured() else \
-                ("type", "value", "a", "b", "c", "d", "drv", "branch")
         if not table.is_spd_structured():
             raise NotImplementedError("row-partitioned solve is implemented for R / A netlists (PCG)")
-        pinned = getattr(table, "_pinned", None)
-        if pinned:
-            share = {k: pinned[k][lo:hi].to(dev.dev, non_blocking=True) for k in names}
-        else:
-            share = {k: dev.to_device(getattr(table, k)[lo:hi]) for k in names}
-        for k in ("c", "d", "drv", "branch"):
-            share.setdefault(k, None)
+        share = upload_share(dev, table, ("type", "value", "a", "b"), r, R)
         rb, re = int(self.bounds[r]), int(self.bounds[r + 1])
-        if R == 1:
-            local, ncomp = share, m
-        else:
-            import torch.distributed as dist
-            pieces, counts = [], []
-            for d in range(R):
-                sel, cnt = dev.select_local(share, hi - lo, int(self.bounds[d]), int(self.bounds[d + 1]))
-                pieces.append(sel)
-                counts.append(cnt)
-            send_counts = torch.tensor(counts, dtype=torch.int64, device=dev.dev)
-            recv_counts = torch.empty_like(send_counts)
-            dist.all_to_all_single(recv_counts, send_counts)
-            recv_split = [int(v) for v in recv_counts.tolist()]
-            ncomp = sum(recv_split)
-            local = {k: None for k in ("c", "d", "drv", "branch")}
-            for k in names:
-                send = torch.cat([pieces[d][k][: counts[d]] for d in range(R)])
-                recv = torch.empty(max(1, ncomp), dtype=send.dtype, device=dev.dev)[:ncomp]
-                dist.all_to_all_single(recv, send, output_split_sizes=recv_split, input_split_sizes=counts)
-                local[k] = recv
+        local, ncomp = exchange_rows(dev, share, m * (r + 1) // R - m * r // R, self.bounds, r, R, dev.select_local)
         csr, rhs = dev.assemble_csr_raw(local, ncomp, table.kcl, self.n, coo_stride(table))
         ip = csr.indptr[rb: re + 1]
         s, e = int(ip[0]), int(ip[-1])

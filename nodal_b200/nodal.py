@@ -24,6 +24,7 @@ import numpy as np
 
 from . import constants as c
 from . import models
+from . import dist_sources
 from . import sources
 from .table import ComponentTable
 
@@ -279,6 +280,7 @@ class Circuit:
         dev = Device.get(self.options.get("device"))
         self._dev = dev
         self._dist = None
+        self._dsrc = None
         self._dtab = None
         if self.options.get("distributed"):
             G, A = self._build_distributed(dev, table)
@@ -311,6 +313,10 @@ class Circuit:
         if not (tdist.is_available() and tdist.is_initialized()):
             raise RuntimeError("distributed=True needs an initialised torch.distributed process group")
         rank, world = tdist.get_rank(), tdist.get_world_size()
+        if dist_sources.applies(table):
+            # R / A / E netlists: through the row-partitioned elimination of the sources (dist_sources.py)
+            self._dsrc = dist_sources.DistSources(self, dev, table, rank, world)
+            return self._dsrc.G, self._dsrc.A
         runner = ndist.GridRunner(dev, table, 0, rank, world, rtol=self.options.get("rtol", 1e-10),
                                   precond="jacobi" if self.options.get("precond") == "jacobi" else "amg",
                                   amg=self.options.get("amg"), solver=ndist.shared_solver(dev, rank, world))
@@ -347,6 +353,9 @@ class Circuit:
         dev = self._dev
         if not self.sparse:
             return dev.lu_solve(self.G.clone(), rhs)
+        if self._dsrc is not None:
+            raise NotImplementedError("the row-partitioned solve of a netlist with voltage sources is implemented "
+                                      "for solve() only")
         kind = self._sparse_solver()
         rtol = self.options.get("rtol", 1e-10)
         warm = self._warm_start()
@@ -488,8 +497,12 @@ class Circuit:
             logging.error("Model error: unconnected circuit")
             raise UnconnectedCircuitError
         # R / A / E netlists: through the elimination of the voltage sources when it applies
-        # (sources.py); otherwise `info` is the stats of why not, or None
-        x, info = sources.solve(self) if self.sparse and self._dist is None else (None, None)
+        # (sources.py; dist_sources.py row-partitioned, x whole on every rank); otherwise `info` is
+        # the stats of why not, or None
+        if self._dsrc is not None:
+            x, info = self._dsrc.solve()
+        else:
+            x, info = sources.solve(self) if self.sparse and self._dist is None else (None, None)
         if x is None:
             skipped = info
             x, info = self._device_solve(self.A)

@@ -51,6 +51,15 @@ def skip_reason(table, mode, dense_limit):
     return ""
 
 
+def forest_reason(finfo):
+    """Why the forest of csrc/sources.cu cannot eliminate the sources ("" when it can)."""
+    if finfo["branch_conflicts"]:
+        return "branch rows not owned by exactly one E row (duplicate names)"
+    if finfo["loops"]:
+        return f"the E rows are not a forest ({finfo['loops']} loop(s); parallel sources or both leads on one node count)"
+    return ""
+
+
 def _ms(t0, dev):
     dev.torch.cuda.current_stream(dev.dev).synchronize()
     return (time.perf_counter() - t0) * 1e3
@@ -73,11 +82,9 @@ def solve(circuit):
     finfo, forest = dev.source_forest(dtab, len(table), table.kcl, table.be)
     stats = dict(eliminated=False, sources=finfo["sources"], supernodes=finfo["floating_trees"],
                  grounded_nodes=finfo["grounded_nodes"], forest_ms=_ms(t0, dev))
-    if finfo["branch_conflicts"]:
-        stats["reason"] = "branch rows not owned by exactly one E row (duplicate names)"
-        return None, stats
-    if finfo["loops"]:
-        stats["reason"] = f"the E rows are not a forest ({finfo['loops']} loop(s); parallel sources or both leads on one node count)"
+    reason = forest_reason(finfo)
+    if reason:
+        stats["reason"] = reason
         return None, stats
     t0 = time.perf_counter()
     red, nred = dev.source_reduce(dtab, len(table), table.kcl, forest)
