@@ -263,6 +263,36 @@ int nodal_source_residual(nodal_ctx* ctx, int32_t n, int64_t nnz_full, int32_t r
                           const int32_t* indptr, const int32_t* indices, const double* data, const double* x,
                           double* sums_h, void* stream);
 
+/* ---------------------------------------------------------------- Schur complement of the branch rows
+ * csrc/schur.cu (rules in csrc/schur_core.cuh).  G is the sorted MNA matrix of n = kcl + m rows
+ * (indptr / indices / data), G = [[L, B], [C, D]] with L the kcl x kcl resistor Laplacian.
+ * nodal_schur_split_scan: l_ptr, b_ptr (kcl + 1 each) receive the row pointers of L and of the B
+ * lists; nnz_h (host, 2) their entry counts.  nodal_schur_split_place then writes L (l_idx, l_val:
+ * the prefix of each node row with column < kcl) and B (b_col = column - kcl, b_val: the suffix).
+ * nodal_schur_rhs_batch: rhs (K x kcl, row-major) = columns j0 .. j0 + K - 1 of B.
+ * nodal_schur_columns: S[:, j0 : j0 + K] = D - C Z for Z (K x kcl, row-major) = L^-1 of that batch;
+ * S is m x m row-major.
+ * nodal_schur_branch_rhs: out (m) = r[kcl:] - C t;  nodal_schur_node_rhs: out (kcl) = r[:kcl] - B xb.
+ * nodal_schur_residual: r = rhs - G x; sums_h = (sum r^2, sum rhs^2), block partials added in a fixed
+ * order.  nodal_schur_add: x += d (count entries).  Every row is summed in CSR order. */
+int nodal_schur_split_scan(nodal_ctx* ctx, int32_t kcl, const int32_t* indptr, const int32_t* indices,
+                           int32_t* l_ptr, int32_t* b_ptr, int64_t* nnz_h, void* stream);
+int nodal_schur_split_place(nodal_ctx* ctx, int32_t kcl, const int32_t* indptr, const int32_t* indices,
+                            const double* data, const int32_t* l_ptr, int32_t* l_idx, double* l_val,
+                            const int32_t* b_ptr, int32_t* b_col, double* b_val, void* stream);
+int nodal_schur_rhs_batch(nodal_ctx* ctx, int32_t kcl, int32_t j0, int32_t K, const int32_t* b_ptr,
+                          const int32_t* b_col, const double* b_val, double* rhs, void* stream);
+int nodal_schur_columns(nodal_ctx* ctx, int32_t kcl, int32_t m, int32_t j0, int32_t K, const int32_t* indptr,
+                        const int32_t* indices, const double* data, const double* Z, double* S, void* stream);
+int nodal_schur_branch_rhs(nodal_ctx* ctx, int32_t kcl, int32_t m, const int32_t* indptr, const int32_t* indices,
+                           const double* data, const double* r, const double* t, double* out, void* stream);
+int nodal_schur_node_rhs(nodal_ctx* ctx, int32_t kcl, const int32_t* b_ptr, const int32_t* b_col,
+                         const double* b_val, const double* r, const double* xb, double* out, void* stream);
+int nodal_schur_residual(nodal_ctx* ctx, int32_t n, const int32_t* indptr, const int32_t* indices,
+                         const double* data, const double* rhs, const double* x, double* r, double* sums_h,
+                         void* stream);
+int nodal_schur_add(nodal_ctx* ctx, int64_t count, double* x, const double* d, void* stream);
+
 /* ---------------------------------------------------------------- dense kernels
  * Blocked FP64 LU with partial pivoting + triangular solves.  Replaces
  * numpy.linalg.solve (LAPACK dgesv) at nodal/nodal.py:327.  G (n x n row-major)
@@ -271,6 +301,14 @@ int nodal_source_residual(nodal_ctx* ctx, int32_t n, int64_t nnz_full, int32_t r
  * matching dgesv's info > 0 -> numpy LinAlgError. */
 int nodal_lu_solve(nodal_ctx* ctx, int32_t n, double* G, const double* rhs, double* x,
                    int32_t* info_h, void* stream);
+
+/* The same in two calls, for a matrix solved against several right-hand sides: nodal_lu_factor
+ * overwrites G with its factors and fills ipiv (device, n entries; NODAL_SINGULAR and *info_h as
+ * above); nodal_lu_solve_factored (asynchronous) then gives x for one rhs.  Factor + solve launch the
+ * kernels of nodal_lu_solve in the same order, so x is bitwise the same. */
+int nodal_lu_factor(nodal_ctx* ctx, int32_t n, double* G, int32_t* ipiv, int32_t* info_h, void* stream);
+int nodal_lu_solve_factored(nodal_ctx* ctx, int32_t n, const double* LU, const int32_t* ipiv, const double* rhs,
+                            double* x, void* stream);
 
 /* Measurement aid: the LU's DMMA trailing-update kernel alone, C[M x N] -= A[M x K] B[K x N] (row-major,
  * even leading dimension ld), average ms per launch over `reps` launches (CUDA events on `stream`).

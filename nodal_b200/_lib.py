@@ -57,7 +57,17 @@ SIGNATURES = {
                                             _vp]),
     "nodal_source_expand": (C.c_int, [_vp, _i32, _i32, _i32] + [_vp] * 9 + [_i32, _vp, _vp, _i64, _vp, _vp, _vp, _vp,
                                                                              C.POINTER(_f64), _vp]),
+    "nodal_schur_split_scan": (C.c_int, [_vp, _i32, _vp, _vp, _vp, _vp, C.POINTER(_i64), _vp]),
+    "nodal_schur_split_place": (C.c_int, [_vp, _i32] + [_vp] * 9 + [_vp]),
+    "nodal_schur_rhs_batch": (C.c_int, [_vp, _i32, _i32, _i32, _vp, _vp, _vp, _vp, _vp]),
+    "nodal_schur_columns": (C.c_int, [_vp, _i32, _i32, _i32, _i32, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "nodal_schur_branch_rhs": (C.c_int, [_vp, _i32, _i32] + [_vp] * 6 + [_vp]),
+    "nodal_schur_node_rhs": (C.c_int, [_vp, _i32] + [_vp] * 6 + [_vp]),
+    "nodal_schur_residual": (C.c_int, [_vp, _i32] + [_vp] * 6 + [C.POINTER(_f64), _vp]),
+    "nodal_schur_add": (C.c_int, [_vp, _i64, _vp, _vp, _vp]),
     "nodal_lu_solve": (C.c_int, [_vp, _i32, _vp, _vp, _vp, C.POINTER(_i32), _vp]),
+    "nodal_lu_factor": (C.c_int, [_vp, _i32, _vp, _vp, C.POINTER(_i32), _vp]),
+    "nodal_lu_solve_factored": (C.c_int, [_vp, _i32, _vp, _vp, _vp, _vp, _vp]),
     "nodal_dgemm_sub_profile": (C.c_int, [_vp, _vp, _vp, _vp, _i32, _i32, _i32, _i32, _i32, C.POINTER(_f64), _vp]),
     "nodal_lu_batched": (C.c_int, [_vp, _i64, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp,
                                    _i32, _i32, _vp, _vp, _vp, _vp]),

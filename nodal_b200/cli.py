@@ -22,6 +22,9 @@ def make_parser(description, file_help):
     parser.add_argument("--eliminate-sources", choices=("auto", "on", "off"), default="auto",
                         help="with -s: solve R / A / E netlists by eliminating the voltage sources and running "
                              "the AMG-PCG on the reduced system (auto: above the dense-LU fallback size)")
+    parser.add_argument("--schur", action="store_true",
+                        help="with -s: solve netlists with op-amps and dependent sources through the Schur "
+                             "complement of the branch rows (AMG on the resistor block, dense LU on the rest)")
     return parser
 
 
@@ -35,6 +38,8 @@ def circuit_options(options):
     mode = getattr(options, "eliminate_sources", "auto")
     if options.sparse and mode != "auto":
         kw["eliminate_sources"] = mode == "on"
+    if options.sparse and getattr(options, "schur", False):
+        kw["schur"] = True
     return kw
 
 

@@ -433,25 +433,26 @@ lu_gemv_sub_kernel(const double* __restrict__ A, int n, int rb, int re, int cb, 
     }
 }
 
-extern "C" int nodal_lu_solve(nodal_ctx* ctx, int32_t n, double* G, const double* rhs, double* x,
-                              int32_t* info_h, void* stream) {
-    NvtxRange nvtx_range("nodal_lu_solve");
-    if (!ctx || n < 0 || !info_h) return NODAL_BAD_ARG;
-    *info_h = 0;
-    if (n == 0) return NODAL_OK;
-    cudaStream_t st = (cudaStream_t)stream;
-    CUDA_TRY(cudaSetDevice(ctx->device));
-    const int sms = ctx->num_sms;
+// Workspace nodal_lu_factor needs in the context arena besides the pivot vector.
+static size_t lu_factor_scratch_bytes(int sms) {
+    return sizeof(int) * 64 + sizeof(PivotCand) * 2 * (size_t)sms + sizeof(double) * (2 * (size_t)sms * LU_NB + 2 * LU_NB) +
+           8192;
+}
+
+static int lu_check_size(nodal_ctx* ctx, int n, const char* what) {
     const int max_rows_per_cta = (226 * 1024 - 4096) / (PANEL_LD * 8) - 1;   // shared-memory limit
-    if ((int64_t)n > (int64_t)sms * max_rows_per_cta) {
-        nodal_set_error("nodal_lu_solve: n=%d exceeds the panel capacity of this build (%d)", n,
-                        sms * max_rows_per_cta);
+    if ((int64_t)n > (int64_t)ctx->num_sms * max_rows_per_cta) {
+        nodal_set_error("%s: n=%d exceeds the panel capacity of this build (%d)", what, n,
+                        ctx->num_sms * max_rows_per_cta);
         return NODAL_BAD_ARG;
     }
-    const size_t need = sizeof(int) * ((size_t)n + 64) + sizeof(PivotCand) * 2 * (size_t)sms +
-                        sizeof(double) * (2 * (size_t)sms * LU_NB + 2 * LU_NB) + 8192;
-    NODAL_TRY(ctx_reserve(ctx, need));
-    int* ipiv = carve<int>(ctx, (size_t)n);
+    return NODAL_OK;
+}
+
+// Factors G in place (P G = L U) on `st`; the scratch is carved from the arena, which the caller has
+// reserved.  Returns NODAL_SINGULAR with *info_h set on an exactly zero pivot.
+static int lu_factor_core(nodal_ctx* ctx, int n, double* G, int* ipiv, int32_t* info_h, cudaStream_t st) {
+    const int sms = ctx->num_sms;
     int* info = carve<int>(ctx, 16);
     PivotCand* cand = carve<PivotCand>(ctx, 2 * (size_t)sms);
     double* candrow = carve<double>(ctx, 2 * (size_t)sms * LU_NB);
@@ -460,12 +461,9 @@ extern "C" int nodal_lu_solve(nodal_ctx* ctx, int32_t n, double* G, const double
     CUDA_TRY(cudaMemsetAsync(info, 0, sizeof(int), st));
 
     const size_t trsm_smem = sizeof(double) * ((size_t)LU_NB * PANEL_LD + (size_t)LU_NB * TRSM_COLS);
-    const size_t trsv_smem = sizeof(double) * ((size_t)LU_NB * PANEL_LD + LU_NB);
     {
         CUDA_TRY(cudaFuncSetAttribute(lu_panel_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 226 * 1024));
         CUDA_TRY(cudaFuncSetAttribute(lu_trsm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)trsm_smem));
-        CUDA_TRY(cudaFuncSetAttribute(lu_trsv_diag_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)trsv_smem));
-        CUDA_TRY(cudaFuncSetAttribute(lu_apply_pivots_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
     }
 
     // Right-looking LU.  Opt-in (NODAL_LU_LOOKAHEAD=1): one panel of look-ahead -- as soon as step k
@@ -566,7 +564,16 @@ extern "C" int nodal_lu_solve(nodal_ctx* ctx, int32_t n, double* G, const double
         *info_h = *info_pinned;
         return NODAL_SINGULAR;
     }
-    // ---- x = U^-1 L^-1 P b
+    return NODAL_OK;
+}
+
+// x = U^-1 L^-1 P rhs with the factors of lu_factor_core; enqueued on `st`.
+static int lu_solve_core(nodal_ctx* ctx, int n, const double* G, const int* ipiv, const double* rhs, double* x,
+                         cudaStream_t st) {
+    const int sms = ctx->num_sms;
+    const size_t trsv_smem = sizeof(double) * ((size_t)LU_NB * PANEL_LD + LU_NB);
+    CUDA_TRY(cudaFuncSetAttribute(lu_trsv_diag_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)trsv_smem));
+    CUDA_TRY(cudaFuncSetAttribute(lu_apply_pivots_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
     const int use_smem = (size_t)n * 8 <= 200 * 1024;
     lu_apply_pivots_kernel<<<1, 256, use_smem ? (size_t)n * 8 : 0, st>>>(rhs, x, ipiv, n, use_smem);
     KERNEL_CHECK();
@@ -589,8 +596,45 @@ extern "C" int nodal_lu_solve(nodal_ctx* ctx, int32_t n, double* G, const double
             KERNEL_CHECK();
         }
     }
+    return NODAL_OK;
+}
+
+extern "C" int nodal_lu_solve(nodal_ctx* ctx, int32_t n, double* G, const double* rhs, double* x,
+                              int32_t* info_h, void* stream) {
+    NvtxRange nvtx_range("nodal_lu_solve");
+    if (!ctx || n < 0 || !info_h) return NODAL_BAD_ARG;
+    *info_h = 0;
+    if (n == 0) return NODAL_OK;
+    cudaStream_t st = (cudaStream_t)stream;
+    CUDA_TRY(cudaSetDevice(ctx->device));
+    NODAL_TRY(lu_check_size(ctx, n, "nodal_lu_solve"));
+    NODAL_TRY(ctx_reserve(ctx, sizeof(int) * (size_t)n + lu_factor_scratch_bytes(ctx->num_sms)));
+    int* ipiv = carve<int>(ctx, (size_t)n);
+    NODAL_TRY(lu_factor_core(ctx, n, G, ipiv, info_h, st));
+    NODAL_TRY(lu_solve_core(ctx, n, G, ipiv, rhs, x, st));
     CUDA_TRY(cudaStreamSynchronize(st));
     return NODAL_OK;
+}
+
+extern "C" int nodal_lu_factor(nodal_ctx* ctx, int32_t n, double* G, int32_t* ipiv, int32_t* info_h, void* stream) {
+    NvtxRange nvtx_range("nodal_lu_factor");
+    if (!ctx || n < 0 || !info_h || (n > 0 && (!G || !ipiv))) return NODAL_BAD_ARG;
+    *info_h = 0;
+    if (n == 0) return NODAL_OK;
+    cudaStream_t st = (cudaStream_t)stream;
+    CUDA_TRY(cudaSetDevice(ctx->device));
+    NODAL_TRY(lu_check_size(ctx, n, "nodal_lu_factor"));
+    NODAL_TRY(ctx_reserve(ctx, lu_factor_scratch_bytes(ctx->num_sms)));
+    return lu_factor_core(ctx, n, G, ipiv, info_h, st);
+}
+
+extern "C" int nodal_lu_solve_factored(nodal_ctx* ctx, int32_t n, const double* LU, const int32_t* ipiv,
+                                       const double* rhs, double* x, void* stream) {
+    NvtxRange nvtx_range("nodal_lu_solve_factored");
+    if (!ctx || n < 0 || (n > 0 && (!LU || !ipiv || !rhs || !x))) return NODAL_BAD_ARG;
+    if (n == 0) return NODAL_OK;
+    CUDA_TRY(cudaSetDevice(ctx->device));
+    return lu_solve_core(ctx, n, LU, ipiv, rhs, x, (cudaStream_t)stream);
 }
 
 // Measurement aid (SURVEY.md section 8(d): "measure an FP64 GEMM-shaped peak on the box"): the

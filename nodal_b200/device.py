@@ -487,6 +487,78 @@ class Device:
                                                   self.stream()), "nodal_source_residual")
         return sums[0], sums[1]
 
+    # ------------------------------------------------------------ Schur complement of the branch rows
+    def schur_split(self, G: DeviceCSR, kcl):
+        """(L, B) of the sorted MNA matrix G (csrc/schur.cu): L the DeviceCSR of the node-node block,
+        B a dict of device tensors ptr (kcl + 1), col (branch index), val: the node rows' branch entries."""
+        torch = self.torch
+        p = self.ptr
+        l_ptr, b_ptr = self.empty(kcl + 1, torch.int32), self.empty(kcl + 1, torch.int32)
+        nnz = (C.c_int64 * 2)()
+        _lib.check(self.lib.nodal_schur_split_scan(self.ctx, kcl, p(G.indptr), p(G.indices), p(l_ptr), p(b_ptr), nnz,
+                                                   self.stream()), "nodal_schur_split_scan")
+        nl, nb = int(nnz[0]), int(nnz[1])
+        l_idx, l_val = self.empty(max(1, nl), torch.int32)[:nl], self.empty(max(1, nl), torch.float64)[:nl]
+        b_col, b_val = self.empty(max(1, nb), torch.int32)[:nb], self.empty(max(1, nb), torch.float64)[:nb]
+        _lib.check(self.lib.nodal_schur_split_place(self.ctx, kcl, p(G.indptr), p(G.indices), p(G.data), p(l_ptr),
+                                                    p(l_idx), p(l_val), p(b_ptr), p(b_col), p(b_val), self.stream()),
+                   "nodal_schur_split_place")
+        return DeviceCSR(kcl, l_ptr, l_idx, l_val), dict(ptr=b_ptr, col=b_col, val=b_val)
+
+    def schur_rhs_batch(self, kcl, j0, K, B):
+        """(K, kcl) device tensor: the branch columns j0 .. j0 + K - 1 of B."""
+        rhs = self.empty(max(2, K * kcl), self.torch.float64)[: K * kcl].view(K, kcl)
+        p = self.ptr
+        _lib.check(self.lib.nodal_schur_rhs_batch(self.ctx, kcl, j0, K, p(B["ptr"]), p(B["col"]), p(B["val"]), p(rhs),
+                                                  self.stream()), "nodal_schur_rhs_batch")
+        return rhs
+
+    def schur_columns(self, G: DeviceCSR, kcl, j0, Z, S):
+        """S[:, j0 : j0 + K] = D - C Z (S: the m x m device tensor, Z: (K, kcl))."""
+        m, K = int(S.shape[0]), int(Z.shape[0])
+        p = self.ptr
+        _lib.check(self.lib.nodal_schur_columns(self.ctx, kcl, m, j0, K, p(G.indptr), p(G.indices), p(G.data),
+                                                p(Z.contiguous()), p(S), self.stream()), "nodal_schur_columns")
+
+    def schur_branch_rhs(self, G: DeviceCSR, kcl, r, t):
+        """r[kcl:] - C t (m entries)."""
+        m = G.n - kcl
+        out = self.empty(max(1, m), self.torch.float64)[:m]
+        p = self.ptr
+        _lib.check(self.lib.nodal_schur_branch_rhs(self.ctx, kcl, m, p(G.indptr), p(G.indices), p(G.data), p(r), p(t),
+                                                   p(out), self.stream()), "nodal_schur_branch_rhs")
+        return out
+
+    def schur_node_rhs(self, kcl, B, r, xb):
+        """r[:kcl] - B xb (kcl entries)."""
+        out = self.empty(max(1, kcl), self.torch.float64)[:kcl]
+        p = self.ptr
+        _lib.check(self.lib.nodal_schur_node_rhs(self.ctx, kcl, p(B["ptr"]), p(B["col"]), p(B["val"]), p(r), p(xb),
+                                                 p(out), self.stream()), "nodal_schur_node_rhs")
+        return out
+
+    def schur_residual(self, G: DeviceCSR, rhs, x, r):
+        """r = rhs - G x in place; returns (sum r^2, sum rhs^2)."""
+        sums = (C.c_double * 2)()
+        p = self.ptr
+        _lib.check(self.lib.nodal_schur_residual(self.ctx, G.n, p(G.indptr), p(G.indices), p(G.data), p(rhs), p(x),
+                                                 p(r), sums, self.stream()), "nodal_schur_residual")
+        return sums[0], sums[1]
+
+    def schur_add(self, x, d):
+        """x += d (same length)."""
+        _lib.check(self.lib.nodal_schur_add(self.ctx, int(d.numel()), self.ptr(x), self.ptr(d), self.stream()),
+                   "nodal_schur_add")
+
+    def r_grounded(self, dtab, ncomp, kcl):
+        """True when every node reaches ground through the R rows of the device table alone."""
+        rt, nr = self.select_type(dtab, ncomp, K.T_R)
+        count, reached = C.c_int32(0), C.c_int32(0)
+        _lib.check(self.lib.nodal_connected_components(self.ctx, nr, self.ptr(rt["a"]), self.ptr(rt["b"]), kcl, None,
+                                                       C.byref(count), C.byref(reached), self.stream()),
+                   "nodal_connected_components")
+        return reached.value == kcl + 1
+
     def amg(self, csr: DeviceCSR, **params):
         """Aggregation-AMG hierarchy for an SPD DeviceCSR (csrc/amg.cu); see DeviceAMG."""
         return DeviceAMG(self, csr, **params)
@@ -520,6 +592,24 @@ class Device:
         st = self.lib.nodal_lu_solve(self.ctx, n, p(G), p(rhs), p(x), C.byref(info), self.stream())
         _lib.check(st, "nodal_lu_solve", allowed=(_lib.OK, _lib.SINGULAR))
         return x, dict(solver="lu", status=st, info=info.value)
+
+    def lu_factor(self, G):
+        """P G = L U in place (G: n x n row-major device tensor); returns (ipiv, info dict)."""
+        n = int(G.shape[0])
+        ipiv = self.empty(max(1, n), self.torch.int32)[:n]
+        info = C.c_int32(0)
+        st = self.lib.nodal_lu_factor(self.ctx, n, self.ptr(G), self.ptr(ipiv), C.byref(info), self.stream())
+        _lib.check(st, "nodal_lu_factor", allowed=(_lib.OK, _lib.SINGULAR))
+        return ipiv, dict(solver="lu", status=st, info=info.value)
+
+    def lu_solve_factored(self, LU, ipiv, rhs):
+        """x for one rhs with the factors of lu_factor."""
+        n = int(LU.shape[0])
+        x = self.empty(max(1, n), self.torch.float64)[:n]
+        p = self.ptr
+        _lib.check(self.lib.nodal_lu_solve_factored(self.ctx, n, p(LU), p(ipiv), p(rhs), p(x), self.stream()),
+                   "nodal_lu_solve_factored")
+        return x
 
     def lu_batched(self, table: ComponentTable, values, layout="aos"):
         """Batched small-system solve.  layout "aos": values (batch, ncomp) -> x (batch, n);

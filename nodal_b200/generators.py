@@ -271,6 +271,120 @@ class _PadNames(Mapping):
         return (f"v{k}" for k in range(self._count))
 
 
+# --------------------------------------------------------------------------- amplifiers on a sheet
+def amplifier_grid(N, stages, seed=0, pitch=None, dependents=4, resistance=1.0, vdd=1.0):
+    """Op-amp stages coupled through a resistive N x N sheet (the workload of the Schur-complement
+    solve, nodal_b200/schur.py): the resistors of grid2d's loop order between nodes "n{x}_{y}", a load
+    resistor "l{k}" to ground "g" on every node (row-major), supply pads every `pitch` nodes (default
+    N // 8) as an E source "v{k}" of `vdd` behind a series resistor "rs{k}" (node "s{k}"), then per stage
+    p a non-inverting amplifier: OPMODEL "q{p}" reading a random sheet node, gain 1 + rf/rg <= 100
+    ("rg{p}" to ground), driving another random sheet node through "rd{p}" from its output "o{p}";
+    then `dependents` each of VCVS "dv{k}", CCVS "hv{k}" (driving "xv{k}" / "xh{k}", tied to the sheet
+    by "rx{k}" / "rh{k}") and CCCS "fv{k}" (into a sheet node), the current-controlled ones driven by
+    sheet resistors.  Every node reaches ground through resistors.  Component order, numbering,
+    anomnum and branches are those of the csv path of the same rows (OPMODEL rows expand after all
+    others, as ri, ro, vcvs, rf)."""
+    N, stages, dependents = int(N), int(stages), int(dependents)
+    pitch = max(1, N // 8) if pitch is None else int(pitch)
+    if N < 2 or stages < 0 or dependents < 0 or pitch < 1:
+        raise ValueError("amplifier_grid needs N >= 2, stages >= 0, dependents >= 0 and pitch >= 1")
+    rng = np.random.default_rng(seed)
+    sites = N * N
+    sid = np.arange(sites, dtype=np.int64)
+    x, y = sid // N, sid % N
+    has = np.stack([x + 1 < N, y + 1 < N], axis=1)
+    nb = np.stack([sid + N, sid + 1], axis=1)
+    ra = np.repeat(sid, 2).reshape(sites, 2)[has]
+    rb = nb[has]
+    m_r = len(ra)
+    gid = sites
+    extra_names = []                                   # node ids gid + 1, ... of the named nodes
+
+    def node(name):
+        extra_names.append(name)
+        return gid + len(extra_names)
+
+    pads = sid[(x % pitch == 0) & (y % pitch == 0)]
+    # (name, type, value, a, b, c, d, driver row) of the rows after the sheet and the loads
+    rows = []
+    for k, p in enumerate(pads):
+        s = node(f"s{k}")
+        rows.append((f"rs{k}", K.T_R, float(10 ** rng.uniform(-2, -1)), s, int(p), -1, -1, -1))
+        rows.append((f"v{k}", K.T_E, float(vdd), s, gid, -1, -1, -1))
+    amp = []
+    for p in range(stages):
+        pos, drive = (int(v) for v in rng.integers(0, sites, size=2))
+        out, neg = node(f"o{p}"), node(f"m{p}")
+        rf = float(10 ** rng.uniform(2, 4))
+        rg = rf / float(rng.uniform(0.5, 99.0))
+        rows.append((f"rg{p}", K.T_R, rg, neg, gid, -1, -1, -1))
+        rows.append((f"rd{p}", K.T_R, float(10 ** rng.uniform(0, 2)), out, drive, -1, -1, -1))
+        amp.append((p, rf, out, pos, neg))
+    for k in range(dependents):
+        c1, c2, t1, t2, t3 = (int(v) for v in rng.integers(0, sites, size=5))
+        dh, df = (int(v) for v in rng.integers(0, m_r, size=2))
+        xv, xh = node(f"xv{k}"), node(f"xh{k}")
+        rows.append((f"dv{k}", K.T_VCVS, float(rng.uniform(-2, 2)), xv, gid, c1, c2, -1))
+        rows.append((f"rx{k}", K.T_R, float(10 ** rng.uniform(1, 3)), xv, t1, -1, -1, -1))
+        rows.append((f"hv{k}", K.T_CCVS, float(rng.uniform(-2, 2)), xh, gid, int(ra[dh]), int(rb[dh]), dh))
+        rows.append((f"rh{k}", K.T_R, float(10 ** rng.uniform(1, 3)), xh, t2, -1, -1, -1))
+        rows.append((f"fv{k}", K.T_CCCS, float(rng.uniform(-0.5, 0.5)), t3, gid, int(ra[df]), int(rb[df]), df))
+    for p, rf, out, pos, neg in amp:                   # the OPMODEL expansion (nodal.py build_opmodel)
+        inner = node(f"q{p}_internal_node")
+        rows.append((f"q{p}_ri", K.T_R, float(str(K.OPMODEL_RI)), pos, neg, -1, -1, -1))
+        rows.append((f"q{p}_ro", K.T_R, float(str(K.OPMODEL_RO)), inner, out, -1, -1, -1))
+        rows.append((f"q{p}_vcvs", K.T_VCVS, float(str(K.OPMODEL_GAIN)), inner, gid, pos, neg, -1))
+        rows.append((f"q{p}_rf", K.T_R, rf, neg, out, -1, -1, -1))
+    col = lambda k, dt: np.array([r[k] for r in rows], dtype=dt).reshape(-1)   # noqa: E731
+    loads = 10 ** rng.uniform(2, 4, sites)
+    a_id = np.concatenate([ra, sid, col(3, np.int64)])
+    b_id = np.concatenate([rb, np.full(sites, gid), col(4, np.int64)])
+    index, kcl = first_appearance_numbering(a_id, b_id, gid)
+    index = np.append(index, -1).astype(np.int32)      # the id -1 of "no control node" maps to ground
+    type_ = np.concatenate([np.full(m_r + sites, K.T_R, np.uint8), col(1, np.uint8)])
+    value = np.concatenate([np.full(m_r, float(resistance)), loads, col(2, np.float64)])
+    dep = np.isin(type_, (K.T_VCVS, K.T_VCCS, K.T_CCVS, K.T_CCCS))
+    c_id = np.concatenate([np.full(m_r + sites, -1), col(5, np.int64)])
+    d_id = np.concatenate([np.full(m_r + sites, -1), col(6, np.int64)])
+    cc = np.where(dep, index[c_id], K.UNUSED).astype(np.int32)
+    dd = np.where(dep, index[d_id], K.UNUSED).astype(np.int32)
+    drv = np.concatenate([np.full(m_r + sites, -1), col(7, np.int64)]).astype(np.int32)
+    anom = type_ != K.T_R
+    branch = np.full(len(type_), -1, np.int32)
+    be = int(anom.sum())
+    branch[anom] = np.arange(be, dtype=np.int32)
+    table = ComponentTable(type_, value, index[a_id], index[b_id], cc, dd, drv, branch, kcl=kcl, be=be)
+    named = {name: gid + 1 + k for k, name in enumerate(extra_names)}
+
+    def encode(name):
+        if name == "g":
+            return gid
+        if name in named:
+            return named[name]
+        if not name.startswith("n"):
+            return None
+        try:
+            px, py = (int(t) for t in name[1:].split("_"))
+        except ValueError:
+            return None
+        return px * N + py if 0 <= px < N and 0 <= py < N else None
+
+    def decode(nid):
+        return "g" if nid == gid else extra_names[nid - gid - 1] if nid > gid else f"n{nid // N}_{nid % N}"
+
+    tail = [r[0] for r in rows]
+
+    def names(k):
+        k = int(k)
+        return f"r{k}" if k < m_r else f"l{k - m_r}" if k < m_r + sites else tail[k - m_r - sites]
+
+    anom_names = [names(k) for k in np.flatnonzero(anom)]
+    net = TableNetlist(table, _LazyNodeMap(index[:-1], encode, decode, kcl), "g", names=names,
+                       anomnum={name: k for k, name in enumerate(anom_names)})
+    net._currents = anom_names
+    return net
+
+
 # --------------------------------------------------------------------------- sparse random networks
 def random_network(nodes, degree=8, seed=0, decades=2.0, locality=None):
     """Connected random resistive network (north star: "random-network netlists"): `nodes` nodes, a

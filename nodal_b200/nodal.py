@@ -25,6 +25,7 @@ import numpy as np
 from . import constants as c
 from . import models
 from . import dist_sources
+from . import schur
 from . import sources
 from .table import ComponentTable
 
@@ -254,7 +255,9 @@ class Circuit:
     numpy.linalg.solve).  ``sparse=True``: CSR G, Jacobi-PCG for R/A-only
     netlists, restarted GMRES otherwise (replaces scipy spsolve); R/A/E netlists
     whose voltage sources form a forest are solved through the elimination of
-    the sources (``eliminate_sources``, see sources.py).
+    the sources (``eliminate_sources``, see sources.py); ``schur=True`` solves
+    netlists with op-amps and dependent sources through the Schur complement of
+    the branch rows (see schur.py).
 
     Attributes as in the reference: netlist, sparse, G, A, currents.  G and A
     live in HBM; ``G`` is a torch tensor (dense) or a DeviceCSR, and
@@ -274,6 +277,7 @@ class Circuit:
     # ---- assembly ---------------------------------------------------------------
     def build_model(self):
         from .device import Device
+        self._schur = schur.check_option(self.options, self.sparse, self.options.get("distributed"))
         table, currents = self.netlist.table_and_currents()
         table.validate()
         self.table = table
@@ -288,10 +292,11 @@ class Circuit:
             # csr_order="first_touch": G's columns in the order the reference's G.tocsr() has before its
             # solve (nodal.py:396-397); the solve then works on the sorted form, as spsolve sorts in place
             order = self.options.get("csr_order", "sorted")
-            # tables the source elimination will take keep their device columns for it (sources.py)
+            # tables the source elimination or the Schur solve will take keep their device columns for
+            # it (sources.py, schur.py)
             self._eliminate = sources.check_option(self.options, table)
             limit = int(self.options.get("dense_fallback_max_rows", 32768))
-            if sources.skip_reason(table, self._eliminate, limit) == "":
+            if sources.skip_reason(table, self._eliminate, limit) == "" or self._schur:
                 self._dtab = dev.upload_table(table)
             G, A = dev.assemble_csr(table, dtab=self._dtab, order=order)
             if order != "sorted":
@@ -505,7 +510,13 @@ class Circuit:
             x, info = sources.solve(self) if self.sparse and self._dist is None else (None, None)
         if x is None:
             skipped = info
-            x, info = self._device_solve(self.A)
+            # then, when requested and the netlist qualifies, the Schur complement of the branch rows
+            x, info = schur.solve(self) if self.sparse and self._dist is None else (None, None)
+            if x is None:
+                declined = info
+                x, info = self._device_solve(self.A)
+                if declined is not None:
+                    info["schur"] = declined
             if skipped is not None:
                 info["reduction"] = skipped
         if self.sparse:
