@@ -263,6 +263,36 @@ int nodal_source_residual(nodal_ctx* ctx, int32_t n, int64_t nnz_full, int32_t r
                           const int32_t* indptr, const int32_t* indices, const double* data, const double* x,
                           double* sums_h, void* stream);
 
+/* Tables with E rows and dependent branch rows (nodal_b200/source_schur.py; the rules are in
+ * csrc/sources_core.cuh).  The forest is built on the E-only table; the reduced system has the mn
+ * reduced node rows, then one row per dependent branch (nr rows in all).
+ * nodal_source_dep_map: d_map (be) = index of each branch among the dependent ones in branch order,
+ * -1 for the others; info_h (host, 2): [0] dependent branches, [1] branches not owned by exactly one
+ * component.
+ * nodal_source_dep_check: *count_h = VCVS / VCCS / CCVS rows whose two output leads share rep_row.
+ * nodal_source_dep_scan / _emit: the keyed triples (row << colbits | col, col == nr for the rhs) of the
+ * reduced system's dependent entries, from the rows of the full sorted MNA matrix (n rows, rhs) in row
+ * and CSR order: pos (n) receives each row's first slot, *count_h the number of triples.
+ * nodal_source_expand_dep: nodal_source_expand (same kernels, same order) with x[kcl + b] =
+ * y[mn + d_map[b]] seeded for the dependent branches before the first G x (n = kcl + be). */
+int nodal_source_dep_map(nodal_ctx* ctx, int64_t ncomp, const uint8_t* type, const int32_t* branch, int32_t be,
+                         int32_t* d_map, int64_t* info_h, void* stream);
+int nodal_source_dep_check(nodal_ctx* ctx, int64_t ncomp, const uint8_t* type, const int32_t* a, const int32_t* b,
+                           int32_t kcl, const int32_t* rep_row, int64_t* count_h, void* stream);
+int nodal_source_dep_scan(nodal_ctx* ctx, int32_t n, int32_t kcl, const int32_t* indptr, const int32_t* indices,
+                          const double* data, const double* rhs, const int32_t* rep_row, const double* offset,
+                          const int32_t* d_map, int32_t mn, int32_t nr, uint32_t* pos, int64_t* count_h, void* stream);
+int nodal_source_dep_emit(nodal_ctx* ctx, int32_t n, int32_t kcl, const int32_t* indptr, const int32_t* indices,
+                          const double* data, const double* rhs, const int32_t* rep_row, const double* offset,
+                          const int32_t* d_map, int32_t mn, int32_t nr, int32_t colbits, const uint32_t* pos,
+                          uint64_t* keys, double* vals, void* stream);
+int nodal_source_expand_dep(nodal_ctx* ctx, int32_t kcl, int32_t n, int32_t nsrc, const int32_t* erow,
+                            const int32_t* a, const int32_t* b, const int32_t* branch, const int32_t* adj_ptr,
+                            const int32_t* adj_row, const int32_t* rep_row, const double* offset,
+                            const int32_t* depth, int32_t max_depth, int32_t be, const int32_t* d_map, int32_t mn,
+                            const double* y, const double* rhs, int64_t nnz, const int32_t* indptr,
+                            const int32_t* indices, const double* data, double* x, double* relres_h, void* stream);
+
 /* ---------------------------------------------------------------- Schur complement of the branch rows
  * csrc/schur.cu (rules in csrc/schur_core.cuh).  G is the sorted MNA matrix of n = kcl + m rows
  * (indptr / indices / data), G = [[L, B], [C, D]] with L the kcl x kcl resistor Laplacian.

@@ -95,6 +95,13 @@ SIGNATURES = {
                                          _vp, _vp, C.POINTER(_i64), _vp]),
     "nodal_source_currents": (C.c_int, [_vp, _i32, _i32] + [_vp] * 7 + [_i32, _i64, _vp, _vp, _vp, _vp, _vp]),
     "nodal_source_residual": (C.c_int, [_vp, _i32, _i64, _i32, _vp, _i64, _vp, _vp, _vp, _vp, C.POINTER(_f64), _vp]),
+    "nodal_source_dep_map": (C.c_int, [_vp, _i64, _vp, _vp, _i32, _vp, C.POINTER(_i64), _vp]),
+    "nodal_source_dep_check": (C.c_int, [_vp, _i64, _vp, _vp, _vp, _i32, _vp, C.POINTER(_i64), _vp]),
+    "nodal_source_dep_scan": (C.c_int, [_vp, _i32, _i32] + [_vp] * 7 + [_i32, _i32, _vp, C.POINTER(_i64), _vp]),
+    "nodal_source_dep_emit": (C.c_int, [_vp, _i32, _i32] + [_vp] * 7 + [_i32, _i32, _i32, _vp, _vp, _vp, _vp]),
+    "nodal_source_expand_dep": (C.c_int, [_vp, _i32, _i32, _i32] + [_vp] * 9 + [_i32, _i32, _vp, _i32, _vp, _vp, _i64,
+                                                                                 _vp, _vp, _vp, _vp, C.POINTER(_f64),
+                                                                                 _vp]),
     "nodal_dist_amg_pcg": (C.c_int, [_vp, _vp, _i32, _vp, _i64, _vp, _vp, _vp, _vp, _vp, C.POINTER(_f64), _f64,
                                      _i32, C.POINTER(_i32), C.POINTER(_f64), C.POINTER(_f64), _vp]),
 }

@@ -21,10 +21,14 @@ def make_parser(description, file_help):
                              "iterative solver returned")
     parser.add_argument("--eliminate-sources", choices=("auto", "on", "off"), default="auto",
                         help="with -s: solve R / A / E netlists by eliminating the voltage sources and running "
-                             "the AMG-PCG on the reduced system (auto: above the dense-LU fallback size)")
+                             "the AMG-PCG on the reduced system (auto: above the dense-LU fallback size); "
+                             "'on' with --schur: eliminate the voltage sources of a netlist with op-amps and "
+                             "dependent sources, then solve the rest through the Schur complement")
     parser.add_argument("--schur", action="store_true",
                         help="with -s: solve netlists with op-amps and dependent sources through the Schur "
-                             "complement of the branch rows (AMG on the resistor block, dense LU on the rest)")
+                             "complement of the branch rows (AMG on the resistor block, dense LU on the rest); "
+                             "with --eliminate-sources on, of the rows left after the voltage sources are "
+                             "eliminated")
     return parser
 
 

@@ -18,6 +18,11 @@
 //   nodal_source_potentials / _tree_rows / _currents / _residual
 //                              the same expansion in stages for a rank of the row-partitioned solve
 //                              (nodal_b200/dist_sources.py), launching the same kernels.
+//   nodal_source_dep_map / _dep_check / _dep_scan / _dep_emit / nodal_source_expand_dep
+//                              tables with E rows and dependent branch rows (nodal_b200/source_schur.py):
+//                              the dependent branches' numbering, the check of their output leads
+//                              against the forest, the keyed triples of the reduced system's dependent
+//                              entries, and the expansion with the dependent currents seeded.
 //
 // Nothing accumulates floating-point values with atomics: results are bitwise reproducible.
 #include <algorithm>
@@ -414,14 +419,24 @@ src_residual_final_kernel(int nparts, const double* __restrict__ part, double* _
     }
 }
 
-extern "C" int nodal_source_expand(nodal_ctx* ctx, int32_t kcl, int32_t n, int32_t nsrc, const int32_t* erow,
-                                   const int32_t* a, const int32_t* b, const int32_t* branch, const int32_t* adj_ptr,
-                                   const int32_t* adj_row, const int32_t* rep_row, const double* offset,
-                                   const int32_t* depth, int32_t max_depth, const double* y, const double* rhs,
-                                   int64_t nnz, const int32_t* indptr, const int32_t* indices, const double* data,
-                                   double* x, double* relres_h, void* stream) {
-    if (!ctx || kcl < 0 || n < kcl || nsrc < 0 || max_depth < 0 || !relres_h) return NODAL_BAD_ARG;
-    NvtxRange nvtx_range("nodal_source_expand");
+// x[kcl + b] = the dependent current of branch b from the reduced solution (entries mn + d)
+__global__ void __launch_bounds__(ST)
+src_seed_dep_kernel(int32_t kcl, int32_t be, const int32_t* __restrict__ d_map, int32_t mn, const double* __restrict__ y,
+                    double* __restrict__ x) {
+    GRID_STRIDE(k, be) {
+        const int32_t d = d_map[k];
+        if (d >= 0) x[kcl + k] = y[mn + d];
+    }
+}
+
+// d_map null: the expansion of an R / A / E table; else the dependent currents are seeded after the
+// potentials, before the first G x
+static int source_expand_impl(nodal_ctx* ctx, int32_t kcl, int32_t n, int32_t nsrc, const int32_t* erow,
+                              const int32_t* a, const int32_t* b, const int32_t* branch, const int32_t* adj_ptr,
+                              const int32_t* adj_row, const int32_t* rep_row, const double* offset,
+                              const int32_t* depth, int32_t max_depth, int32_t be, const int32_t* d_map, int32_t mn,
+                              const double* y, const double* rhs, int64_t nnz, const int32_t* indptr,
+                              const int32_t* indices, const double* data, double* x, double* relres_h, void* stream) {
     CUDA_TRY(cudaSetDevice(ctx->device));
     cudaStream_t st = (cudaStream_t)stream;
     const int parts = src_grid(ctx, n);
@@ -434,6 +449,10 @@ extern "C" int nodal_source_expand(nodal_ctx* ctx, int32_t kcl, int32_t n, int32
         }
         src_potentials_kernel<<<parts, ST, 0, st>>>(kcl, n, rep_row, offset, y, x);
         KERNEL_CHECK();
+        if (d_map && be > 0) {
+            src_seed_dep_kernel<<<src_grid(ctx, be), ST, 0, st>>>(kcl, be, d_map, mn, y, x);
+            KERNEL_CHECK();
+        }
         NODAL_TRY(csr_spmv_launch(ctx, n, nnz, indptr, indices, data, x, gx, st));
         for (int32_t level = max_depth; level >= 1 && nsrc > 0; --level) {
             src_subtree_level_kernel<<<src_grid(ctx, nsrc), ST, 0, st>>>(nsrc, erow, a, b, branch, kcl, adj_ptr,
@@ -455,6 +474,216 @@ extern "C" int nodal_source_expand(nodal_ctx* ctx, int32_t kcl, int32_t n, int32
     ctx_pool_free(ctx, gx);
     ctx_pool_free(ctx, part);
     return rc;
+}
+
+extern "C" int nodal_source_expand(nodal_ctx* ctx, int32_t kcl, int32_t n, int32_t nsrc, const int32_t* erow,
+                                   const int32_t* a, const int32_t* b, const int32_t* branch, const int32_t* adj_ptr,
+                                   const int32_t* adj_row, const int32_t* rep_row, const double* offset,
+                                   const int32_t* depth, int32_t max_depth, const double* y, const double* rhs,
+                                   int64_t nnz, const int32_t* indptr, const int32_t* indices, const double* data,
+                                   double* x, double* relres_h, void* stream) {
+    if (!ctx || kcl < 0 || n < kcl || nsrc < 0 || max_depth < 0 || !relres_h) return NODAL_BAD_ARG;
+    NvtxRange nvtx_range("nodal_source_expand");
+    return source_expand_impl(ctx, kcl, n, nsrc, erow, a, b, branch, adj_ptr, adj_row, rep_row, offset, depth,
+                              max_depth, 0, nullptr, 0, y, rhs, nnz, indptr, indices, data, x, relres_h, stream);
+}
+
+extern "C" int nodal_source_expand_dep(nodal_ctx* ctx, int32_t kcl, int32_t n, int32_t nsrc, const int32_t* erow,
+                                       const int32_t* a, const int32_t* b, const int32_t* branch,
+                                       const int32_t* adj_ptr, const int32_t* adj_row, const int32_t* rep_row,
+                                       const double* offset, const int32_t* depth, int32_t max_depth, int32_t be,
+                                       const int32_t* d_map, int32_t mn, const double* y, const double* rhs,
+                                       int64_t nnz, const int32_t* indptr, const int32_t* indices, const double* data,
+                                       double* x, double* relres_h, void* stream) {
+    if (!ctx || kcl < 0 || n < kcl || nsrc < 0 || max_depth < 0 || be < 0 || kcl + (int64_t)be != n || mn < 0 ||
+        (be > 0 && !d_map) || !relres_h)
+        return NODAL_BAD_ARG;
+    NvtxRange nvtx_range("nodal_source_expand_dep");
+    return source_expand_impl(ctx, kcl, n, nsrc, erow, a, b, branch, adj_ptr, adj_row, rep_row, offset, depth,
+                              max_depth, be, d_map, mn, y, rhs, nnz, indptr, indices, data, x, relres_h, stream);
+}
+
+// ---------------------------------------------------------------- E rows plus dependent branch rows
+// branch use counts (integer atomics) and the flags of the branches a dependent source owns
+__global__ void __launch_bounds__(ST)
+src_dep_use_kernel(int64_t ncomp, const uint8_t* __restrict__ type, const int32_t* __restrict__ branch, int32_t be,
+                   u32* __restrict__ used, u32* __restrict__ dep) {
+    GRID_STRIDE(i, ncomp) {
+        const int32_t br = branch[i];
+        if (br < 0 || br >= be) continue;
+        atomicAdd(&used[br], 1u);
+        const int t = type[i];
+        if (t >= NODAL_T_VCVS && t <= NODAL_T_CCCS) dep[br] = 1u;
+    }
+}
+
+// d_map holds the exclusive scan of the flags on entry; counts[1] += branches not used exactly once
+__global__ void __launch_bounds__(ST)
+src_dep_number_kernel(int32_t be, const u32* __restrict__ used, const u32* __restrict__ dep, int32_t* __restrict__ d_map,
+                      u32* __restrict__ counts) {
+    u32 bad = 0;
+    GRID_STRIDE(k, be) {
+        if (!dep[k]) d_map[k] = -1;
+        bad += used[k] != 1u;
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) bad += __shfl_xor_sync(0xffffffffu, bad, o);
+    if ((threadIdx.x & 31) == 0 && bad) atomicAdd(&counts[1], bad);
+}
+
+__global__ void __launch_bounds__(ST)
+src_dep_check_kernel(int64_t ncomp, const uint8_t* __restrict__ type, const int32_t* __restrict__ a,
+                     const int32_t* __restrict__ b, int32_t kcl, const int32_t* __restrict__ rep_row,
+                     u32* __restrict__ count) {
+    u32 c = 0;
+    GRID_STRIDE(i, ncomp) c += src_dep_collapsed(type[i], a[i], b[i], kcl, rep_row) ? 1u : 0u;
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) c += __shfl_xor_sync(0xffffffffu, c, o);
+    if ((threadIdx.x & 31) == 0 && c) atomicAdd(count, c);
+}
+
+struct DepCount {
+    u32 n = 0;
+    __device__ void operator()(int32_t, int32_t, double) { ++n; }
+};
+
+struct DepKeys {
+    u64* keys;
+    double* vals;
+    int32_t colbits;
+    int64_t p;
+    __device__ void operator()(int32_t row, int32_t col, double v) {
+        keys[p] = ((u64)(u32)row << colbits) | (u64)(u32)col;
+        vals[p] = v;
+        ++p;
+    }
+};
+
+__global__ void __launch_bounds__(ST)
+src_dep_count_kernel(int32_t n, int32_t kcl, const int32_t* __restrict__ indptr, const int32_t* __restrict__ indices,
+                     const double* __restrict__ data, const double* __restrict__ rhs,
+                     const int32_t* __restrict__ rep_row, const double* __restrict__ offset,
+                     const int32_t* __restrict__ d_map, int32_t mn, int32_t nr, u32* __restrict__ pos) {
+    GRID_STRIDE(i, n) {
+        DepCount c;
+        src_dep_row((int32_t)i, indptr, indices, data, rhs, kcl, rep_row, offset, d_map, mn, nr, c);
+        pos[i] = c.n;
+    }
+}
+
+__global__ void __launch_bounds__(ST)
+src_dep_emit_kernel(int32_t n, int32_t kcl, const int32_t* __restrict__ indptr, const int32_t* __restrict__ indices,
+                    const double* __restrict__ data, const double* __restrict__ rhs, const int32_t* __restrict__ rep_row,
+                    const double* __restrict__ offset, const int32_t* __restrict__ d_map, int32_t mn, int32_t nr,
+                    int32_t colbits, const u32* __restrict__ pos, u64* __restrict__ keys, double* __restrict__ vals) {
+    GRID_STRIDE(i, n) {
+        DepKeys k{keys, vals, colbits, (int64_t)pos[i]};
+        src_dep_row((int32_t)i, indptr, indices, data, rhs, kcl, rep_row, offset, d_map, mn, nr, k);
+    }
+}
+
+extern "C" int nodal_source_dep_map(nodal_ctx* ctx, int64_t ncomp, const uint8_t* type, const int32_t* branch,
+                                    int32_t be, int32_t* d_map, int64_t* info_h, void* stream) {
+    if (!ctx || ncomp < 0 || be < 0 || !info_h || ncomp >= ((int64_t)1 << 32)) return NODAL_BAD_ARG;
+    info_h[0] = info_h[1] = 0;
+    if (be == 0) return NODAL_OK;
+    NvtxRange nvtx_range("nodal_source_dep_map");
+    CUDA_TRY(cudaSetDevice(ctx->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    NODAL_TRY(ctx_reserve(ctx, scan_scratch_bytes(be) + 4096));
+    u32* counts = carve<u32>(ctx, 16);
+    if (!counts) return NODAL_CUDA_ERROR;
+    u32* used = static_cast<u32*>(ctx_pool_alloc(ctx, sizeof(u32) * (size_t)be));
+    u32* dep = static_cast<u32*>(ctx_pool_alloc(ctx, sizeof(u32) * (size_t)be));
+    auto run = [&]() -> int {
+        if (!used || !dep) {
+            nodal_set_error("nodal_source_dep_map: out of device memory");
+            return NODAL_CUDA_ERROR;
+        }
+        CUDA_TRY(cudaMemsetAsync(counts, 0, 16 * sizeof(u32), st));
+        CUDA_TRY(cudaMemsetAsync(used, 0, sizeof(u32) * (size_t)be, st));
+        CUDA_TRY(cudaMemsetAsync(dep, 0, sizeof(u32) * (size_t)be, st));
+        if (ncomp > 0) {
+            src_dep_use_kernel<<<src_grid(ctx, ncomp), ST, 0, st>>>(ncomp, type, branch, be, used, dep);
+            KERNEL_CHECK();
+        }
+        NODAL_TRY(scan_exclusive_u32(ctx, dep, reinterpret_cast<u32*>(d_map), be, counts, st));
+        src_dep_number_kernel<<<src_grid(ctx, be), ST, 0, st>>>(be, used, dep, d_map, counts);
+        KERNEL_CHECK();
+        u32* host = reinterpret_cast<u32*>(ctx->pinned);
+        CUDA_TRY(cudaMemcpyAsync(host, counts, 2 * sizeof(u32), cudaMemcpyDeviceToHost, st));
+        CUDA_TRY(cudaStreamSynchronize(st));
+        info_h[0] = host[0];
+        info_h[1] = host[1];
+        return NODAL_OK;
+    };
+    const int rc = run();
+    ctx_pool_free(ctx, used);
+    ctx_pool_free(ctx, dep);
+    return rc;
+}
+
+extern "C" int nodal_source_dep_check(nodal_ctx* ctx, int64_t ncomp, const uint8_t* type, const int32_t* a,
+                                      const int32_t* b, int32_t kcl, const int32_t* rep_row, int64_t* count_h,
+                                      void* stream) {
+    if (!ctx || ncomp < 0 || kcl < 0 || !count_h) return NODAL_BAD_ARG;
+    *count_h = 0;
+    if (ncomp == 0) return NODAL_OK;
+    CUDA_TRY(cudaSetDevice(ctx->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    NODAL_TRY(ctx_reserve(ctx, 4096));
+    u32* count = carve<u32>(ctx, 16);
+    if (!count) return NODAL_CUDA_ERROR;
+    CUDA_TRY(cudaMemsetAsync(count, 0, sizeof(u32), st));
+    src_dep_check_kernel<<<src_grid(ctx, ncomp), ST, 0, st>>>(ncomp, type, a, b, kcl, rep_row, count);
+    KERNEL_CHECK();
+    u32* host = reinterpret_cast<u32*>(ctx->pinned);
+    CUDA_TRY(cudaMemcpyAsync(host, count, sizeof(u32), cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
+    *count_h = host[0];
+    return NODAL_OK;
+}
+
+extern "C" int nodal_source_dep_scan(nodal_ctx* ctx, int32_t n, int32_t kcl, const int32_t* indptr,
+                                     const int32_t* indices, const double* data, const double* rhs,
+                                     const int32_t* rep_row, const double* offset, const int32_t* d_map, int32_t mn,
+                                     int32_t nr, uint32_t* pos, int64_t* count_h, void* stream) {
+    if (!ctx || n < kcl || kcl < 0 || mn < 0 || nr < mn || !count_h) return NODAL_BAD_ARG;
+    *count_h = 0;
+    if (n == 0) return NODAL_OK;
+    NvtxRange nvtx_range("nodal_source_dep_scan");
+    CUDA_TRY(cudaSetDevice(ctx->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    NODAL_TRY(ctx_reserve(ctx, scan_scratch_bytes(n) + 4096));
+    u32* total = carve<u32>(ctx, 16);
+    if (!total) return NODAL_CUDA_ERROR;
+    src_dep_count_kernel<<<src_grid(ctx, n), ST, 0, st>>>(n, kcl, indptr, indices, data, rhs, rep_row, offset, d_map, mn,
+                                                          nr, pos);
+    KERNEL_CHECK();
+    NODAL_TRY(scan_exclusive_u32(ctx, pos, pos, n, total, st));
+    u32* host = reinterpret_cast<u32*>(ctx->pinned);
+    CUDA_TRY(cudaMemcpyAsync(host, total, sizeof(u32), cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
+    *count_h = host[0];
+    return NODAL_OK;
+}
+
+extern "C" int nodal_source_dep_emit(nodal_ctx* ctx, int32_t n, int32_t kcl, const int32_t* indptr,
+                                     const int32_t* indices, const double* data, const double* rhs,
+                                     const int32_t* rep_row, const double* offset, const int32_t* d_map, int32_t mn,
+                                     int32_t nr, int32_t colbits, const uint32_t* pos, uint64_t* keys, double* vals,
+                                     void* stream) {
+    if (!ctx || n < kcl || kcl < 0 || mn < 0 || nr < mn || colbits < 1 || colbits > 31 ||
+        ((int64_t)nr >> colbits) != 0)
+        return NODAL_BAD_ARG;
+    if (n == 0) return NODAL_OK;
+    NvtxRange nvtx_range("nodal_source_dep_emit");
+    CUDA_TRY(cudaSetDevice(ctx->device));
+    src_dep_emit_kernel<<<src_grid(ctx, n), ST, 0, (cudaStream_t)stream>>>(
+        n, kcl, indptr, indices, data, rhs, rep_row, offset, d_map, mn, nr, colbits, pos, reinterpret_cast<u64*>(keys),
+        vals);
+    KERNEL_CHECK();
+    return NODAL_OK;
 }
 
 // ---------------------------------------------------------------- expansion in stages (row-partitioned)

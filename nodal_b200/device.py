@@ -269,16 +269,19 @@ class Device:
 
     def assemble_csr_raw(self, dtab, ncomp, kcl, n, stride, order="sorted"):
         """The same from device-resident columns (`dtab`: name -> tensor, `ncomp` rows used)."""
-        torch = self.torch
         if order not in ("sorted", "first_touch"):
             raise ValueError("order must be 'sorted' or 'first_touch'")
         keys, vals, cb = self.stamp_coo(dtab, ncomp, kcl, n, stride)
+        return self._csr_from_triples(keys, vals, stride * ncomp, n, cb, 1 if order == "first_touch" else 0)
+
+    def _csr_from_triples(self, keys, vals, nslots, n, cb, order):
+        """(DeviceCSR, rhs) of `nslots` keyed triples (csrc/csr.cu: sort, in-order sums, col == n the rhs)."""
+        torch = self.torch
         rhs = self.empty(max(1, n), torch.float64)[:n]
         nnz = C.c_int64(0)
         p = self.ptr
-        _lib.check(self.lib.nodal_csr_build_ordered(self.ctx, n, stride * ncomp, cb, p(keys), p(vals),
-                                                    1 if order == "first_touch" else 0, p(rhs), C.byref(nnz),
-                                                    self.stream()), "nodal_csr_build")
+        _lib.check(self.lib.nodal_csr_build_ordered(self.ctx, n, nslots, cb, p(keys), p(vals), order, p(rhs),
+                                                    C.byref(nnz), self.stream()), "nodal_csr_build")
         nnz = nnz.value
         indptr = self.empty(n + 1, torch.int32)
         indices = self.empty(max(1, nnz), torch.int32)[:nnz]
@@ -486,6 +489,63 @@ class Device:
                                                   p(rows.indptr), p(rows.indices), p(rows.data), p(x), sums,
                                                   self.stream()), "nodal_source_residual")
         return sums[0], sums[1]
+
+    # ------------------------------------------------------------ E rows plus dependent branch rows
+    def source_dep_map(self, dtab, ncomp, be):
+        """(d_map, dependent branches, branches not owned by exactly one component): d_map (be) numbers
+        the dependent branches in branch order, -1 for the others."""
+        d_map = self.empty(max(1, be), self.torch.int32)
+        info = (C.c_int64 * 2)()
+        _lib.check(self.lib.nodal_source_dep_map(self.ctx, ncomp, self.ptr(dtab["type"]), self.ptr(dtab["branch"]), be,
+                                                 self.ptr(d_map), info, self.stream()), "nodal_source_dep_map")
+        return d_map, int(info[0]), int(info[1])
+
+    def source_dep_check(self, dtab, ncomp, kcl, forest):
+        """Number of VCVS / VCCS / CCVS rows whose output leads lie in one source tree."""
+        count = C.c_int64(0)
+        p = self.ptr
+        _lib.check(self.lib.nodal_source_dep_check(self.ctx, ncomp, p(dtab["type"]), p(dtab["a"]), p(dtab["b"]), kcl,
+                                                   p(forest["rep_row"]), C.byref(count), self.stream()),
+                   "nodal_source_dep_check")
+        return count.value
+
+    def source_dep_assemble(self, red, nred, mn, md, kcl, forest, d_map, G: DeviceCSR, rhs):
+        """(DeviceCSR, rhs) of the reduced system (mn + md rows, sorted columns): the triples of the
+        reduced R / A table's stamp, then those of nodal_source_dep_emit, summed in that order."""
+        torch = self.torch
+        nr = mn + md
+        cb = colbits_for(nr)
+        p = self.ptr
+        pos = self.empty(max(1, G.n), torch.int32)
+        cnt = C.c_int64(0)
+        args = (p(G.indptr), p(G.indices), p(G.data), p(rhs), p(forest["rep_row"]), p(forest["offset"]), p(d_map),
+                mn, nr)
+        _lib.check(self.lib.nodal_source_dep_scan(self.ctx, G.n, kcl, *args, p(pos), C.byref(cnt), self.stream()),
+                   "nodal_source_dep_scan")
+        ns, nd = 4 * nred, cnt.value                     # stride of R rows (A rows need 2)
+        keys = self.empty(max(1, ns + nd), torch.int64)
+        vals = self.empty(max(1, ns + nd), torch.float64)
+        if nred > 0:
+            _lib.check(self.lib.nodal_stamp_coo(self.ctx, nred, p(red["type"]), p(red["value"]), p(red["a"]),
+                                                p(red["b"]), None, None, None, None, mn, nr, 4, cb, p(keys), p(vals),
+                                                self.stream()), "nodal_stamp_coo")
+        _lib.check(self.lib.nodal_source_dep_emit(self.ctx, G.n, kcl, *args, cb, p(pos), p(keys[ns:]), p(vals[ns:]),
+                                                  self.stream()), "nodal_source_dep_emit")
+        return self._csr_from_triples(keys, vals, ns + nd, nr, cb, 0)
+
+    def source_expand_dep(self, etab, kcl, forest, info, d_map, mn, y, csr: DeviceCSR, rhs):
+        """source_expand on a table with dependent branch rows: `etab` the E-only table the forest was
+        built on (with the table's branch numbers), y = [reduced node rows; dependent currents]."""
+        n = csr.n
+        x = self.empty(max(1, n), self.torch.float64)[:n]
+        relres = C.c_double(0.0)
+        p, f = self.ptr, forest
+        _lib.check(self.lib.nodal_source_expand_dep(
+            self.ctx, kcl, n, info["sources"], p(f["erow"]), p(etab["a"]), p(etab["b"]), p(etab["branch"]),
+            p(f["adj_ptr"]), p(f["adj_row"]), p(f["rep_row"]), p(f["offset"]), p(f["depth"]), info["depth"], n - kcl,
+            p(d_map), mn, p(y), p(rhs), csr.nnz, p(csr.indptr), p(csr.indices), p(csr.data), p(x), C.byref(relres),
+            self.stream()), "nodal_source_expand_dep")
+        return x, relres.value
 
     # ------------------------------------------------------------ Schur complement of the branch rows
     def schur_split(self, G: DeviceCSR, kcl):

@@ -272,7 +272,7 @@ class _PadNames(Mapping):
 
 
 # --------------------------------------------------------------------------- amplifiers on a sheet
-def amplifier_grid(N, stages, seed=0, pitch=None, dependents=4, resistance=1.0, vdd=1.0):
+def amplifier_grid(N, stages, seed=0, pitch=None, dependents=4, resistance=1.0, vdd=1.0, ideal_pads=False):
     """Op-amp stages coupled through a resistive N x N sheet (the workload of the Schur-complement
     solve, nodal_b200/schur.py): the resistors of grid2d's loop order between nodes "n{x}_{y}", a load
     resistor "l{k}" to ground "g" on every node (row-major), supply pads every `pitch` nodes (default
@@ -283,7 +283,13 @@ def amplifier_grid(N, stages, seed=0, pitch=None, dependents=4, resistance=1.0, 
     by "rx{k}" / "rh{k}") and CCCS "fv{k}" (into a sheet node), the current-controlled ones driven by
     sheet resistors.  Every node reaches ground through resistors.  Component order, numbering,
     anomnum and branches are those of the csv path of the same rows (OPMODEL rows expand after all
-    others, as ri, ro, vcvs, rf)."""
+    others, as ri, ro, vcvs, rf).
+
+    ideal_pads=True: the sheet is held by ideal pads, as in power_grid -- every pad is an E source
+    "v{k}" of `vdd` from its sheet node straight to ground (no "rs{k}" / "s{k}"), and the load "l{k}"
+    on every node is an A row from ground drawing vdd / (the load resistance).  The sheet then reaches
+    ground through the pads and, through resistors, only by way of the amplifier stages; every pad is a
+    branch row (the workload of nodal_b200/source_schur.py)."""
     N, stages, dependents = int(N), int(stages), int(dependents)
     pitch = max(1, N // 8) if pitch is None else int(pitch)
     if N < 2 or stages < 0 or dependents < 0 or pitch < 1:
@@ -308,6 +314,9 @@ def amplifier_grid(N, stages, seed=0, pitch=None, dependents=4, resistance=1.0, 
     # (name, type, value, a, b, c, d, driver row) of the rows after the sheet and the loads
     rows = []
     for k, p in enumerate(pads):
+        if ideal_pads:
+            rows.append((f"v{k}", K.T_E, float(vdd), int(p), gid, -1, -1, -1))
+            continue
         s = node(f"s{k}")
         rows.append((f"rs{k}", K.T_R, float(10 ** rng.uniform(-2, -1)), s, int(p), -1, -1, -1))
         rows.append((f"v{k}", K.T_E, float(vdd), s, gid, -1, -1, -1))
@@ -337,19 +346,22 @@ def amplifier_grid(N, stages, seed=0, pitch=None, dependents=4, resistance=1.0, 
         rows.append((f"q{p}_rf", K.T_R, rf, neg, out, -1, -1, -1))
     col = lambda k, dt: np.array([r[k] for r in rows], dtype=dt).reshape(-1)   # noqa: E731
     loads = 10 ** rng.uniform(2, 4, sites)
-    a_id = np.concatenate([ra, sid, col(3, np.int64)])
-    b_id = np.concatenate([rb, np.full(sites, gid), col(4, np.int64)])
+    load_a, load_b = (np.full(sites, gid), sid) if ideal_pads else (sid, np.full(sites, gid))
+    a_id = np.concatenate([ra, load_a, col(3, np.int64)])
+    b_id = np.concatenate([rb, load_b, col(4, np.int64)])
     index, kcl = first_appearance_numbering(a_id, b_id, gid)
     index = np.append(index, -1).astype(np.int32)      # the id -1 of "no control node" maps to ground
-    type_ = np.concatenate([np.full(m_r + sites, K.T_R, np.uint8), col(1, np.uint8)])
-    value = np.concatenate([np.full(m_r, float(resistance)), loads, col(2, np.float64)])
+    type_ = np.concatenate([np.full(m_r, K.T_R, np.uint8), np.full(sites, K.T_A if ideal_pads else K.T_R, np.uint8),
+                            col(1, np.uint8)])
+    value = np.concatenate([np.full(m_r, float(resistance)), float(vdd) / loads if ideal_pads else loads,
+                            col(2, np.float64)])
     dep = np.isin(type_, (K.T_VCVS, K.T_VCCS, K.T_CCVS, K.T_CCCS))
     c_id = np.concatenate([np.full(m_r + sites, -1), col(5, np.int64)])
     d_id = np.concatenate([np.full(m_r + sites, -1), col(6, np.int64)])
     cc = np.where(dep, index[c_id], K.UNUSED).astype(np.int32)
     dd = np.where(dep, index[d_id], K.UNUSED).astype(np.int32)
     drv = np.concatenate([np.full(m_r + sites, -1), col(7, np.int64)]).astype(np.int32)
-    anom = type_ != K.T_R
+    anom = (type_ != K.T_R) & (type_ != K.T_A)
     branch = np.full(len(type_), -1, np.int32)
     be = int(anom.sum())
     branch[anom] = np.arange(be, dtype=np.int32)

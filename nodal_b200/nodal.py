@@ -26,6 +26,7 @@ from . import constants as c
 from . import models
 from . import dist_sources
 from . import schur
+from . import source_schur
 from . import sources
 from .table import ComponentTable
 
@@ -257,7 +258,8 @@ class Circuit:
     whose voltage sources form a forest are solved through the elimination of
     the sources (``eliminate_sources``, see sources.py); ``schur=True`` solves
     netlists with op-amps and dependent sources through the Schur complement of
-    the branch rows (see schur.py).
+    the branch rows (see schur.py), and with ``eliminate_sources=True`` it
+    eliminates their voltage sources first (see source_schur.py).
 
     Attributes as in the reference: netlist, sparse, G, A, currents.  G and A
     live in HBM; ``G`` is a torch tensor (dense) or a DeviceCSR, and
@@ -510,6 +512,14 @@ class Circuit:
             x, info = sources.solve(self) if self.sparse and self._dist is None else (None, None)
         if x is None:
             skipped = info
+            # schur=True with eliminate_sources=True on a table with E rows and dependent rows: the
+            # elimination, then the Schur complement of the reduced system (source_schur.py)
+            x, info = source_schur.solve(self) if self.sparse and self._dist is None else (None, None)
+            if x is not None:
+                skipped = None
+            elif info is not None:
+                skipped = info
+        if x is None:
             # then, when requested and the netlist qualifies, the Schur complement of the branch rows
             x, info = schur.solve(self) if self.sparse and self._dist is None else (None, None)
             if x is None:

@@ -11,8 +11,10 @@ Circuit(netlist, sparse=True, eliminate_sources=...):
     "auto"  (default) eliminate when the table holds only R, A and E rows, every R is positive, the
             E rows form a forest and the system has more rows than dense_fallback_max_rows (32 768);
             smaller systems keep the GMRES / dense-LU path
-    True    eliminate at any size (ValueError with dependent sources); a table that does not qualify
-            keeps the existing path, and Solution.stats["reduction"] says why
+    True    eliminate at any size (ValueError with dependent sources, unless schur=True: then
+            source_schur.py eliminates the E rows and solves the rest through the Schur complement);
+            a table that does not qualify keeps the existing path, and Solution.stats["reduction"]
+            says why
     False   the existing path
 """
 from __future__ import annotations
@@ -27,13 +29,15 @@ _RAE = (1 << K.T_R) | (1 << K.T_A) | (1 << K.T_E)
 
 
 def check_option(options, table):
-    """Validate eliminate_sources; True with dependent sources is an error."""
+    """Validate eliminate_sources; True with dependent sources is an error unless schur=True
+    (source_schur.py)."""
     mode = options.get("eliminate_sources", "auto")
     if not (mode is True or mode is False or mode == "auto"):
         raise ValueError(f"eliminate_sources must be 'auto', True or False, got {mode!r}")
-    if mode is True and table.facts()["present"] & ~_RAE:
+    if mode is True and table.facts()["present"] & ~_RAE and options.get("schur") is not True:
         raise ValueError("eliminate_sources=True needs a netlist of R, A and E rows only "
-                         "(dependent sources cannot be eliminated)")
+                         "(dependent sources cannot be eliminated; with schur=True they go through the "
+                         "Schur complement of the reduced system)")
     return mode
 
 
