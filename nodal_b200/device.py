@@ -7,6 +7,7 @@ from __future__ import annotations
 
 import ctypes as C
 import threading
+import time
 
 import numpy as np
 
@@ -206,6 +207,11 @@ class Device:
         self.launches = 0   # kernels-of-ours launch counter is kept by the callers' estimates
 
     # ------------------------------------------------------------ helpers
+    def ms_since(self, t0):
+        """Milliseconds since time.perf_counter() gave t0, once the work queued on the current stream is done."""
+        self.torch.cuda.current_stream(self.dev).synchronize()
+        return (time.perf_counter() - t0) * 1e3
+
     def stream(self):
         return C.c_void_p(self.torch.cuda.current_stream(self.dev).cuda_stream)
 

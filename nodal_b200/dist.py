@@ -38,6 +38,13 @@ def local_component_table(table: ComponentTable, rb: int, re: int) -> ComponentT
                           table.drv[sel], table.branch[sel], kcl=table.kcl, be=table.be)
 
 
+def row_slice(csr, rhs, rb, re):
+    """Rows [rb, re) of a CSR and rhs over all rows: (indptr rebased to 0, global indices, data, rhs slice)."""
+    ip = csr.indptr[rb: re + 1]
+    s, e = int(ip[0]), int(ip[-1])
+    return (ip - ip[0]).contiguous(), csr.indices[s:e], csr.data[s:e], rhs[rb:re]
+
+
 def broadcast_bytes(payload: bytes | None, nbytes: int, src: int = 0, device=None) -> bytes:
     """Rank `src` sends `nbytes` bytes to everyone through torch.distributed (gloo or nccl)."""
     import torch
@@ -91,10 +98,7 @@ class DistPCG:
         dev = self.dev
         rb, re = int(bounds[self.rank]), int(bounds[self.rank + 1])
         csr, rhs = dev.assemble_csr(table_local, dtab=dtab)
-        ip = csr.indptr[rb: re + 1]
-        s, e = int(ip[0]), int(ip[-1])
-        indptr = (ip - ip[0]).contiguous()
-        return indptr, csr.indices[s:e], csr.data[s:e], rhs[rb:re]
+        return row_slice(csr, rhs, rb, re)
 
     AMG_PARAMS = ("passes", "coarse", "omega", "scale", "maxlevels", "rounds", "direct_max", "gather_below", "max_fill")
 
@@ -146,6 +150,25 @@ class DistPCG:
                     host_ms=dict(run=stats[14], graph_teardown=stats[15], buffer_teardown=stats[11],
                                  graph_capture=stats[10]))
         return x, info
+
+
+def amg_then_jacobi(solver, rows, rhs, opts):
+    """(x, info) of the row-partitioned SPD system `rows` (LocalRows) through `solver` (DistPCG): AMG-PCG
+    and, when it does not converge, a Jacobi-PCG retry unless precond="amg"; Jacobi-PCG alone with
+    precond="jacobi".  opts: options.SolveOptions.  A NodalLibraryError is not caught: a rank that
+    fell back alone would leave the others waiting in a collective."""
+    first = None
+    if opts.precond != "jacobi":
+        x, info = solver.solve_amg(rows.n, rows.bounds, rows.indptr, rows.indices, rows.data, rhs,
+                                   rtol=opts.spd_rtol, maxit=opts.maxit, **opts.amg_params)
+        if info["status"] == 0 or opts.precond == "amg":
+            return x, info
+        first = f"dist_amg_pcg status {info['status']}"          # same status on every rank
+    x, info = solver.solve(rows.n, rows.bounds, rows.indptr, rows.indices, rows.data, rhs, rtol=opts.spd_rtol,
+                           maxit=opts.maxit)
+    if first:
+        info["fallback_from_amg"] = first
+    return x, info
 
 
 class LocalRows:
@@ -279,9 +302,7 @@ class GridRunner:
         if self.world > 1:
             dtab, ncomp = dev.select_local(dtab, ncomp, rb, re)
         csr, rhs = dev.assemble_csr_raw(dtab, ncomp, self.table.kcl, self.n, coo_stride(self.table))
-        ip = csr.indptr[rb: re + 1]
-        s, e = int(ip[0]), int(ip[-1])
-        return (ip - ip[0]).contiguous(), csr.indices[s:e], csr.data[s:e], rhs[rb:re]
+        return row_slice(csr, rhs, rb, re)
 
     def assemble_from_host(self):
         """Rows of this rank straight from the HOST table, scalable in the number of ranks: every rank
@@ -300,9 +321,7 @@ class GridRunner:
         rb, re = int(self.bounds[r]), int(self.bounds[r + 1])
         local, ncomp = exchange_rows(dev, share, m * (r + 1) // R - m * r // R, self.bounds, r, R, dev.select_local)
         csr, rhs = dev.assemble_csr_raw(local, ncomp, table.kcl, self.n, coo_stride(table))
-        ip = csr.indptr[rb: re + 1]
-        s, e = int(ip[0]), int(ip[-1])
-        return (ip - ip[0]).contiguous(), csr.indices[s:e], csr.data[s:e], rhs[rb:re]
+        return row_slice(csr, rhs, rb, re)
 
     def step(self, dtab, download=False):
         import time

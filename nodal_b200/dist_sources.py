@@ -35,12 +35,6 @@ from . import sources
 _COLUMNS = ("type", "value", "a", "b", "branch")
 
 
-def applies(table):
-    """R / A / E tables with at least one E row take this path; other tables keep dist.GridRunner."""
-    f = table.facts()
-    return table.has_type(K.T_E) and not f["unknown_type"] and not f["present"] & ~sources._RAE
-
-
 def _allgather(dev, cols, count, world):
     """Every rank's `count` rows of the device columns `cols`, concatenated in rank order.
     Returns (columns, total, counts of the ranks); None columns stay None."""
@@ -69,11 +63,8 @@ def _allgather(dev, cols, count, world):
 
 def _rows_of(dev, csr, rhs, bounds, rank):
     """The rank's rows [rb, re) of a CSR built over all rows: (LocalRows, rhs slice)."""
-    rb, re = int(bounds[rank]), int(bounds[rank + 1])
-    ip = csr.indptr[rb: re + 1]
-    s, e = int(ip[0]), int(ip[-1])
-    rows = ndist.LocalRows(csr.n, bounds, rank, (ip - ip[0]).contiguous(), csr.indices[s:e], csr.data[s:e])
-    return rows, rhs[rb:re]
+    indptr, indices, data, rhs = ndist.row_slice(csr, rhs, int(bounds[rank]), int(bounds[rank + 1]))
+    return ndist.LocalRows(csr.n, bounds, rank, indptr, indices, data), rhs
 
 
 class DistSources:
@@ -81,10 +72,9 @@ class DistSources:
 
     def __init__(self, circuit, dev, table, rank, world):
         from .device import coo_stride
-        mode = sources.check_option(circuit.options, table)
         # one rule at any size: there is no other row-partitioned path for E rows
-        reason = sources.skip_reason(table, True if mode == "auto" else mode, 0)
-        if reason is None:
+        reason = sources.skip_reason(table, True, 0)
+        if circuit.opts.eliminate_sources is False:
             raise NotImplementedError("row-partitioned solve of a netlist with voltage sources needs their "
                                       "elimination (eliminate_sources=False)")
         if reason:
@@ -97,7 +87,7 @@ class DistSources:
         self.stats = {}
         t0 = time.perf_counter()
         self.share = ndist.upload_share(dev, table, _COLUMNS, rank, world)
-        self.stats["upload_ms"] = sources._ms(t0, dev)
+        self.stats["upload_ms"] = dev.ms_since(t0)
         t0 = time.perf_counter()
         self.bounds = ndist.partition_rows(n, world)
         local, cnt = ndist.exchange_rows(dev, self.share, self.nshare, self.bounds, rank, world,
@@ -106,7 +96,7 @@ class DistSources:
         self.G, self.A = _rows_of(dev, csr, rhs, self.bounds, rank)
         del csr, local
         self.nnz_full = self._sum_int(self.G.nnz)
-        self.stats["full_assemble_ms"] = sources._ms(t0, dev)
+        self.stats["full_assemble_ms"] = dev.ms_since(t0)
 
     def _sum_int(self, v):
         if self.world == 1:
@@ -138,7 +128,7 @@ class DistSources:
         dev = self.dev
         t0 = time.perf_counter()
         red, nred = dev.source_reduce(self.share, self.nshare, self.table.kcl, forest)
-        stats["reduce_ms"] = sources._ms(t0, dev)
+        stats["reduce_ms"] = dev.ms_since(t0)
         stats["reduced_components"] = self._sum_int(nred)
         if m == 0:
             stats["assemble_ms"] = 0.0
@@ -148,7 +138,7 @@ class DistSources:
         local, cnt = ndist.exchange_rows(dev, red, nred, bounds, self.rank, self.world, dev.select_local)
         csr, rhs = dev.assemble_csr_raw(local, cnt, m, m, 4)          # stride of R rows (A rows need 2)
         rows, rhs = _rows_of(dev, csr, rhs, bounds, self.rank)
-        stats["assemble_ms"] = sources._ms(t0, dev)
+        stats["assemble_ms"] = dev.ms_since(t0)
         return rows, rhs
 
     def expand(self, info, forest, etab, y):
@@ -177,22 +167,6 @@ class DistSources:
                 rr, bb = rr + float(parts[k, 0]), bb + float(parts[k, 1])
         return float(np.sqrt(rr / bb) if bb > 0.0 else np.sqrt(rr))
 
-    def _reduced_solve(self, rows, rhs):
-        opts = self.circuit.options
-        self.circuit._sparse_solver()                               # validates precond
-        rtol, maxit, pcg = opts.get("rtol", 1e-10), opts.get("maxit"), self.solver
-        first = None
-        if opts.get("precond") != "jacobi":
-            y, info = pcg.solve_amg(rows.n, rows.bounds, rows.indptr, rows.indices, rows.data, rhs, rtol=rtol,
-                                    maxit=maxit, **(opts.get("amg") or {}))
-            if info["status"] == 0 or opts.get("precond") == "amg":
-                return y, info
-            first = f"dist_amg_pcg status {info['status']}"         # same status on every rank
-        y, info = pcg.solve(rows.n, rows.bounds, rows.indptr, rows.indices, rows.data, rhs, rtol=rtol, maxit=maxit)
-        if first:
-            info["fallback_from_amg"] = first
-        return y, info
-
     def solve(self):
         """(x, info): x the whole solution on every rank, info the reduced solve's plus
         info["reduction"] (the single-GPU keys, world and the build's upload_ms / full_assemble_ms)."""
@@ -202,7 +176,7 @@ class DistSources:
         t0 = time.perf_counter()
         finfo, forest, etab = self.forest()
         stats.update(eliminated=False, sources=finfo["sources"], supernodes=finfo["floating_trees"],
-                     grounded_nodes=finfo["grounded_nodes"], forest_ms=sources._ms(t0, dev))
+                     grounded_nodes=finfo["grounded_nodes"], forest_ms=dev.ms_since(t0))
         reason = sources.forest_reason(finfo)
         if reason:
             raise NotImplementedError(f"row-partitioned solve of a netlist with voltage sources: {reason}")
@@ -211,8 +185,8 @@ class DistSources:
         rows, rhs = self.reduced_rows(forest, m, stats)
         if m > 0:
             t0 = time.perf_counter()
-            y_local, info = self._reduced_solve(rows, rhs)
-            stats["solve_ms"] = sources._ms(t0, dev)
+            y_local, info = ndist.amg_then_jacobi(self.solver, rows, rhs, self.circuit.opts)
+            stats["solve_ms"] = dev.ms_since(t0)
             y, _, _ = _allgather(dev, dict(y=y_local), int(y_local.numel()), self.world)
             y = y["y"]
             del rows, rhs
@@ -222,8 +196,8 @@ class DistSources:
             stats["solve_ms"] = 0.0
         t0 = time.perf_counter()
         x = self.expand(finfo, forest, etab, y)
-        stats["expand_ms"] = sources._ms(t0, dev)
+        stats["expand_ms"] = dev.ms_since(t0)
         t0 = time.perf_counter()
         stats["relres_full"] = self.relres(x)
-        stats["relres_ms"] = sources._ms(t0, dev)
+        stats["relres_ms"] = dev.ms_since(t0)
         return x, dict(info, reduction=stats)

@@ -24,7 +24,9 @@ import numpy as np
 
 from . import constants as c
 from . import models
+from . import dist as ndist
 from . import dist_sources
+from . import options as solve_options
 from . import schur
 from . import source_schur
 from . import sources
@@ -253,13 +255,16 @@ class Circuit:
     """Builds and solves the MNA system  G e = A  of a Netlist on the GPU.
 
     ``sparse=False``: dense G, blocked FP64 LU with partial pivoting (replaces
-    numpy.linalg.solve).  ``sparse=True``: CSR G, Jacobi-PCG for R/A-only
-    netlists, restarted GMRES otherwise (replaces scipy spsolve); R/A/E netlists
-    whose voltage sources form a forest are solved through the elimination of
-    the sources (``eliminate_sources``, see sources.py); ``schur=True`` solves
-    netlists with op-amps and dependent sources through the Schur complement of
-    the branch rows (see schur.py), and with ``eliminate_sources=True`` it
-    eliminates their voltage sources first (see source_schur.py).
+    numpy.linalg.solve).  ``sparse=True``: CSR G (replaces scipy spsolve); on one
+    GPU the exact paths asked for run in this order, the first that qualifies
+    solves (options.plan, see solve() for what the others report): the
+    elimination of the voltage sources (sources.py), with ``schur=True,
+    eliminate_sources=True`` the elimination then the Schur complement
+    (source_schur.py), with ``schur=True`` the Schur complement of the branch
+    rows (schur.py); then PCG for R/A netlists, restarted GMRES otherwise.
+    ``distributed=True``: dist_sources.py for R/A/E netlists, else dist.GridRunner.
+    The options are parsed once (``circuit.opts``); ``circuit.options`` is the
+    dict the caller passed.
 
     Attributes as in the reference: netlist, sparse, G, A, currents.  G and A
     live in HBM; ``G`` is a torch tensor (dense) or a DeviceCSR, and
@@ -279,32 +284,32 @@ class Circuit:
     # ---- assembly ---------------------------------------------------------------
     def build_model(self):
         from .device import Device
-        self._schur = schur.check_option(self.options, self.sparse, self.options.get("distributed"))
         table, currents = self.netlist.table_and_currents()
+        self.opts = opts = solve_options.parse(self.options, self.sparse, table)
         table.validate()
         self.table = table
-        dev = Device.get(self.options.get("device"))
+        dev = Device.get(opts.device)
         self._dev = dev
         self._dist = None
         self._dsrc = None
         self._dtab = None
-        if self.options.get("distributed"):
+        self._G_sorted = None
+        self._plan = []
+        if opts.distributed:
             G, A = self._build_distributed(dev, table)
         elif self.sparse:
+            self._plan = solve_options.plan(table, opts)
+            # the paths left after the host checks read the table's device columns (sources.py, schur.py,
+            # source_schur.py)
+            if any(not step.reason for step in self._plan):
+                self._dtab = dev.upload_table(table)
             # csr_order="first_touch": G's columns in the order the reference's G.tocsr() has before its
             # solve (nodal.py:396-397); the solve then works on the sorted form, as spsolve sorts in place
-            order = self.options.get("csr_order", "sorted")
-            # tables the source elimination or the Schur solve will take keep their device columns for
-            # it (sources.py, schur.py)
-            self._eliminate = sources.check_option(self.options, table)
-            limit = int(self.options.get("dense_fallback_max_rows", 32768))
-            if sources.skip_reason(table, self._eliminate, limit) == "" or self._schur:
-                self._dtab = dev.upload_table(table)
-            G, A = dev.assemble_csr(table, dtab=self._dtab, order=order)
-            if order != "sorted":
+            G, A = dev.assemble_csr(table, dtab=self._dtab, order=opts.csr_order)
+            if opts.csr_order != "sorted":
                 self._G_sorted = dev.assemble_csr(table)[0]
         else:
-            G, A = dev.assemble_dense(table, atomic=bool(self.options.get("atomic_stamp", False)))
+            G, A = dev.assemble_dense(table, atomic=bool(opts.atomic_stamp))
         logging.debug(f"currents={currents}")
         return [G, A, currents]
 
@@ -314,19 +319,18 @@ class Circuit:
         components touching its rows on the device and builds its rows of G only.  G is then a
         LocalRows view (the rank's rows, global columns), A the rank's slice of the right-hand side."""
         import torch.distributed as tdist
-        from . import dist as ndist
         if not self.sparse:
             raise ValueError("distributed=True needs sparse=True (the dense LU is single-GPU)")
         if not (tdist.is_available() and tdist.is_initialized()):
             raise RuntimeError("distributed=True needs an initialised torch.distributed process group")
         rank, world = tdist.get_rank(), tdist.get_world_size()
-        if dist_sources.applies(table):
-            # R / A / E netlists: through the row-partitioned elimination of the sources (dist_sources.py)
+        if sources.skip_reason(table, True, 0) is not None:
+            # R / A / E netlists with E rows: through the row-partitioned elimination of the sources (dist_sources.py)
             self._dsrc = dist_sources.DistSources(self, dev, table, rank, world)
             return self._dsrc.G, self._dsrc.A
-        runner = ndist.GridRunner(dev, table, 0, rank, world, rtol=self.options.get("rtol", 1e-10),
-                                  precond="jacobi" if self.options.get("precond") == "jacobi" else "amg",
-                                  amg=self.options.get("amg"), solver=ndist.shared_solver(dev, rank, world))
+        runner = ndist.GridRunner(dev, table, 0, rank, world, rtol=self.opts.spd_rtol,
+                                  precond="jacobi" if self.opts.precond == "jacobi" else "amg",
+                                  amg=self.opts.amg, solver=ndist.shared_solver(dev, rank, world))
         indptr, indices, data, rhs = runner.assemble_from_host()
         self._dist = runner
         return ndist.LocalRows(table.n, runner.bounds, rank, indptr, indices, data), rhs
@@ -342,62 +346,41 @@ class Circuit:
         return self.G.cpu().numpy()
 
     # ---- solve ------------------------------------------------------------------
-    def _sparse_solver(self):
-        """Which device solver the sparse path uses: "amg", "pcg" or "gmres".
-        precond: "auto" (default) = aggregation-AMG preconditioned CG for R / A netlists, with a
-        Jacobi-PCG retry if the hierarchy cannot be built or the solve does not converge (the
-        behaviour on singular systems is then the Jacobi path's); "amg" / "jacobi" force one."""
-        precond = self.options.get("precond", "auto")
-        if precond not in ("auto", "jacobi", "amg"):
-            raise ValueError(f"precond must be 'auto', 'jacobi' or 'amg', got {precond!r}")
-        if not self.table.is_spd_structured():
-            return "gmres"
-        return "pcg" if precond == "jacobi" else "amg"
+    def _sorted_G(self):
+        """G, sorted (csr_order="first_touch" sorts before a solve reads G, as spsolve does: SURVEY.md app. C-5)."""
+        if self._G_sorted is not None:
+            self.G, self._G_sorted = self._G_sorted, None
+        return self.G
 
     def _device_solve(self, rhs, amg=None):
         """x, info for G x = rhs on the device (rhs is a device tensor; dense G is not modified).
         Distributed circuits: rhs and x are the rank's slices."""
-        dev = self._dev
+        dev, opts = self._dev, self.opts
         if not self.sparse:
             return dev.lu_solve(self.G.clone(), rhs)
         if self._dsrc is not None:
             raise NotImplementedError("the row-partitioned solve of a netlist with voltage sources is implemented "
                                       "for solve() only")
-        kind = self._sparse_solver()
-        rtol = self.options.get("rtol", 1e-10)
-        warm = self._warm_start()
-        if getattr(self, "_G_sorted", None) is not None:
-            self.G = self._G_sorted        # spsolve leaves circuit.G with sorted indices too (SURVEY.md app. C-5)
-            self._G_sorted = None
+        # R / A netlists: precond "auto" = AMG-PCG with a Jacobi-PCG retry if the hierarchy cannot be built or
+        # the solve does not converge (singular systems behave as on the Jacobi path); "amg" / "jacobi" force one
+        kind = opts.spd_solver if self.table.is_spd_structured() else "gmres"
+        G = self._sorted_G()
         if self._dist is not None:
             if kind == "gmres":
                 raise NotImplementedError("row-partitioned solve is implemented for R / A netlists")
-            g, run = self.G, self._dist
-            first = None
-            if kind == "amg":
-                x, info = run.pcg.solve_amg(g.n, g.bounds, g.indptr, g.indices, g.data, rhs, rtol=rtol,
-                                            maxit=self.options.get("maxit"), **(self.options.get("amg") or {}))
-                if info["status"] == 0 or self.options.get("precond") == "amg":
-                    return x, info
-                first = f"dist_amg_pcg status {info['status']}"      # same status on every rank
-            x, info = run.pcg.solve(g.n, g.bounds, g.indptr, g.indices, g.data, rhs, rtol=rtol,
-                                    maxit=self.options.get("maxit"))
-            if first:
-                info["fallback_from_amg"] = first
-            return x, info
+            return ndist.amg_then_jacobi(self._dist.pcg, G, rhs, opts)
         if kind in ("amg", "pcg"):
-            return self._spd_solve(self.G, rhs, kind, rtol, warm, amg)
-        x, info = dev.gmres(self.G, rhs, rtol=self.options.get("rtol", 1e-12),
-                            restart=self.options.get("restart", 60),
-                            maxit=self.options.get("maxit") or 20000)
+            warm = None if opts.x0 is None else dev.to_device(opts.x0)      # Circuit(..., x0=): SURVEY.md section 5
+            return self._spd_solve(G, rhs, kind, opts.spd_rtol, warm, amg)
+        x, info = dev.gmres(G, rhs, rtol=opts.gmres_rtol, restart=opts.restart, maxit=opts.gmres_maxit)
         # The reference's sparse path is a direct solve, exact for any non-singular MNA system; the
         # diagonally preconditioned GMRES can stall on indefinite systems with many source /
         # op-amp rows.  Rather than handing back an unconverged iterate, systems that fit the dense
         # LU go through it; larger ones are reported (NaNs + warning in solve(), as for breakdown).
-        if info["status"] == 2 and self.options.get("gmres_fallback", True):
-            limit = int(self.options.get("dense_fallback_max_rows", 32768))
-            if self.G.n <= limit:
-                x, lu = dev.lu_solve(dev.csr_to_dense(self.G), rhs)
+        if info["status"] == 2 and opts.gmres_fallback:
+            limit = opts.dense_fallback_max_rows
+            if G.n <= limit:
+                x, lu = dev.lu_solve(dev.csr_to_dense(G), rhs)
                 lu.update(solver="lu (after gmres did not converge)", gmres_iterations=info["iterations"],
                           gmres_relres=info["relres"], relres=None)
                 if lu["status"] == 1:
@@ -411,23 +394,22 @@ class Circuit:
     def _spd_solve(self, G, rhs, kind, rtol, warm, amg=None):
         """x, info for an SPD DeviceCSR G (R / A netlists, or the reduced system of csrc/sources.cu) on
         one GPU: "amg" (with the "auto" Jacobi probe and the Jacobi-PCG retry) or "pcg"."""
-        dev = self._dev
-        if kind == "amg" and amg is None and warm is None and self.options.get("precond", "auto") == "auto":
+        dev, opts = self._dev, self.opts
+        if kind == "amg" and amg is None and warm is None and opts.precond == "auto":
             # "auto": which preconditioner pays depends on the graph, not on its size -- on a 4 M-node
             # expander-like random network Jacobi-PCG needs 98 iterations (43 ms) and the AMG hierarchy
             # 265 ms; on a banded random network of the same size it is 4 616 iterations (1.9 s)
             # against 68 (156 ms); grids are the second kind.  A short Jacobi-PCG probe tells them
             # apart: if 24 iterations gained two digits it will finish in ~100, otherwise its iterate
             # is the initial guess of the AMG solve.
-            probe_its = int(self.options.get("auto_probe_iterations", 24))
-            if G.n >= self.options.get("auto_probe_min_rows", 50_000) and probe_its > 0:
-                x0, info0 = dev.pcg(G, rhs, rtol=rtol, maxit=probe_its, flags=self.options.get("pcg_flags", 0))
+            probe_its = opts.auto_probe_iterations
+            if G.n >= opts.auto_probe_min_rows and probe_its > 0:
+                x0, info0 = dev.pcg(G, rhs, rtol=rtol, maxit=probe_its, flags=opts.pcg_flags)
                 if info0["status"] == 0:
                     info0["auto"] = "jacobi (converged inside the probe)"
                     return x0, info0
                 if info0["status"] == 2 and info0["relres"] <= 1e-2:
-                    x, info = dev.pcg(G, rhs, rtol=rtol, maxit=self.options.get("maxit"), x0=x0,
-                                      flags=self.options.get("pcg_flags", 0))
+                    x, info = dev.pcg(G, rhs, rtol=rtol, maxit=opts.maxit, x0=x0, flags=opts.pcg_flags)
                     info["iterations"] += info0["iterations"]
                     info["auto"] = f"jacobi (probe relres {info0['relres']:.1e})"
                     if info["status"] == 0:
@@ -442,48 +424,33 @@ class Circuit:
                 return x, info
         if kind == "amg":
             return self._amg_solve(G, rhs, amg, rtol, warm)
-        return dev.pcg(G, rhs, rtol=rtol, maxit=self.options.get("maxit"),
-                      flags=self.options.get("pcg_flags", 0), x0=warm)
-
-    def _warm_start(self):
-        """Initial guess of the iterative solvers: Circuit(..., x0=array of n values) -- e.g. the
-        previous solution of a parameter sweep (SURVEY.md section 5).  None: start from zero."""
-        x0 = self.options.get("x0")
-        if x0 is None or not self.sparse or self._dist is not None:
-            return None
-        arr = np.ascontiguousarray(x0, dtype=np.float64)
-        if arr.shape != (self.table.n,):
-            raise ValueError(f"x0 must have {self.table.n} entries")
-        return self._dev.to_device(arr)
+        return dev.pcg(G, rhs, rtol=rtol, maxit=opts.maxit, flags=opts.pcg_flags, x0=warm)
 
     def _amg_solve(self, G, rhs, amg, rtol, x0):
         """AMG-preconditioned CG on one GPU; Jacobi-PCG retry unless precond="amg" was forced."""
-        dev = self._dev
+        dev, opts = self._dev, self.opts
         from . import _lib
         try:
             if amg is not None:
-                x, info = amg.solve(rhs, rtol=rtol, maxit=self.options.get("maxit"), x0=x0)
-            elif G.n >= self.options.get("amg_graph_min_rows", 100_000):
+                x, info = amg.solve(rhs, rtol=rtol, maxit=opts.maxit, x0=x0)
+            elif G.n >= opts.amg_graph_min_rows:
                 # large systems: the graph-captured form (csrc/dist_amg.cu with one rank):
                 # one CUDA graph per iteration, no host round trip inside the iteration
-                from . import dist as ndist
                 g = G
                 bounds = np.array([0, g.n], dtype=np.int32)
                 x, info = ndist.single_solver(dev).solve_amg(
-                    g.n, bounds, g.indptr, g.indices, g.data, rhs, rtol=rtol, maxit=self.options.get("maxit"),
-                    x0=x0, **(self.options.get("amg") or {}))
+                    g.n, bounds, g.indptr, g.indices, g.data, rhs, rtol=rtol, maxit=opts.maxit,
+                    x0=x0, **opts.amg_params)
             else:
-                x, info = dev.amg_pcg(G, rhs, rtol=rtol, maxit=self.options.get("maxit"), x0=x0,
-                                      **(self.options.get("amg") or {}))
-            if info["status"] == 0 or self.options.get("precond") == "amg":
+                x, info = dev.amg_pcg(G, rhs, rtol=rtol, maxit=opts.maxit, x0=x0, **opts.amg_params)
+            if info["status"] == 0 or opts.precond == "amg":
                 return x, info
             first = f"amg_pcg status {info['status']} after {info['iterations']} iterations"
         except _lib.NodalLibraryError as err:
-            if self.options.get("precond") == "amg":
+            if opts.precond == "amg":
                 raise
             first = str(err)
-        x, info = dev.pcg(G, rhs, rtol=rtol, maxit=self.options.get("maxit"),
-                          flags=self.options.get("pcg_flags", 0))
+        x, info = dev.pcg(G, rhs, rtol=rtol, maxit=opts.maxit, flags=opts.pcg_flags)
         info["fallback_from_amg"] = first
         return x, info
 
@@ -499,36 +466,33 @@ class Circuit:
         mirrors scipy (no exception; a Krylov solver even returns a finite solution when the
         singular system is consistent) unless the Circuit was built with check_connected=True:
         then the lead graph is checked on the device first and an unconnected circuit raises
-        UnconnectedCircuitError like the dense path."""
-        if self.sparse and self.options.get("check_connected") and not self.is_connected():
+        UnconnectedCircuitError like the dense path.
+
+        On one GPU the sparse solve runs the candidates of options.plan in order (sources,
+        source_schur, schur; a path's solve(circuit) gives (x, info), or (None, stats) when it
+        declines) and _device_solve when none solves.  The stats of a declined sources or
+        source_schur go under info["reduction"] (the two are exclusive by table content), those of
+        a declined schur under info["schur"], never over a key the path which solved set (the schur
+        stats of a successful source_schur stay); a path not asked for leaves no key."""
+        if self.sparse and self.opts.check_connected and not self.is_connected():
             logging.error("Model error: unconnected circuit")
             raise UnconnectedCircuitError
-        # R / A / E netlists: through the elimination of the voltage sources when it applies
-        # (sources.py; dist_sources.py row-partitioned, x whole on every rank); otherwise `info` is
-        # the stats of why not, or None
         if self._dsrc is not None:
-            x, info = self._dsrc.solve()
-        else:
-            x, info = sources.solve(self) if self.sparse and self._dist is None else (None, None)
-        if x is None:
-            skipped = info
-            # schur=True with eliminate_sources=True on a table with E rows and dependent rows: the
-            # elimination, then the Schur complement of the reduced system (source_schur.py)
-            x, info = source_schur.solve(self) if self.sparse and self._dist is None else (None, None)
-            if x is not None:
-                skipped = None
-            elif info is not None:
-                skipped = info
-        if x is None:
-            # then, when requested and the netlist qualifies, the Schur complement of the branch rows
-            x, info = schur.solve(self) if self.sparse and self._dist is None else (None, None)
-            if x is None:
-                declined = info
+            x, info = self._dsrc.solve()            # dist_sources.py: x whole on every rank
+        elif self.sparse and self._dist is None:
+            self._sorted_G()
+            declined = {}
+            for step in self._plan:
+                x, info = _PATHS[step.path].solve(self) if not step.reason else (None, dict(step.declined))
+                if x is not None:
+                    break
+                declined[step.key] = info
+            else:
                 x, info = self._device_solve(self.A)
-                if declined is not None:
-                    info["schur"] = declined
-            if skipped is not None:
-                info["reduction"] = skipped
+            for key, stats in declined.items():
+                info.setdefault(key, stats)
+        else:
+            x, info = self._device_solve(self.A)
         if self.sparse:
             e = self._dist_gather(x) if self._dist is not None else x.cpu().numpy()
             if info["status"] != 0:
@@ -596,17 +560,18 @@ class Circuit:
         pairs = list(pairs)
         # several right-hand sides share one hierarchy; a single solve goes through _device_solve's
         # own choice (auto probe, graph-captured form for large systems)
-        if self.sparse and run is None and self._sparse_solver() == "amg" and len(pairs) > 1:
+        if self.sparse and run is None and self.table.is_spd_structured() and self.opts.spd_solver == "amg" \
+                and len(pairs) > 1:
             from . import _lib
             try:
-                amg = dev.amg(self.G, **(self.options.get("amg") or {}))
+                amg = dev.amg(self.G, **self.opts.amg_params)
             except _lib.NodalLibraryError:
-                if self.options.get("precond") == "amg":
+                if self.opts.precond == "amg":
                     raise
                 amg = None             # _device_solve retries per right-hand side and falls back to Jacobi
         values, stats = [], []
         try:
-            if amg is not None and self.options.get("multi_rhs", True):
+            if amg is not None and self.opts.multi_rhs:
                 # several ports against one hierarchy: batches of up to 8 right-hand sides advance
                 # together, every level operator is read once per sweep for the whole batch
                 # (csrc/amg_multi.cu); a batch that does not converge is redone pair by pair below
@@ -622,7 +587,7 @@ class Circuit:
                             rhs[j, ia] = 1.0
                         if ib != c.GROUND:
                             rhs[j, ib] = -1.0
-                    xs, infos = amg.solve_multi(rhs, rtol=self.options.get("rtol", 1e-10), maxit=self.options.get("maxit"))
+                    xs, infos = amg.solve_multi(rhs, rtol=self.opts.spd_rtol, maxit=self.opts.maxit)
                     for j, k in enumerate(batch):
                         if infos[j]["status"] == 0:
                             ia, ib = rows_of[k]
@@ -662,6 +627,9 @@ class Circuit:
                 amg.close()
         self.stats = stats
         return values
+
+
+_PATHS = {"sources": sources, "source_schur": source_schur, "schur": schur}
 
 
 class Solution:

@@ -19,10 +19,10 @@ Circuit(netlist, sparse=True, schur=...):
     False  (default) the existing path
     True   solve through the Schur complement when the netlist qualifies: at least one branch row,
            every R positive, every node reaching ground through resistors alone and
-           m <= schur_max_branches (default 8192; S and its factors are m^2 doubles).  Otherwise,
-           or when the refinement does not reach rtol, the existing path runs and
-           Solution.stats["schur"]["reason"] says why.
-    schur_rtol (default rtol) is the tolerance of the L solves, schur_refine (default 5) the most
+           m <= schur_max_branches (S and its factors are m^2 doubles).  Otherwise, or when the
+           refinement does not reach rtol, the existing path runs and Solution.stats["schur"]["reason"]
+           says why.
+    schur_rtol (rtol when not given) is the tolerance of the L solves, schur_refine the most
     applications of the block inverse.  A step that does not halve the residual ends the refinement.
 """
 from __future__ import annotations
@@ -31,22 +31,6 @@ import math
 import time
 
 from . import _lib
-
-
-def check_option(options, sparse, distributed):
-    """Validate schur and its parameters; True with sparse=False or distributed=True is an error."""
-    mode = options.get("schur", False)
-    if mode is not True and mode is not False:
-        raise ValueError(f"schur must be True or False, got {mode!r}")
-    if mode and not sparse:
-        raise ValueError("schur=True needs sparse=True (the dense path already solves by LU)")
-    if mode and distributed:
-        raise NotImplementedError("the Schur-complement solve runs on one GPU (distributed=True is not supported)")
-    if int(options.get("schur_refine", 5)) < 0:
-        raise ValueError("schur_refine must be >= 0")
-    if int(options.get("schur_max_branches", 8192)) < 1:
-        raise ValueError("schur_max_branches must be >= 1")
-    return mode
 
 
 def skip_reason(table, max_branches):
@@ -64,55 +48,39 @@ def skip_reason(table, max_branches):
     return ""
 
 
-def _ms(t0, dev):
-    dev.torch.cuda.current_stream(dev.dev).synchronize()
-    return (time.perf_counter() - t0) * 1e3
-
-
 def solve(circuit):
-    """(x, info) of the full system through the Schur complement, or (None, stats) when it is not
-    requested (stats None), does not apply or does not converge (stats["reason"] says why)."""
-    if not circuit._schur:
-        return None, None
-    table, dev, opts = circuit.table, circuit._dev, circuit.options
+    """(x, info) of the full system through the Schur complement of a table skip_reason lets through,
+    or (None, stats) when it does not apply or does not converge (stats["reason"] says why)."""
+    table, dev, opts = circuit.table, circuit._dev, circuit.opts
     kcl, m = table.kcl, table.be
     stats = dict(applied=False, branches=m, node_rows=kcl)
-    reason = skip_reason(table, int(opts.get("schur_max_branches", 8192)))
-    if reason:
-        stats["reason"] = reason
-        return None, stats
-    if getattr(circuit, "_G_sorted", None) is not None:     # as in Circuit._device_solve
-        circuit.G, circuit._G_sorted = circuit._G_sorted, None
     G, A = circuit.G, circuit.A
-    rtol = opts.get("rtol", 1e-10)
-    inner = opts.get("schur_rtol", rtol)
-    refine = int(opts.get("schur_refine", 5))
-    maxit = opts.get("maxit")
 
     t0 = time.perf_counter()
     grounded = dev.r_grounded(circuit._dtab, len(table), kcl)
-    stats["check_ms"] = _ms(t0, dev)
+    stats["check_ms"] = dev.ms_since(t0)
     if not grounded:
         stats["reason"] = "a node does not reach ground through resistors (L would be singular)"
         return None, stats
     t0 = time.perf_counter()
     L, B = dev.schur_split(G, kcl)
-    stats["split_ms"] = _ms(t0, dev)
+    stats["split_ms"] = dev.ms_since(t0)
     t0 = time.perf_counter()
     try:
-        amg = dev.amg(L, **(opts.get("amg") or {}))
+        amg = dev.amg(L, **opts.amg_params)
     except _lib.NodalLibraryError as err:
         stats["reason"] = f"AMG setup on L failed: {err}"
         return None, stats
-    stats["amg_setup_ms"] = _ms(t0, dev)
+    stats["amg_setup_ms"] = dev.ms_since(t0)
     try:
-        return _solve_with(dev, amg, G, A, B, kcl, m, rtol, inner, refine, maxit, stats)
+        return _solve_with(dev, amg, G, A, B, kcl, m, opts, stats)
     finally:
         amg.close()
 
 
-def _solve_with(dev, amg, G, A, B, kcl, m, rtol, inner, refine, maxit, stats):
+def _solve_with(dev, amg, G, A, B, kcl, m, opts, stats):
     torch = dev.torch
+    rtol, inner, refine, maxit = opts.spd_rtol, opts.inner_rtol, opts.schur_refine, opts.maxit
     # ---- columns of S, eight at a time
     t0 = time.perf_counter()
     S = dev.empty(m * m, torch.float64).view(m, m)
@@ -130,11 +98,11 @@ def _solve_with(dev, amg, G, A, B, kcl, m, rtol, inner, refine, maxit, stats):
             return None, stats
         dev.schur_columns(G, kcl, j0, Z, S)
         del Z
-    stats.update(batches=batches, batch_iterations_max=worst, columns_ms=_ms(t0, dev))
+    stats.update(batches=batches, batch_iterations_max=worst, columns_ms=dev.ms_since(t0))
     # ---- S = P^T L U once
     t0 = time.perf_counter()
     ipiv, finfo = dev.lu_factor(S)
-    stats["factor_ms"] = _ms(t0, dev)
+    stats["factor_ms"] = dev.ms_since(t0)
     if finfo["status"] != 0:
         stats["reason"] = f"S is singular (zero pivot {finfo['info']})"
         return None, stats
@@ -168,7 +136,7 @@ def _solve_with(dev, amg, G, A, B, kcl, m, rtol, inner, refine, maxit, stats):
         dev.schur_add(x[:kcl], xn)
         dev.schur_add(x[kcl:], xb)
         step += 1
-        step_ms.append(_ms(t0, dev))
+        step_ms.append(dev.ms_since(t0))
     stats.update(refine_steps=step, refine_ms=step_ms, relres_history=history, relres_full=history[-1],
                  refine_iterations=inner_its)
     if reason:

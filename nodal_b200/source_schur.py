@@ -31,14 +31,6 @@ from . import sources
 _DEP = (1 << K.T_VCVS) | (1 << K.T_VCCS) | (1 << K.T_CCVS) | (1 << K.T_CCCS)
 
 
-def applies(circuit):
-    """The combined path is asked for: schur=True and eliminate_sources=True on a table with E rows
-    and dependent rows."""
-    t = circuit.table
-    return (circuit.sparse and circuit._dist is None and circuit._schur and circuit._eliminate is True
-            and t.has_type(K.T_E) and bool(t.facts()["present"] & _DEP))
-
-
 def skip_reason(table):
     """What the host can tell before the forest ("" when nothing)."""
     f = table.facts()
@@ -61,38 +53,29 @@ def e_forest(dev, dtab, ncomp, kcl):
 
 
 def solve(circuit):
-    """(x, info) of the full system, or (None, stats) when the path does not apply (stats None) or
-    declines (stats["reason"] says why)."""
-    if not applies(circuit):
-        return None, None
-    table, dev, opts = circuit.table, circuit._dev, circuit.options
+    """(x, info) of the full system for a table skip_reason lets through, or (None, stats) when the
+    path declines (stats["reason"] says why)."""
+    table, dev, opts = circuit.table, circuit._dev, circuit.opts
     kcl, be, ncomp = table.kcl, table.be, len(table)
-    max_branches = int(opts.get("schur_max_branches", 8192))
     stats = dict(eliminated=False, applied=False)
-    reason = skip_reason(table)
-    if reason:
-        return None, dict(stats, reason=reason)
-    if getattr(circuit, "_G_sorted", None) is not None:     # as in Circuit._device_solve
-        circuit.G, circuit._G_sorted = circuit._G_sorted, None
     dtab = circuit._dtab
-    ms = sources._ms
 
     # ---- forest of the E rows alone, the dependent branches numbered in branch order
     t0 = time.perf_counter()
     d_map, md, conflicts = dev.source_dep_map(dtab, ncomp, be)
     stats["dependent_rows"] = md
     if conflicts:
-        stats.update(reason="branch rows not owned by exactly one component (duplicate names)", forest_ms=ms(t0, dev))
+        stats.update(reason="branch rows not owned by exactly one component (duplicate names)", forest_ms=dev.ms_since(t0))
         return None, stats
-    if md > max_branches:
-        stats.update(reason=f"{md} dependent branch rows > schur_max_branches ({max_branches})", forest_ms=ms(t0, dev))
+    if md > opts.schur_max_branches:
+        stats.update(reason=f"{md} dependent branch rows > schur_max_branches ({opts.schur_max_branches})", forest_ms=dev.ms_since(t0))
         return None, stats
     finfo, forest, etab = e_forest(dev, dtab, ncomp, kcl)
     stats.update(sources=finfo["sources"], supernodes=finfo["floating_trees"], grounded_nodes=finfo["grounded_nodes"])
     reason = sources.forest_reason(finfo)
     if not reason and dev.source_dep_check(dtab, ncomp, kcl, forest):
         reason = "a VCVS / VCCS / CCVS has both output leads in one source tree (its current is undetermined)"
-    stats["forest_ms"] = ms(t0, dev)
+    stats["forest_ms"] = dev.ms_since(t0)
     if reason:
         stats["reason"] = reason
         return None, stats
@@ -103,21 +86,20 @@ def solve(circuit):
     red, nred = dev.source_reduce(dtab, ncomp, kcl, forest)
     if mn > 0 and not dev.r_grounded(red, nred, mn):
         stats.update(reason="a reduced node does not reach ground through the reduced resistors "
-                            "(L would be singular)", reduced_rows=mn, reduce_ms=ms(t0, dev))
+                            "(L would be singular)", reduced_rows=mn, reduce_ms=dev.ms_since(t0))
         return None, stats
-    stats.update(reduced_rows=mn, reduced_components=nred, forest_depth=finfo["depth"], reduce_ms=ms(t0, dev))
+    stats.update(reduced_rows=mn, reduced_components=nred, forest_depth=finfo["depth"], reduce_ms=dev.ms_since(t0))
     t0 = time.perf_counter()
     Gr, Ar = dev.source_dep_assemble(red, nred, mn, md, kcl, forest, d_map, circuit.G, circuit.A)
     del red
-    stats["assemble_ms"] = ms(t0, dev)
+    stats["assemble_ms"] = dev.ms_since(t0)
 
     # ---- the Schur solve of schur.py on the reduced system
-    rtol = opts.get("rtol", 1e-10)
     sstats = dict(applied=False, branches=md, node_rows=mn)
     if mn == 0:                                 # every node is in ground's tree: the branch rows alone
         t0 = time.perf_counter()
         y, lu = dev.lu_solve(dev.csr_to_dense(Gr), Ar)
-        sstats["factor_ms"] = ms(t0, dev)
+        sstats["factor_ms"] = dev.ms_since(t0)
         if lu["status"] != 0:
             stats["reason"] = f"the dependent rows are singular (zero pivot {lu['info']})"
             return None, dict(stats, schur=sstats)
@@ -126,17 +108,16 @@ def solve(circuit):
     else:
         t0 = time.perf_counter()
         L, B = dev.schur_split(Gr, mn)
-        sstats["split_ms"] = ms(t0, dev)
+        sstats["split_ms"] = dev.ms_since(t0)
         t0 = time.perf_counter()
         try:
-            amg = dev.amg(L, **(opts.get("amg") or {}))
+            amg = dev.amg(L, **opts.amg_params)
         except _lib.NodalLibraryError as err:
             stats["reason"] = f"AMG setup on the reduced L failed: {err}"
             return None, dict(stats, schur=sstats)
-        sstats["amg_setup_ms"] = ms(t0, dev)
+        sstats["amg_setup_ms"] = dev.ms_since(t0)
         try:
-            y, info = schur._solve_with(dev, amg, Gr, Ar, B, mn, md, rtol, opts.get("schur_rtol", rtol),
-                                        int(opts.get("schur_refine", 5)), opts.get("maxit"), sstats)
+            y, info = schur._solve_with(dev, amg, Gr, Ar, B, mn, md, opts, sstats)
         finally:
             amg.close()
         if y is None:
@@ -148,6 +129,6 @@ def solve(circuit):
     # ---- expansion on the full system
     t0 = time.perf_counter()
     x, relres = dev.source_expand_dep(etab, kcl, forest, finfo, d_map, mn, y, circuit.G, circuit.A)
-    stats.update(eliminated=True, applied=True, reason="", expand_ms=ms(t0, dev), relres_full=relres)
+    stats.update(eliminated=True, applied=True, reason="", expand_ms=dev.ms_since(t0), relres_full=relres)
     info.update(solver="source_schur", relres_full=relres, reduction=stats, schur=sstats)
     return x, info

@@ -15,6 +15,7 @@ from nodal_b200 import constants as K
 from nodal_b200 import generators as gen
 from nodal_b200 import schur
 from nodal_b200.device import coo_stride
+from nodal_b200.options import parse
 from oracle import mna_oracle as orc
 
 DOC = golden("doc_netlists.json")
@@ -136,7 +137,7 @@ def test_core_matches_statement_bit_for_bit(case, tmp_path):
     assert np.array_equal(mirror.rhs_batch((b_ptr, b_col, b_val), kcl, 0, min(8, m)), B[:, :min(8, m)].T)
 
 
-def test_eligibility_rules(tmp_path):
+def test_eligibility_and_option_parsing(tmp_path):
     base = DOC["opmodel_amplifier.csv"]["rows"]
     table = table_of(base, tmp_path)
     assert schur.skip_reason(table, 8192) == "" and mirror.r_grounded(table)
@@ -149,10 +150,10 @@ def test_eligibility_rules(tmp_path):
     assert schur.skip_reason(floating, 8192) == "" and not mirror.r_grounded(floating)
     for bad in ("yes", 1, None):
         with pytest.raises(ValueError):
-            schur.check_option({"schur": bad}, True, False)
+            parse({"schur": bad}, True, table)
     with pytest.raises(ValueError):
-        schur.check_option({"schur": True, "schur_refine": -1}, True, False)
-    assert schur.check_option({}, True, True) is False
+        parse({"schur": True, "schur_refine": -1}, True, table)
+    assert parse({"distributed": True}, True, table).schur is False
 
 
 def test_option_errors_at_construction(tmp_path):

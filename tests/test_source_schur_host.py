@@ -2,8 +2,6 @@
 numpy statement (source_schur_mirror.py) against the oracle, the dependent-row rules of
 csrc/sources_core.cuh compiled for the host against the statement bit for bit, the eligibility rules,
 the options, amplifier_grid(ideal_pads=True) against its csv and the CLI mapping."""
-from types import SimpleNamespace
-
 import numpy as np
 import pytest
 import scipy.sparse as sps
@@ -17,7 +15,8 @@ from test_schur_host import _csv_rows
 import nodal_b200 as n
 from nodal_b200 import constants as K
 from nodal_b200 import generators as gen
-from nodal_b200 import schur, source_schur, sources
+from nodal_b200 import source_schur
+from nodal_b200.options import parse, plan
 from oracle import mna_oracle as orc
 
 DOC = golden("doc_netlists.json")
@@ -169,28 +168,26 @@ def test_eligibility_rules(tmp_path):
     assert mirror.reason(table_of(HAND_TREE, tmp_path), max_branches=2) == "schur_max_branches"
 
 
-def _circuit(table, **opts):
-    mode = sources.check_option(opts, table)
-    return SimpleNamespace(table=table, sparse=True, _dist=None, _eliminate=mode,
-                           _schur=schur.check_option(opts, True, opts.get("distributed")))
+def _paths(table, **opts):
+    return [step.path for step in plan(table, parse(opts, True, table))]
 
 
-def test_option_matrix(tmp_path):
+def test_option_plan_matrix(tmp_path):
     mixed = table_of(HAND_TREE, tmp_path)
-    assert source_schur.applies(_circuit(mixed, schur=True, eliminate_sources=True))
+    assert _paths(mixed, schur=True, eliminate_sources=True) == ["source_schur", "schur"]
     with pytest.raises(ValueError):                                  # True alone: as before
-        sources.check_option({"eliminate_sources": True}, mixed)
+        parse({"eliminate_sources": True}, True, mixed)
     with pytest.raises(ValueError):
-        sources.check_option({"eliminate_sources": True, "schur": False}, mixed)
-    assert not source_schur.applies(_circuit(mixed, schur=True))     # "auto": the full-system Schur
-    assert not source_schur.applies(_circuit(mixed, schur=True, eliminate_sources=False))
+        parse({"eliminate_sources": True, "schur": False}, True, mixed)
+    assert _paths(mixed, schur=True) == ["schur"]                    # "auto": the full-system Schur
+    assert _paths(mixed, schur=True, eliminate_sources=False) == ["schur"]
     # without E rows or without dependent rows the combination is not asked for
-    assert not source_schur.applies(_circuit(table_of(DOC["x_vcvs_null_control.csv"]["rows"], tmp_path), schur=True,
-                                             eliminate_sources=True))
-    assert not source_schur.applies(_circuit(table_of(orc.grid2d_rows(3) + [["v", "E", "1", "0", "g"]], tmp_path),
-                                             schur=True, eliminate_sources=True))
+    assert "source_schur" not in _paths(table_of(DOC["x_vcvs_null_control.csv"]["rows"], tmp_path), schur=True,
+                                        eliminate_sources=True)
+    assert "source_schur" not in _paths(table_of(orc.grid2d_rows(3) + [["v", "E", "1", "0", "g"]], tmp_path),
+                                        schur=True, eliminate_sources=True)
     with pytest.raises(NotImplementedError):
-        schur.check_option({"schur": True, "eliminate_sources": True}, True, True)
+        parse({"schur": True, "eliminate_sources": True, "distributed": True}, True, mixed)
 
 
 def test_amplifier_grid_ideal_pads_matches_csv(tmp_path):

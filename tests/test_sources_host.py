@@ -13,6 +13,7 @@ import nodal_b200 as n
 from nodal_b200 import constants as K
 from nodal_b200 import generators as gen
 from nodal_b200 import sources
+from nodal_b200.options import parse
 from oracle import mna_oracle as orc
 
 
@@ -134,7 +135,7 @@ def test_shared_branch_is_not_eliminated(tmp_path):
     assert not f["ok"] and f["branch_conflicts"] == 2
 
 
-def test_eligibility_rules(tmp_path):
+def test_eligibility_and_option_parsing(tmp_path):
     base = orc.grid2d_rows(6) + [["v1", "E", "1", "n0_0", "g"]]
     table = table_of(base, tmp_path)
     assert sources.skip_reason(table, "auto", 32768).startswith(f"{table.n} rows")
@@ -146,10 +147,10 @@ def test_eligibility_rules(tmp_path):
     dep = table_of(base + [["d1", "VCVS", "2", "n5_5", "g", "n0_0", "g"]], tmp_path)
     assert sources.skip_reason(dep, "auto", 10) is None
     with pytest.raises(ValueError):
-        sources.check_option({"eliminate_sources": True}, dep)
-    assert sources.check_option({"eliminate_sources": "auto"}, dep) == "auto"
+        parse({"eliminate_sources": True}, True, dep)
+    assert parse({"eliminate_sources": "auto"}, True, dep).eliminate_sources == "auto"
     with pytest.raises(ValueError):
-        sources.check_option({"eliminate_sources": "yes"}, table)
+        parse({"eliminate_sources": "yes"}, True, table)
     assert sources.skip_reason(table_of(orc.grid2d_rows(6), tmp_path), True, 0) is None    # no E rows
 
 
