@@ -128,6 +128,8 @@ int nodal_sell_create(nodal_ctx* ctx, int32_t n, int64_t nnz, const int32_t* ind
                       const int32_t* indices, const double* data, nodal_sell** out, void* stream);
 int nodal_sell_destroy(nodal_sell* m);
 int64_t nodal_sell_padded_nnz(const nodal_sell* m);
+/* 1 when m stores its entries compact (16-bit column offsets, 1-byte value indices), 0 when wide */
+int nodal_sell_compact(const nodal_sell* m);
 int nodal_sell_spmv(nodal_ctx* ctx, const nodal_sell* m, const double* x, double* y, void* stream);
 
 /* Jacobi-preconditioned conjugate gradients, FP64.  Replaces

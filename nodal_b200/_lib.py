@@ -35,6 +35,7 @@ SIGNATURES = {
     "nodal_sell_create": (C.c_int, [_vp, _i32, _i64, _vp, _vp, _vp, C.POINTER(_vp), _vp]),
     "nodal_sell_destroy": (C.c_int, [_vp]),
     "nodal_sell_padded_nnz": (_i64, [_vp]),
+    "nodal_sell_compact": (C.c_int, [_vp]),
     "nodal_sell_spmv": (C.c_int, [_vp, _vp, _vp, _vp, _vp]),
     "nodal_pcg": (C.c_int, [_vp, _i32, _i64, _vp, _vp, _vp, _vp, _vp, _f64, _i32, _i32,
                             C.POINTER(_i32), C.POINTER(_f64), C.POINTER(_f64), _vp]),

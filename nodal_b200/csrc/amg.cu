@@ -321,8 +321,10 @@ template <int MODE>
 int sell_sweep(const nodal_amg* h, const AmgLevel& V, const double* b, const double* x, double* y,
                double* part, cudaStream_t st) {
     const nodal_sell* m = V.sell;
-    amg_sell_kernel<MODE><<<sell_grid(h->ctx, m->nslices), AT, 0, st>>>(
-        m->n, m->nslices, m->slice_w, m->cols, m->vals, m->dinv, b, x, h->omega, y, part);
+    sell_launch(m, [&](auto a) {
+        amg_sell_kernel<MODE><<<sell_grid(h->ctx, m->nslices), AT, 0, st>>>(
+            m->n, m->nslices, m->slice_w, a, m->dinv, b, x, h->omega, y, part);
+    });
     KERNEL_CHECK();
     return NODAL_OK;
 }
@@ -333,8 +335,10 @@ template <int MODE>
 int cycle_sweep(const nodal_amg* h, const AmgLevel& V, const double* b, const double* xc, double* y,
                 cudaStream_t st) {
     const nodal_sell* m = V.sell;
-    amg_cycle_sweep_kernel<MODE><<<sell_grid(h->ctx, m->nslices), AT, 0, st>>>(
-        m->n, m->nslices, m->slice_w, m->cols, m->vals, m->dinv, b, h->omega, V.agg, xc, h->scale, y);
+    sell_launch(m, [&](auto a) {
+        amg_cycle_sweep_kernel<MODE><<<sell_grid(h->ctx, m->nslices), AT, 0, st>>>(
+            m->n, m->nslices, m->slice_w, a, m->dinv, b, h->omega, V.agg, xc, h->scale, y);
+    });
     KERNEL_CHECK();
     return NODAL_OK;
 }

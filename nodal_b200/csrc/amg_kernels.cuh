@@ -136,13 +136,13 @@ amg_jacobi0_kernel(int32_t n, const double* __restrict__ dinv, const double* __r
 //   MODE 0: y = A x, per-block partial sums of x.y        (CG: q = A p, p.q)
 //   MODE 1: y = b - A x                                   (residual)
 //   MODE 2: y = x + omega D^-1 (b - A x)                  (damped Jacobi sweep, out of place)
-template <int MODE>
+template <int MODE, class A>
 static __global__ void __launch_bounds__(AT, 5)
-amg_sell_kernel(int32_t n, int32_t nslices, const u32* __restrict__ slice_w,
-                const int32_t* __restrict__ cols, const double* __restrict__ vals,
+amg_sell_kernel(int32_t n, int32_t nslices, const u32* __restrict__ slice_w, A a0,
                 const double* __restrict__ dinv, const double* __restrict__ b,
                 const double* __restrict__ x, double omega, double* __restrict__ y,
                 double* __restrict__ part) {
+    const A a = a0.staged();
     __shared__ double red[33];
     const int lane = threadIdx.x & 31;
     const int64_t warp = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
@@ -151,8 +151,8 @@ amg_sell_kernel(int32_t n, int32_t nslices, const u32* __restrict__ slice_w,
     for (int64_t s = warp; s < nslices; s += nwarps) {
         const u32 w0 = slice_w[s];
         const int w = (int)(slice_w[s + 1] - w0);
-        const double acc = sell_row_dot(cols, vals, (int64_t)w0 * 32 + lane, w, x);
         const int64_t r = s * 32 + lane;
+        const double acc = sell_row_dot(a, (int64_t)w0 * 32 + lane, r, w, x);
         if (r < n) {
             if (MODE == 0) { y[r] = acc; dot = fma(x[r], acc, dot); }
             if (MODE == 1) y[r] = amg_residual(b[r], acc);
@@ -207,13 +207,13 @@ struct ProlongatedAt {
     }
 };
 
-template <int MODE>
+template <int MODE, class A>
 static __global__ void __launch_bounds__(AT, 5)
-amg_cycle_sweep_kernel(int32_t n, int32_t nslices, const u32* __restrict__ slice_w,
-                       const int32_t* __restrict__ cols, const double* __restrict__ vals,
+amg_cycle_sweep_kernel(int32_t n, int32_t nslices, const u32* __restrict__ slice_w, A a0,
                        const double* __restrict__ dinv, const double* __restrict__ b, double omega,
                        const int32_t* __restrict__ agg, const double* __restrict__ xc, double scale,
                        double* __restrict__ y) {
+    const A a = a0.staged();
     const int lane = threadIdx.x & 31;
     const int64_t warp = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     const int64_t nwarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
@@ -225,11 +225,11 @@ amg_cycle_sweep_kernel(int32_t n, int32_t nslices, const u32* __restrict__ slice
         const int64_t base = (int64_t)w0 * 32 + lane;
         const int64_t r = s * 32 + lane;
         if (MODE == 1) {
-            const double acc = sell_row_gather(cols, vals, base, w, x0);
+            const double acc = sell_row_gather(a, base, r, w, x0);
             if (r < n) y[r] = amg_residual(b[r], acc);
         }
         if (MODE == 2) {
-            const double acc = sell_row_gather(cols, vals, base, w, xa);
+            const double acc = sell_row_gather(a, base, r, w, xa);
             if (r < n) y[r] = amg_jacobi_update(omega, dinv[r], b[r], acc, xa((int32_t)r));
         }
     }

@@ -16,17 +16,17 @@ namespace {
 
 constexpr int MK = 8;      // right-hand sides per batch
 
-// dot products of one SELL row (lane) with K vectors: columns / values loaded once
-template <int W>
-__device__ __forceinline__ void sell_dot_fixed_multi(const int32_t* __restrict__ cols, const double* __restrict__ vals,
-                                                     int64_t base, const double* __restrict__ x, int64_t stride, int K,
-                                                     double* acc) {
+// dot products of one SELL row (lane, row r) with K vectors: columns / values loaded once
+template <int W, class A>
+__device__ __forceinline__ void sell_dot_fixed_multi(const A& a, int64_t base, int64_t r, const double* __restrict__ x,
+                                                     int64_t stride, int K, double* acc) {
     int32_t c[W];
     double v[W];
 #pragma unroll
     for (int i = 0; i < W; ++i) {
-        c[i] = cols[base + (int64_t)i * 32];
-        v[i] = vals[base + (int64_t)i * 32];
+        const typename A::Entry e = a.load(base + (int64_t)i * 32);
+        c[i] = a.col(e, r);
+        v[i] = a.val(e);
     }
 #pragma unroll
     for (int k = 0; k < 8; ++k) {          // compile-time indices keep acc[] in registers
@@ -40,28 +40,28 @@ __device__ __forceinline__ void sell_dot_fixed_multi(const int32_t* __restrict__
     }
 }
 
-__device__ __forceinline__ void sell_row_dot_multi(const int32_t* __restrict__ cols, const double* __restrict__ vals,
-                                                   int64_t base, int w, const double* __restrict__ x, int64_t stride,
-                                                   int K, double* acc) {
+template <class A>
+__device__ __forceinline__ void sell_row_dot_multi(const A& a, int64_t base, int64_t r, int w,
+                                                   const double* __restrict__ x, int64_t stride, int K, double* acc) {
     int k = 0;
-    for (; k + 4 <= w; k += 4) sell_dot_fixed_multi<4>(cols, vals, base + (int64_t)k * 32, x, stride, K, acc);
+    for (; k + 4 <= w; k += 4) sell_dot_fixed_multi<4>(a, base + (int64_t)k * 32, r, x, stride, K, acc);
     const int64_t b = base + (int64_t)k * 32;
     switch (w - k) {   // warp-uniform
-        case 3: sell_dot_fixed_multi<3>(cols, vals, b, x, stride, K, acc); break;
-        case 2: sell_dot_fixed_multi<2>(cols, vals, b, x, stride, K, acc); break;
-        case 1: sell_dot_fixed_multi<1>(cols, vals, b, x, stride, K, acc); break;
+        case 3: sell_dot_fixed_multi<3>(a, b, r, x, stride, K, acc); break;
+        case 2: sell_dot_fixed_multi<2>(a, b, r, x, stride, K, acc); break;
+        case 1: sell_dot_fixed_multi<1>(a, b, r, x, stride, K, acc); break;
         default: break;
     }
 }
 
 // MODE 0: y = A x and per-block partials of x.y   MODE 1: y = b - A x   MODE 2: y = x + omega D^-1 (b - A x)
-template <int MODE>
+template <int MODE, class A>
 __global__ void __launch_bounds__(AT, 3)
-amgm_sell_kernel(int32_t n, int32_t nslices, const u32* __restrict__ slice_w, const int32_t* __restrict__ cols,
-                 const double* __restrict__ vals, const double* __restrict__ dinv, const double* __restrict__ b,
+amgm_sell_kernel(int32_t n, int32_t nslices, const u32* __restrict__ slice_w, A a0, const double* __restrict__ dinv, const double* __restrict__ b,
                  const double* __restrict__ x, double omega, double* __restrict__ y, double* __restrict__ part, int K,
                  int nparts) {
     __shared__ double red[33];
+    const A a = a0.staged();
     const int lane = threadIdx.x & 31;
     const int64_t warp = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     const int64_t nwarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
@@ -74,8 +74,8 @@ amgm_sell_kernel(int32_t n, int32_t nslices, const u32* __restrict__ slice_w, co
         double acc[MK];
 #pragma unroll
         for (int k = 0; k < MK; ++k) acc[k] = 0.0;
-        sell_row_dot_multi(cols, vals, (int64_t)w0 * 32 + lane, w, x, n, K, acc);
         const int64_t r = s * 32 + lane;
+        sell_row_dot_multi(a, (int64_t)w0 * 32 + lane, r, w, x, n, K, acc);
         if (r < n) {
             const double di = MODE == 2 ? dinv[r] : 0.0;
 #pragma unroll
@@ -225,8 +225,10 @@ template <int MODE>
 int sweep(const nodal_amg* h, const AmgLevel& V, int K, const double* b, const double* x, double* y, double* part,
           int nparts, cudaStream_t st) {
     const nodal_sell* m = V.sell;
-    amgm_sell_kernel<MODE><<<amg_sell_grid(h->ctx, m->nslices), AT, 0, st>>>(
-        m->n, m->nslices, m->slice_w, m->cols, m->vals, m->dinv, b, x, h->omega, y, part, K, nparts);
+    sell_launch(m, [&](auto a) {
+        amgm_sell_kernel<MODE><<<amg_sell_grid(h->ctx, m->nslices), AT, 0, st>>>(
+            m->n, m->nslices, m->slice_w, a, m->dinv, b, x, h->omega, y, part, K, nparts);
+    });
     KERNEL_CHECK();
     return NODAL_OK;
 }

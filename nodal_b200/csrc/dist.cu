@@ -666,10 +666,10 @@ dist_vector_push_kernel(PcgDev* __restrict__ dev, int32_t n, double* __restrict_
 
 // SpMV of the fused iteration; the CTA that finishes last runs the all-reduce through the
 // peers' mailboxes (fixed reduction order: the result does not depend on which CTA is last).
+template <class A>
 __global__ void __launch_bounds__(PCG_THREADS, 5)
 dist_spmv_allreduce_sell_kernel(PcgDev* __restrict__ dev, int32_t n, int32_t nslices,
-                                const u32* __restrict__ slice_w, const int32_t* __restrict__ cols,
-                                const double* __restrict__ vals, const double* __restrict__ u,
+                                const u32* __restrict__ slice_w, A a0, const double* __restrict__ u,
                                 double* __restrict__ w, double* part_d, const double* __restrict__ part_g,
                                 const double* __restrict__ part_rr, int cnt_v, DistSync* sy,
                                 unsigned long long* seq, int R, int me,
@@ -687,6 +687,7 @@ dist_spmv_allreduce_sell_kernel(PcgDev* __restrict__ dev, int32_t n, int32_t nsl
         sy->dbg[9] = now;
     }
     // (the halo part of u is complete: dist_vector_push_kernel does not finish before it is)
+    const A a = a0.staged();
     const int lane = threadIdx.x & 31;
     const int64_t warp = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     const int64_t nwarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
@@ -695,8 +696,8 @@ dist_spmv_allreduce_sell_kernel(PcgDev* __restrict__ dev, int32_t n, int32_t nsl
         const u32 w0 = slice_w[s];
         const int wd = (int)(slice_w[s + 1] - w0);
         const int64_t base = (int64_t)w0 * 32 + lane;
-        const double acc = sell_row_dot(cols, vals, base, wd, u);
         const int64_t row = s * 32 + lane;
+        const double acc = sell_row_dot(a, base, row, wd, u);
         if (row < n) {
             w[row] = acc;
             dot = fma(acc, __ldg(&u[row]), dot);
@@ -1193,9 +1194,11 @@ extern "C" int nodal_dist_pcg(nodal_ctx* ctx, nodal_dist* d, int32_t n_global, c
                         send_idx, send_off_dev, dest_off_dev, need_cnt_dev, blist_dev, nb_rows, nbc, push_rng_dev,
                         bmask_dev, d->pcg.peer_dev);
                 KERNEL_CHECK();
-                dist_spmv_allreduce_sell_kernel<<<A.g1, PCG_THREADS, 0, sx>>>(
-                    dev, nloc, sell->nslices, sell->slice_w, sell->cols, sell->vals, ext, w, part_d, part_g,
-                    part_rr, g2, sy, d->pcg.seq, R, me, d->pcg.peer_dev, nxt);
+                sell_launch(sell, [&](auto a) {
+                    dist_spmv_allreduce_sell_kernel<<<A.g1, PCG_THREADS, 0, sx>>>(
+                        dev, nloc, sell->nslices, sell->slice_w, a, ext, w, part_d, part_g, part_rr, g2, sy,
+                        d->pcg.seq, R, me, d->pcg.peer_dev, nxt);
+                });
                 KERNEL_CHECK();
                 return NODAL_OK;
             }

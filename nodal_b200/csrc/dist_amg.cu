@@ -264,11 +264,12 @@ acg_vector_kernel(PcgDev* __restrict__ dev, int32_t n, double* __restrict__ cur,
 }
 
 // w = A u (SELL-32, one warp per slice) + partial sums of r.u and w.u
+template <class A>
 __global__ void __launch_bounds__(DA, 5)
-acg_spmv_dots_kernel(int32_t n, int32_t nslices, const u32* __restrict__ slice_w, const int32_t* __restrict__ cols,
-                     const double* __restrict__ vals, const double* __restrict__ u, const double* __restrict__ r,
+acg_spmv_dots_kernel(int32_t n, int32_t nslices, const u32* __restrict__ slice_w, A a0, const double* __restrict__ u, const double* __restrict__ r,
                      double* __restrict__ w, double* __restrict__ part_g, double* __restrict__ part_d) {
     __shared__ double sm[40];
+    const A a = a0.staged();
     const int lane = threadIdx.x & 31;
     const int64_t warp = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     const int64_t nwarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
@@ -276,8 +277,8 @@ acg_spmv_dots_kernel(int32_t n, int32_t nslices, const u32* __restrict__ slice_w
     for (int64_t s = warp; s < nslices; s += nwarps) {
         const u32 w0 = slice_w[s];
         const int wd = (int)(slice_w[s + 1] - w0);
-        const double acc = sell_row_dot(cols, vals, (int64_t)w0 * 32 + lane, wd, u);
         const int64_t row = s * 32 + lane;
+        const double acc = sell_row_dot(a, (int64_t)w0 * 32 + lane, row, wd, u);
         if (row < n) {
             const double uv = __ldg(&u[row]);
             w[row] = acc;
@@ -834,8 +835,10 @@ int gather_operator(Solver& S, const AmgCsr& A, const std::vector<int32_t>& boun
 template <int MODE>
 int sweep(Solver& S, const DLevel& L, const double* b, const double* x, double* y, cudaStream_t sx) {
     const nodal_sell* m = L.sell;
-    amg_sell_kernel<MODE><<<amg_sell_grid(S.ctx, m->nslices), AT, 0, sx>>>(
-        m->n, m->nslices, m->slice_w, m->cols, m->vals, m->dinv, b, x, S.omega, y, nullptr);
+    sell_launch(m, [&](auto a) {
+        amg_sell_kernel<MODE><<<amg_sell_grid(S.ctx, m->nslices), AT, 0, sx>>>(
+            m->n, m->nslices, m->slice_w, a, m->dinv, b, x, S.omega, y, nullptr);
+    });
     KERNEL_CHECK();
     return NODAL_OK;
 }
@@ -846,8 +849,10 @@ int sweep(Solver& S, const DLevel& L, const double* b, const double* x, double* 
 template <int MODE>
 int cycle_sweep(Solver& S, const DLevel& L, const double* b, const double* xc, double* y, cudaStream_t sx) {
     const nodal_sell* m = L.sell;
-    amg_cycle_sweep_kernel<MODE><<<amg_sell_grid(S.ctx, m->nslices), AT, 0, sx>>>(
-        m->n, m->nslices, m->slice_w, m->cols, m->vals, m->dinv, b, S.omega, L.agg, xc, S.scale, y);
+    sell_launch(m, [&](auto a) {
+        amg_cycle_sweep_kernel<MODE><<<amg_sell_grid(S.ctx, m->nslices), AT, 0, sx>>>(
+            m->n, m->nslices, m->slice_w, a, m->dinv, b, S.omega, L.agg, xc, S.scale, y);
+    });
     KERNEL_CHECK();
     return NODAL_OK;
 }
@@ -1109,8 +1114,9 @@ extern "C" int nodal_dist_amg_pcg(nodal_ctx* ctx, nodal_dist* d, int32_t n_globa
             KERNEL_CHECK();
             NODAL_TRY(cycle(S, nullptr, r, u, st));
             NODAL_TRY(exchange(S, nullptr, 2 * ND, F.halo, u_off, st));
-            acg_spmv_dots_kernel<<<gs, DA, 0, st>>>(n, F.sell->nslices, F.sell->slice_w, F.sell->cols, F.sell->vals, u, r, w,
-                                                    part_g, part_d);
+            sell_launch(F.sell, [&](auto a) {
+                acg_spmv_dots_kernel<<<gs, DA, 0, st>>>(n, F.sell->nslices, F.sell->slice_w, a, u, r, w, part_g, part_d);
+            });
             KERNEL_CHECK();
             NODAL_TRY(allreduce(0, part_g, gs, part_d, gs, part_rr, gv, part_bb, gv, SC, 0, st));
             acg_scalars_kernel<<<1, 32, 0, st>>>(dev, SC, rtol, maxit, first);
@@ -1124,8 +1130,9 @@ extern "C" int nodal_dist_amg_pcg(nodal_ctx* ctx, nodal_dist* d, int32_t n_globa
             KERNEL_CHECK();
             NODAL_TRY(cycle(S, dev, r, u, sx));
             NODAL_TRY(exchange(S, dev, 2 * ND, F.halo, u_off, sx));
-            acg_spmv_dots_kernel<<<gs, DA, 0, sx>>>(n, F.sell->nslices, F.sell->slice_w, F.sell->cols, F.sell->vals, u, r, w,
-                                                    part_g, part_d);
+            sell_launch(F.sell, [&](auto a) {
+                acg_spmv_dots_kernel<<<gs, DA, 0, sx>>>(n, F.sell->nslices, F.sell->slice_w, a, u, r, w, part_g, part_d);
+            });
             KERNEL_CHECK();
             NODAL_TRY(allreduce(1, part_g, gs, part_d, gs, part_rr, gv, nullptr, 0, nxt, 1, sx));
             return NODAL_OK;

@@ -21,14 +21,14 @@ __device__ __forceinline__ bool block_done(const int* done) {
 }
 
 // ---------------------------------------------------------------- K1
-template <int MINB>
+template <int MINB, class A>
 static __global__ void __launch_bounds__(PCG_THREADS, MINB)
 pcg_spmv_dot_sell_kernel(const PcgDev* __restrict__ dev, int32_t n, int32_t nslices,
-                         const u32* __restrict__ slice_w, const int32_t* __restrict__ cols,
-                         const double* __restrict__ vals, const double* __restrict__ p,
+                         const u32* __restrict__ slice_w, A a0, const double* __restrict__ p,
                          double* __restrict__ q, double* __restrict__ part_pq) {
     __shared__ double sm[40];
     if (block_done(&dev->done)) return;
+    const A a = a0.staged();
     const int lane = threadIdx.x & 31;
     const int64_t warp = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     const int64_t nwarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
@@ -37,8 +37,8 @@ pcg_spmv_dot_sell_kernel(const PcgDev* __restrict__ dev, int32_t n, int32_t nsli
         const u32 w0 = slice_w[s];
         const int w = (int)(slice_w[s + 1] - w0);
         const int64_t base = (int64_t)w0 * 32 + lane;
-        const double acc = sell_row_dot(cols, vals, base, w, p);
         const int64_t r = s * 32 + lane;
+        const double acc = sell_row_dot(a, base, r, w, p);
         if (r < n) {
             q[r] = acc;
             dot = fma(acc, __ldg(&p[r]), dot);
@@ -313,13 +313,14 @@ static inline int launch_k1(const Mat& A, const PcgDev* dev, const double* p, do
     if (A.sell) {
 #define GOS(M)                                                                                 \
     pcg_spmv_dot_sell_kernel<M><<<A.g1, PCG_THREADS, 0, st>>>(dev, A.n, A.sell->nslices,       \
-                                                              A.sell->slice_w, A.sell->cols,   \
-                                                              A.sell->vals, p, q, part_pq)
-        switch (A.minb) {
-            case 5: GOS(5); break;
-            case 6: GOS(6); break;
-            default: GOS(4); break;
-        }
+                                                              A.sell->slice_w, a, p, q, part_pq)
+        sell_launch(A.sell, [&](auto a) {
+            switch (A.minb) {
+                case 5: GOS(5); break;
+                case 6: GOS(6); break;
+                default: GOS(4); break;
+            }
+        });
 #undef GOS
     } else {
 #define GO(T)                                                                                  \
