@@ -65,28 +65,6 @@ int amg_aggregate(nodal_ctx* ctx, int rounds, const AmgCsr& A, int32_t nown, int
     return NODAL_OK;
 }
 
-int amg_transpose_pattern(nodal_ctx* ctx, int32_t n, const int32_t* agg, int32_t** pt_ptr_out,
-                          int32_t** pt_idx_out, cudaStream_t st) {
-    AmgScratch<u64> keys(ctx, n);
-    AmgScratch<double> vals(ctx, n), rhs(ctx, (size_t)n + 1), ones(ctx, n);
-    if (!keys.ptr || !vals.ptr || !rhs.ptr || !ones.ptr) return NODAL_CUDA_ERROR;
-    const int cb = amg_bit_length(n);
-    amg_pt_keys_kernel<<<amg_rows_grid(ctx, n), AT, 0, st>>>(n, agg, cb, keys, vals);
-    KERNEL_CHECK();
-    int64_t cnt = 0;
-    NODAL_TRY(nodal_csr_build(ctx, n, n, cb, reinterpret_cast<uint64_t*>(keys.ptr), vals, rhs, &cnt, st));
-    if (cnt != n) {
-        nodal_set_error("amg: internal error, P^T has %lld entries for %d rows", (long long)cnt, n);
-        return NODAL_CUDA_ERROR;
-    }
-    AmgScratch<int32_t> pp(ctx, (size_t)n + 1), pi(ctx, n);
-    if (!pp.ptr || !pi.ptr) return NODAL_CUDA_ERROR;
-    NODAL_TRY(nodal_csr_fetch(ctx, n, n, pp, pi, ones, st));
-    *pt_ptr_out = pp.keep();
-    *pt_idx_out = pi.keep();
-    return NODAL_OK;
-}
-
 int amg_members(nodal_ctx* ctx, int32_t n, const int32_t* agg, int32_t nc, int32_t** pt_ptr_out,
                 int32_t** pt_idx_out, cudaStream_t st) {
     AmgScratch<u32> cnt(ctx, (size_t)nc + 1), cursor(ctx, (size_t)nc + 1);
@@ -164,14 +142,9 @@ int aggregate(nodal_amg* h, const Csr& A, int32_t** agg_out, int32_t* nc_out, cu
 }
 
 // Ac = P^T A P for the piecewise-constant P of `agg`.
-bool sorted_galerkin() {
-    static const bool on = getenv("NODAL_AMG_SORT_GALERKIN") != nullptr;
-    return on;
-}
-
 int galerkin(nodal_amg* h, const Csr& A, const int32_t* agg, int32_t nc, Csr* out, cudaStream_t st) {
     nodal_ctx* ctx = h->ctx;
-    if (!sorted_galerkin() && amg_merge_pays(A.nnz, nc)) {
+    if (amg_merge_pays(A.nnz, nc)) {
         // sort-free: members of every aggregate, then one thread merges the member rows of its
         // coarse row (same summation order as the sort-based product below: bit-identical)
         int32_t *pp = nullptr, *pi = nullptr;
@@ -202,11 +175,6 @@ int galerkin(nodal_amg* h, const Csr& A, const int32_t* agg, int32_t nc, Csr* ou
     out->data = dv.keep();
     out->owned = true;
     return NODAL_OK;
-}
-
-int transpose_pattern(nodal_amg* h, AmgLevel& L, cudaStream_t st) {
-    if (!sorted_galerkin()) return amg_members(h->ctx, L.n, L.agg, L.nc, &L.pt_ptr, &L.pt_idx, st);
-    return amg_transpose_pattern(h->ctx, L.n, L.agg, &L.pt_ptr, &L.pt_idx, st);
 }
 
 int invert_coarsest(nodal_amg* h, const AmgLevel& L, cudaStream_t st) {
@@ -293,9 +261,9 @@ int build_hierarchy(nodal_amg* h, int32_t n, int64_t nnz, const int32_t* indptr,
         L.owned = cur.owned;
         L.agg = comp;
         L.nc = A.n;
+        rc = amg_members(ctx, L.n, L.agg, L.nc, &L.pt_ptr, &L.pt_idx, st);
         h->lv.push_back(L);
         cur = A;
-        rc = transpose_pattern(h, h->lv.back(), st);
         if (rc != NODAL_OK) {
             free_csr(ctx, cur);
             return rc;

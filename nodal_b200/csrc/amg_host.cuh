@@ -87,12 +87,8 @@ void amg_free_csr(nodal_ctx* ctx, AmgCsr& a);
 // (amg_core.cuh); the single-GPU setup passes nown = INT32_MAX, base = 0.
 int amg_aggregate(nodal_ctx* ctx, int rounds, const AmgCsr& A, int32_t nown, int32_t base,
                   int32_t** agg_out, int32_t* nc_out, cudaStream_t st);
-// Members of every aggregate (CSR pattern of P^T), rows in increasing order; pool buffers
-// pt_ptr[n + 1] / pt_idx[n] owned by the caller.
-int amg_transpose_pattern(nodal_ctx* ctx, int32_t n, const int32_t* agg, int32_t** pt_ptr,
-                          int32_t** pt_idx, cudaStream_t st);
-
-// The same without a sort (count / scan / place / per-aggregate ordering): nc aggregates.
+// Members of the nc aggregates (CSR pattern of P^T), rows in increasing order, by count / scan /
+// place / per-aggregate ordering; pool buffers pt_ptr[nc + 1] / pt_idx[n] owned by the caller.
 int amg_members(nodal_ctx* ctx, int32_t n, const int32_t* agg, int32_t nc, int32_t** pt_ptr, int32_t** pt_idx,
                 cudaStream_t st);
 // Rows [0, nc) of P^T A P by merging the member rows of every coarse row (amg_merge_core.cuh):

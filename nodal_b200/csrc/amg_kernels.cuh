@@ -65,15 +65,6 @@ amg_relabel_kernel(int32_t n, const int32_t* __restrict__ indptr, const int32_t*
     }
 }
 
-static __global__ void __launch_bounds__(AT)
-amg_pt_keys_kernel(int32_t n, const int32_t* __restrict__ agg, int cb, u64* __restrict__ keys,
-                   double* __restrict__ vals) {
-    ROW_LOOP(i, n) {
-        keys[i] = ((u64)agg[i] << cb) | (u64)i;
-        vals[i] = 1.0;
-    }
-}
-
 // ------------------------------------------------------------------ coarsest level: explicit inverse
 // [A | I] -> [I | A^-1] by Gauss-Jordan without pivoting (A is symmetric positive definite),
 // one launch per pivot, ping-pong between two n x 2n buffers so a step has no read/write race.

@@ -820,6 +820,10 @@ int peer_heap_ensure(nodal_ctx* ctx, nodal_dist* d, PeerHeap* hp, size_t bytes, 
     return NODAL_OK;
 }
 
+// CTAs per SM of the vector kernels (measured best); it also sizes the push ranges of the fused
+// vector pass, so both grids use it.
+constexpr int DIST_G2_PER_SM = 8;
+
 extern "C" int nodal_dist_pcg(nodal_ctx* ctx, nodal_dist* d, int32_t n_global, const int32_t* bounds_h,
                               int64_t nnz, const int32_t* indptr, const int32_t* indices,
                               const double* data, const double* rhs_local, double* x_local,
@@ -1017,8 +1021,7 @@ extern "C" int nodal_dist_pcg(nodal_ctx* ctx, nodal_dist* d, int32_t n_global, c
             if (!blist_dev || !bmask_dev) return NODAL_CUDA_ERROR;
             CUDA_TRY(cudaMemsetAsync(bmask_dev, 0, (size_t)nloc + 16, st));
             // CTA c of the vector pass owns blist[c*chunk, (c+1)*chunk); which send entries are those?
-            const int g2_per_sm_ = getenv("NODAL_DIST_G2") ? atoi(getenv("NODAL_DIST_G2")) : 8;
-            const int g2_ = (int)std::min<int64_t>((int64_t)ctx->num_sms * g2_per_sm_,
+            const int g2_ = (int)std::min<int64_t>((int64_t)ctx->num_sms * DIST_G2_PER_SM,
                                                    std::max<int64_t>(1, ((nloc >> 1) + PCG_THREADS - 1) / PCG_THREADS));
             nbc = std::max(1, std::min(g2_, (nb_rows + PCG_THREADS - 1) / PCG_THREADS));
             const int chunk = (nb_rows + nbc - 1) / nbc;
@@ -1068,7 +1071,7 @@ extern "C" int nodal_dist_pcg(nodal_ctx* ctx, nodal_dist* d, int32_t n_global, c
         sc = static_cast<double*>(dmalloc(sizeof(double) * ((size_t)nloc + nhalo + 2) + 256));
         if (!sc) return NODAL_CUDA_ERROR;
         bool unit = false;
-        if (getenv("NODAL_PCG_NO_SCALE") == nullptr) {
+        {
             int* flag = reinterpret_cast<int*>(sc + (size_t)nloc + nhalo + 2);
             CUDA_TRY(cudaMemsetAsync(flag, 0, sizeof(int), st));
             pcg_scale_factors_kernel<<<grid_of(ctx, nloc), PCG_THREADS, 0, st>>>(nloc, indptr, lcols, data, sc, flag);
@@ -1100,18 +1103,16 @@ extern "C" int nodal_dist_pcg(nodal_ctx* ctx, nodal_dist* d, int32_t n_global, c
         }
         if (use_sell) A.sell = sell;
         else unit = false;      // too irregular for SELL-32 (padding > 1.5x): CSR kernels on the unscaled operator
-        const int g2_per_sm = getenv("NODAL_DIST_G2") ? atoi(getenv("NODAL_DIST_G2")) : 8;
-        const int g2 = (int)std::min<int64_t>((int64_t)ctx->num_sms * g2_per_sm,
+        const int g2 = (int)std::min<int64_t>((int64_t)ctx->num_sms * DIST_G2_PER_SM,
                                               std::max<int64_t>(1, ((nloc >> 1) + PCG_THREADS - 1) / PCG_THREADS));
         if (A.sell) {
             const int64_t want = ((int64_t)sell->nslices * 32 + PCG_THREADS - 1) / PCG_THREADS;
-            const int per_sm = getenv("NODAL_SPMV_CTAS_PER_SM") ? atoi(getenv("NODAL_SPMV_CTAS_PER_SM")) : 5;
-            A.g1 = (int)std::min<int64_t>((int64_t)ctx->num_sms * per_sm, want);
+            A.g1 = (int)std::min<int64_t>((int64_t)ctx->num_sms * PCG_SELL_CTAS_PER_SM, want);
         } else {
             const int64_t want = ((int64_t)nloc * A.tpr + PCG_THREADS - 1) / PCG_THREADS;
             A.g1 = (int)std::min<int64_t>((int64_t)ctx->num_sms * 8, want);
         }
-        const bool fused = p2p && A.sell && getenv("NODAL_DIST_NO_FUSE") == nullptr;
+        const bool fused = p2p && A.sell;
         const int gmax = std::max(A.g1, g2) + 1;
         const size_t vloc = align_up(sizeof(double) * (size_t)nloc, 256);
         const size_t vext = align_up(sizeof(double) * (size_t)(nloc + nhalo + 2), 256);
@@ -1234,12 +1235,10 @@ extern "C" int nodal_dist_pcg(nodal_ctx* ctx, nodal_dist* d, int32_t n_global, c
 
         NODAL_TRY(start(1));
         const int CH = 32;
-        const bool use_graph = getenv("NODAL_DIST_NO_GRAPH") == nullptr;
-        if (use_graph) {
+        {
             const auto c0 = std::chrono::steady_clock::now();
             const unsigned long long before = g_nodal_launches;
             CUDA_TRY(cudaStreamCreateWithFlags(&cap, cudaStreamNonBlocking));
-            if (A.sell) NODAL_TRY(sell_set_l2_window(ctx, A.sell, cap));
             CUDA_TRY(cudaStreamBeginCapture(cap, cudaStreamCaptureModeThreadLocal));
             int crc = NODAL_OK;
             for (int i = 0; i < CH && crc == NODAL_OK; ++i) crc = iteration(i & 1, cap);
@@ -1258,12 +1257,8 @@ extern "C" int nodal_dist_pcg(nodal_ctx* ctx, nodal_dist* d, int32_t n_global, c
             const int64_t max_chunks = (int64_t)maxit / CH + 3;
             int64_t k = 0;
             for (;; ++k) {
-                if (use_graph) {
-                    CUDA_TRY(cudaGraphLaunch(gexec, st));
-                    g_nodal_launches += launches_per_chunk;
-                } else {
-                    for (int i = 0; i < CH; ++i) NODAL_TRY(iteration(i & 1, st));
-                }
+                CUDA_TRY(cudaGraphLaunch(gexec, st));
+                g_nodal_launches += launches_per_chunk;
                 CUDA_TRY(cudaMemcpyAsync(&poll[k & 1], dev, sizeof(PcgDev), cudaMemcpyDeviceToHost, st));
                 CUDA_TRY(cudaEventRecord(ev_poll[k & 1], st));
                 if (k >= 1) {
@@ -1366,7 +1361,7 @@ extern "C" int nodal_dist_pcg(nodal_ctx* ctx, nodal_dist* d, int32_t n_global, c
     const auto h1 = std::chrono::steady_clock::now();
     if (gexec) cudaGraphExecDestroy(gexec);
     if (graph) cudaGraphDestroy(graph);
-    if (cap) { sell_clear_l2_window(cap); cudaStreamDestroy(cap); }
+    if (cap) cudaStreamDestroy(cap);
     const auto h2 = std::chrono::steady_clock::now();
     if (sell) sell_free(sell);
     for (void* p : owned) ctx_pool_free(ctx, p);

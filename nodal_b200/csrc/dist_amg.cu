@@ -440,7 +440,6 @@ struct Solver {
     int32_t gmax = 0;
     double omega = 0.8, scale = 1.8, max_fill = 1.2, max_complexity = 4.0;
     double nnz_k_fine = 0.0, nnz_k_total = 0.0;      // entries (in units of 1024) of level 0 / of all levels so far
-    bool sorted_galerkin = getenv("NODAL_AMG_SORT_GALERKIN") != nullptr;   // round-2 first version: sort-based products
     int passes = 2, rounds = 8, maxlevels = 30;
     int64_t gather_below = 400000;
     double params_rep[8] = {0};
@@ -687,7 +686,7 @@ int coarsen(Solver& S, DLevel& L, AmgCsr* next, std::vector<int32_t>* next_bound
             amg_compose_kernel<<<amg_rows_grid(ctx, nloc), AT, 0, st>>>(nloc, comp, agg);
             KERNEL_CHECK();
         }
-        if (pass + 1 < S.passes && !S.sorted_galerkin && amg_merge_pays(cur.nnz, nc)) {
+        if (pass + 1 < S.passes && amg_merge_pays(cur.nnz, nc)) {
             // operator the next pass aggregates: the local-local block of P^T A P (couplings to
             // other ranks are invisible to the matching, see amg_core.cuh), merged per coarse row
             int32_t *pp = nullptr, *pi = nullptr;
@@ -740,7 +739,7 @@ int coarsen(Solver& S, DLevel& L, AmgCsr* next, std::vector<int32_t>* next_bound
     KERNEL_CHECK();
     NODAL_TRY(exchange_nccl(S, L.halo, lab, st));
     bool have_members = false;
-    if (!S.sorted_galerkin && amg_merge_pays(nnz, ncur)) {
+    if (amg_merge_pays(nnz, ncur)) {
         // members of the composed aggregates (also the restriction pattern), then one thread merges
         // the member rows of its coarse row with the global coarse column ids
         AmgScratch<int32_t> lab32(ctx, (size_t)L.halo.ext_len + 2);
@@ -780,7 +779,7 @@ int coarsen(Solver& S, DLevel& L, AmgCsr* next, std::vector<int32_t>* next_bound
     S.owned.push_back(comp);
     L.nc = ncur;
     if (!have_members) {
-        NODAL_TRY(amg_transpose_pattern(ctx, nloc, comp, &L.pt_ptr, &L.pt_idx, st));
+        NODAL_TRY(amg_members(ctx, nloc, comp, ncur, &L.pt_ptr, &L.pt_idx, st));
         S.owned.push_back(L.pt_ptr);
         S.owned.push_back(L.pt_idx);
     }
@@ -1141,8 +1140,7 @@ extern "C" int nodal_dist_amg_pcg(nodal_ctx* ctx, nodal_dist* d, int32_t n_globa
         const int start_rc = start(1);
         nvtxRangePop();
         NODAL_TRY(start_rc);
-        const bool use_graph = getenv("NODAL_DIST_NO_GRAPH") == nullptr;
-        if (use_graph) {
+        {
             const unsigned long long before = g_nodal_launches;
             CUDA_TRY(cudaStreamCreateWithFlags(&cap, cudaStreamNonBlocking));
             for (int par = 0; par < 2; ++par) {
@@ -1166,12 +1164,8 @@ extern "C" int nodal_dist_amg_pcg(nodal_ctx* ctx, nodal_dist* d, int32_t n_globa
             int64_t k = 0;
             const int64_t max_iters = (int64_t)maxit + 4;
             for (;; ++k) {
-                if (use_graph) {
-                    CUDA_TRY(cudaGraphLaunch(gexec[par], st));
-                    g_nodal_launches += launches_per_iter;
-                } else {
-                    NODAL_TRY(iteration(par, st));
-                }
+                CUDA_TRY(cudaGraphLaunch(gexec[par], st));
+                g_nodal_launches += launches_per_iter;
                 par ^= 1;
                 CUDA_TRY(cudaMemcpyAsync(&poll[k & 1], dev, sizeof(PcgDev), cudaMemcpyDeviceToHost, st));
                 CUDA_TRY(cudaEventRecord(ev_poll[k & 1], st));

@@ -200,7 +200,7 @@ extern "C" int nodal_lu_batched(nodal_ctx* ctx, int64_t batch, int32_t ncomp, co
     }
     if (batch == 0 || n == 0) return NODAL_OK;
     CUDA_TRY(cudaSetDevice(ctx->device));
-    if (n <= 8 && getenv("NODAL_LU_BATCHED_GENERIC") == nullptr)
+    if (n <= 8)
         return launch_reg<false>(ctx, batch, ncomp, type, a, b, c, d, drv, branch, kcl, n, values, x, info,
                                  (cudaStream_t)stream);
     const size_t per_thread = sizeof(double) * (size_t)n * (n + 1);

@@ -254,9 +254,9 @@ __device__ __forceinline__ void dmma_8x8x4(double& c0, double& c1, double a, dou
 }
 
 // C[M x N] -= Amat[M x K] * Bmat[K x N], all row-major with leading dimension ld.
-// 8 warps as 4 (M) x 2 (N); warp tile 32 x (8 TN).  TN = 8: 128 x 128 CTA tile, 1 CTA/SM;
-// TN = 4: 128 x 64 tile, 64 accumulator registers, 2 CTAs/SM (one CTA's barrier / cp.async wait
-// overlaps the other's DMMA).  VEC2: ld and all offsets even -> 16-byte cp.async.
+// 8 warps as 4 (M) x 2 (N); warp tile 32 x (8 TN).  TN = 4: 128 x 64 tile, 64 accumulator
+// registers, 2 CTAs/SM (one CTA's barrier / cp.async wait overlaps the other's DMMA).
+// VEC2: ld and all offsets even -> 16-byte cp.async.
 template <int TN, bool VEC2>
 __global__ void __launch_bounds__(GM_THREADS, GemmCfg<TN>::MINB)
 lu_gemm_kernel(double* __restrict__ C, const double* __restrict__ Amat, const double* __restrict__ Bmat,
@@ -466,24 +466,13 @@ static int lu_factor_core(nodal_ctx* ctx, int n, double* G, int* ipiv, int32_t* 
         CUDA_TRY(cudaFuncSetAttribute(lu_trsm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)trsm_smem));
     }
 
-    // Right-looking LU.  Opt-in (NODAL_LU_LOOKAHEAD=1): one panel of look-ahead -- as soon as step k
-    // has updated the NEXT panel's columns, panel k+1 is launched on a second (high-priority)
-    // stream while the main stream applies step k to the remaining columns.  Measured on B200
-    // (round 2): no gain, 261 vs 252 ms at n = 16 384 -- the cooperative panel grid (one CTA per SM,
-    // ~117 KB of shared memory each) does not become co-resident next to the DMMA update's two
-    // 108 KB CTAs per SM, so the two kernels still run back to back and the split update only adds
-    // launches.  Kept off by default; the schedule is here for a panel that needs fewer SMs.
-    const bool lookahead = getenv("NODAL_LU_LOOKAHEAD") != nullptr && n > 2 * LU_NB;
-    cudaStream_t sp = st;
-    cudaEvent_t ev_panel = nullptr, ev_ready = nullptr;
-    if (lookahead) {
-        int lo = 0, hi = 0;
-        CUDA_TRY(cudaDeviceGetStreamPriorityRange(&lo, &hi));
-        CUDA_TRY(cudaStreamCreateWithPriority(&sp, cudaStreamNonBlocking, hi));
-        CUDA_TRY(cudaEventCreateWithFlags(&ev_panel, cudaEventDisableTiming));
-        CUDA_TRY(cudaEventCreateWithFlags(&ev_ready, cudaEventDisableTiming));
-    }
-    auto launch_panel = [&](int k, cudaStream_t s) -> int {
+    // Right-looking LU: after panel k, the row interchanges left of it, the update of the columns
+    // right of it, then panel k+1.  One panel of look-ahead (panel k+1 on a second, high-priority
+    // stream while the rest of step k runs) was measured on B200 (round 2) and removed: no gain,
+    // 261 vs 252 ms at n = 16 384 -- the cooperative panel grid (one CTA per SM, ~117 KB of shared
+    // memory each) does not become co-resident next to the DMMA update's two 108 KB CTAs per SM, so
+    // the two kernels still ran back to back and the split update only added launches.
+    auto launch_panel = [&](int k) -> int {
         int jb = std::min(LU_NB, n - k);
         int m = n - k;
         int rows_per_cta = std::max(32, (m + sms - 1) / sms);
@@ -493,7 +482,7 @@ static int lu_factor_core(nodal_ctx* ctx, int n, double* G, int* ipiv, int32_t* 
         int n_ = n, k_ = k;
         void* args[] = {&Aptr, &n_, &k_, &jb, &rows_per_cta, &ipiv, &cand, &candrow, &diagrow, &info};
         CUDA_TRY(cudaLaunchCooperativeKernel((void*)lu_panel_kernel, dim3(ncta), dim3(PANEL_THREADS), args,
-                                             panel_smem, s));
+                                             panel_smem, st));
         ++g_nodal_launches;
         return NODAL_OK;
     };
@@ -512,51 +501,19 @@ static int lu_factor_core(nodal_ctx* ctx, int n, double* G, int* ipiv, int32_t* 
         const double* Bp = G + (size_t)k * n + c0;
         // all offsets are even when n is even (k, jb, c0 are multiples of 2): 16-byte copies
         const bool vec2 = (n % 2 == 0) && (((uintptr_t)G & 15) == 0) && (jb % 2 == 0) && (c0 % 2 == 0);
-        const int tn = getenv("NODAL_LU_GEMM_TN") ? atoi(getenv("NODAL_LU_GEMM_TN")) : 4;
-        if (tn == 8) {
-            if (vec2) NODAL_TRY((launch_gemm<8, true>(Cp, Ap, Bp, rest, c1 - c0, jb, n, st)));
-            else NODAL_TRY((launch_gemm<8, false>(Cp, Ap, Bp, rest, c1 - c0, jb, n, st)));
-        } else {
-            if (vec2) NODAL_TRY((launch_gemm<4, true>(Cp, Ap, Bp, rest, c1 - c0, jb, n, st)));
-            else NODAL_TRY((launch_gemm<4, false>(Cp, Ap, Bp, rest, c1 - c0, jb, n, st)));
-        }
+        if (vec2) NODAL_TRY((launch_gemm<4, true>(Cp, Ap, Bp, rest, c1 - c0, jb, n, st)));
+        else NODAL_TRY((launch_gemm<4, false>(Cp, Ap, Bp, rest, c1 - c0, jb, n, st)));
         return NODAL_OK;
     };
-    auto factor = [&]() -> int {
-        NODAL_TRY(launch_panel(0, st));
-        for (int k = 0; k < n; k += LU_NB) {
-            const int jb = std::min(LU_NB, n - k);
-            const int right = k + jb;                       // first column right of the panel
-            if (lookahead && k > 0) CUDA_TRY(cudaStreamWaitEvent(st, ev_panel, 0));   // panel k (on sp) is done
-            if (right >= n) {
-                NODAL_TRY(update_cols(k, jb, 0, k, false));
-                break;
-            }
-            const int next_jb = std::min(LU_NB, n - right);
-            if (lookahead) {
-                NODAL_TRY(update_cols(k, jb, right, right + next_jb, true));          // the next panel's columns first
-                CUDA_TRY(cudaEventRecord(ev_ready, st));
-                CUDA_TRY(cudaStreamWaitEvent(sp, ev_ready, 0));
-                NODAL_TRY(launch_panel(right, sp));                                   // overlaps the wide update below
-                CUDA_TRY(cudaEventRecord(ev_panel, sp));
-                NODAL_TRY(update_cols(k, jb, 0, k, false));
-                NODAL_TRY(update_cols(k, jb, right + next_jb, n, true));
-            } else {
-                NODAL_TRY(update_cols(k, jb, 0, k, false));
-                NODAL_TRY(update_cols(k, jb, right, n, true));
-                NODAL_TRY(launch_panel(right, st));
-            }
-        }
-        return NODAL_OK;
-    };
-    const int frc = factor();
-    if (lookahead) {
-        cudaStreamSynchronize(sp);
-        cudaStreamDestroy(sp);
-        cudaEventDestroy(ev_panel);
-        cudaEventDestroy(ev_ready);
+    NODAL_TRY(launch_panel(0));
+    for (int k = 0; k < n; k += LU_NB) {
+        const int jb = std::min(LU_NB, n - k);
+        const int right = k + jb;                       // first column right of the panel
+        NODAL_TRY(update_cols(k, jb, 0, k, false));
+        if (right >= n) break;
+        NODAL_TRY(update_cols(k, jb, right, n, true));
+        NODAL_TRY(launch_panel(right));
     }
-    NODAL_TRY(frc);
     int* info_pinned = reinterpret_cast<int*>(ctx->pinned);
     CUDA_TRY(cudaMemcpyAsync(info_pinned, info, sizeof(int), cudaMemcpyDeviceToHost, st));
     CUDA_TRY(cudaStreamSynchronize(st));

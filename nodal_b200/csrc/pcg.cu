@@ -19,6 +19,8 @@
 
 #include "pcg_kernels.cuh"
 
+constexpr int PCG_G2_PER_SM = 5;   // CTAs per SM of the vector kernels (measured best)
+
 // ---------------------------------------------------------------- driver
 
 extern "C" int nodal_pcg(nodal_ctx* ctx, int32_t n, int64_t nnz, const int32_t* indptr,
@@ -62,8 +64,7 @@ extern "C" int nodal_pcg(nodal_ctx* ctx, int32_t n, int64_t nnz, const int32_t* 
         A.n = n; A.nnz = nnz; A.indptr = indptr; A.indices = indices; A.data = data;
         const double mean = (double)nnz / n;
         A.tpr = mean <= 2.5 ? 2 : mean <= 6.0 ? 4 : mean <= 12.0 ? 8 : mean <= 24.0 ? 16 : 32;
-        const int g2_per_sm = getenv("NODAL_PCG_G2") ? atoi(getenv("NODAL_PCG_G2")) : 5;   // CTAs per SM of the vector kernels (measured best)
-        const int g2 = (int)std::min<int64_t>((int64_t)ctx->num_sms * g2_per_sm,
+        const int g2 = (int)std::min<int64_t>((int64_t)ctx->num_sms * PCG_G2_PER_SM,
                                               std::max<int64_t>(1, ((n >> 1) + PCG_THREADS - 1) / PCG_THREADS));
         // symmetric diagonal scaling (only with the private SELL copy, only for positive diagonals)
         bool scaled = false;
@@ -83,15 +84,10 @@ extern "C" int nodal_pcg(nodal_ctx* ctx, int32_t n, int64_t nnz, const int32_t* 
             NODAL_TRY(sell_from_csr(ctx, n, nnz, indptr, indices, data, &sell, st, scaled ? sc : nullptr));
             if ((double)sell->padded <= 1.5 * (double)nnz + 1024.0) A.sell = sell;
             else scaled = false;
-            if (!scaled && sell && sc && A.sell) {   // values were scaled but the padding rule vetoed: rebuild
-                /* unreachable: scaled is only cleared here when A.sell is not used */
-            }
         }
         if (A.sell) {
             const int64_t want = ((int64_t)sell->nslices * 32 + PCG_THREADS - 1) / PCG_THREADS;
-            A.minb = getenv("NODAL_SPMV_MINB") ? atoi(getenv("NODAL_SPMV_MINB")) : 5;   // measured: 5 CTAs/SM (46 regs) -> 0.98 of the copy peak
-            if (A.minb < 4 || A.minb > 6) A.minb = 4;
-            A.g1 = (int)std::min<int64_t>((int64_t)ctx->num_sms * A.minb, want);
+            A.g1 = (int)std::min<int64_t>((int64_t)ctx->num_sms * PCG_SELL_CTAS_PER_SM, want);
         } else {
             const int64_t want = ((int64_t)n * A.tpr + PCG_THREADS - 1) / PCG_THREADS;
             A.g1 = (int)std::min<int64_t>((int64_t)ctx->num_sms * 8, want);
@@ -186,7 +182,6 @@ extern "C" int nodal_pcg(nodal_ctx* ctx, int32_t n, int64_t nnz, const int32_t* 
         if (use_graph) {
             const unsigned long long before = g_nodal_launches;
             CUDA_TRY(cudaStreamCreateWithFlags(&cap, cudaStreamNonBlocking));
-            if (A.sell) NODAL_TRY(sell_set_l2_window(ctx, A.sell, cap));
             CUDA_TRY(cudaStreamBeginCapture(cap, cudaStreamCaptureModeThreadLocal));
             int crc = NODAL_OK;
             for (int i = 0; i < PCG_CHUNK && crc == NODAL_OK; ++i) crc = iteration(i & 1, cap);
@@ -326,7 +321,7 @@ extern "C" int nodal_pcg(nodal_ctx* ctx, int32_t n, int64_t nnz, const int32_t* 
     rc = run();
     if (gexec) cudaGraphExecDestroy(gexec);
     if (graph) cudaGraphDestroy(graph);
-    if (cap) { sell_clear_l2_window(cap); cudaStreamDestroy(cap); }
+    if (cap) cudaStreamDestroy(cap);
     for (auto& e : prof_ev) cudaEventDestroy(e);
     if (sell) { cudaStreamSynchronize(st); sell_free(sell); }
     if (sc) ctx_pool_free(ctx, sc);

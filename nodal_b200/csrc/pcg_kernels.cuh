@@ -21,8 +21,12 @@ __device__ __forceinline__ bool block_done(const int* done) {
 }
 
 // ---------------------------------------------------------------- K1
-template <int MINB, class A>
-static __global__ void __launch_bounds__(PCG_THREADS, MINB)
+// resident CTAs per SM the SELL kernel is compiled and launched for
+// (measured: 5 CTAs/SM (46 regs) -> 0.98 of the copy peak)
+constexpr int PCG_SELL_CTAS_PER_SM = 5;
+
+template <class A>
+static __global__ void __launch_bounds__(PCG_THREADS, PCG_SELL_CTAS_PER_SM)
 pcg_spmv_dot_sell_kernel(const PcgDev* __restrict__ dev, int32_t n, int32_t nslices,
                          const u32* __restrict__ slice_w, A a0, const double* __restrict__ p,
                          double* __restrict__ q, double* __restrict__ part_pq) {
@@ -305,23 +309,15 @@ struct Mat {
     const double* data = nullptr;
     int tpr = 4;
     int g1 = 1;
-    int minb = 5;      // resident CTAs per SM the SELL kernel is compiled for
 };
 
 static inline int launch_k1(const Mat& A, const PcgDev* dev, const double* p, double* q, double* part_pq,
               cudaStream_t st) {
     if (A.sell) {
-#define GOS(M)                                                                                 \
-    pcg_spmv_dot_sell_kernel<M><<<A.g1, PCG_THREADS, 0, st>>>(dev, A.n, A.sell->nslices,       \
-                                                              A.sell->slice_w, a, p, q, part_pq)
         sell_launch(A.sell, [&](auto a) {
-            switch (A.minb) {
-                case 5: GOS(5); break;
-                case 6: GOS(6); break;
-                default: GOS(4); break;
-            }
+            pcg_spmv_dot_sell_kernel<<<A.g1, PCG_THREADS, 0, st>>>(dev, A.n, A.sell->nslices, A.sell->slice_w, a,
+                                                                   p, q, part_pq);
         });
-#undef GOS
     } else {
 #define GO(T)                                                                                  \
     pcg_spmv_dot_csr_kernel<T><<<A.g1, PCG_THREADS, 0, st>>>(dev, A.n, A.indptr, A.indices,    \

@@ -2,14 +2,14 @@
 // pairs, hand written for the CSR build (no CUB / Thrust).
 //
 // Radix sort: 8-bit digits, one pass per digit over only the key bits in use.
-// Per pass:
-//   1. digit_histogram_kernel  per-tile digit counts -> hist[digit][tile] (digit-major)
-//   2. scan_exclusive_u32      global exclusive scan of that table = first output slot of
-//                              every (digit, tile) bucket
-//   3. scatter_kernel          re-reads the tile, ranks keys stably inside the tile
-//                              (warp match-any multi-split, warps own consecutive key
-//                              ranges), reorders the tile by digit in shared memory and
-//                              writes every digit run to its bucket with coalesced stores.
+//   1. onesweep_hist_kernel   digit histograms of all passes from one read of the keys
+//   2. onesweep_bases_kernel  exclusive scan of each pass's histogram = first output slot of
+//                             every digit
+//   3. onesweep_pass_kernel   one kernel per pass: ranks the keys of a tile stably (warp
+//                             match-any multi-split, warps own consecutive key ranges), finds
+//                             the tile's output offsets by decoupled look-back, reorders the
+//                             tile by digit in shared memory and writes every digit run to its
+//                             place with coalesced stores.
 // Stability: inside a tile, warp w owns keys [w*32*IPT, (w+1)*32*IPT) and visits them in
 // rounds of 32 consecutive keys, so (warp, round, lane) order == input order.
 #include <algorithm>
@@ -130,122 +130,15 @@ int scan_exclusive_u32(nodal_ctx* ctx, const u32* in, u32* out, int64_t count, u
 
 // ------------------------------------------------------------------ radix sort
 constexpr int RS_THREADS = 256;
-constexpr int RS_WARPS = RS_THREADS / 32;
-constexpr int RS_IPT = 16;                     // rounds per warp
-constexpr int RS_TILE = RS_THREADS * RS_IPT;   // 4096 keys per tile
 constexpr int RS_BINS = 256;
-
-__global__ void __launch_bounds__(RS_THREADS)
-digit_histogram_kernel(const u64* __restrict__ keys, int64_t count, int shift, int64_t tiles,
-                       u32* __restrict__ hist /* [RS_BINS][tiles] */) {
-    __shared__ u32 h[RS_BINS];
-    for (int64_t tile = blockIdx.x; tile < tiles; tile += gridDim.x) {
-        h[threadIdx.x] = 0;
-        __syncthreads();
-        const int64_t base = tile * RS_TILE;
-#pragma unroll
-        for (int k = 0; k < RS_IPT; ++k) {
-            const int64_t i = base + (int64_t)k * RS_THREADS + threadIdx.x;
-            if (i < count) atomicAdd(&h[(u32)(keys[i] >> shift) & 0xffu], 1u);
-        }
-        __syncthreads();
-        hist[(int64_t)threadIdx.x * tiles + tile] = h[threadIdx.x];
-        __syncthreads();
-    }
-}
-
-__global__ void __launch_bounds__(RS_THREADS)
-scatter_kernel(const u64* __restrict__ keys_in, const u64* __restrict__ vals_in,
-               u64* __restrict__ keys_out, u64* __restrict__ vals_out, int64_t count, int shift,
-               int64_t tiles, const u32* __restrict__ bucket /* scanned [RS_BINS][tiles] */) {
-    __shared__ u32 warp_cnt[RS_WARPS][RS_BINS];  // per-warp digit counts -> exclusive offsets
-    __shared__ u32 digit_start[RS_BINS];         // start of each digit run inside the tile
-    __shared__ u32 digit_gbase[RS_BINS];         // global slot of the run's first element
-    __shared__ u32 scan_sm[40];
-    __shared__ u64 stage[RS_TILE];               // tile reordered by digit
-    __shared__ uint8_t stage_dg[RS_TILE];        // digit of every reordered slot
-    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
-    const u32 lt = lanemask_lt();
-
-    for (int64_t tile = blockIdx.x; tile < tiles; tile += gridDim.x) {
-        const int64_t base = tile * RS_TILE + (int64_t)w * 32 * RS_IPT;
-        for (int i = threadIdx.x; i < RS_WARPS * RS_BINS; i += RS_THREADS)
-            (&warp_cnt[0][0])[i] = 0;
-        __syncthreads();
-
-        u64 key[RS_IPT];
-        u32 rank[RS_IPT];  // rank of the key among equal digits seen earlier by this warp
-#pragma unroll
-        for (int k = 0; k < RS_IPT; ++k) {
-            const int64_t i = base + k * 32 + lane;
-            const bool live = i < count;
-            key[k] = live ? keys_in[i] : 0ull;
-            const u32 dg = live ? ((u32)(key[k] >> shift) & 0xffu) : 256u;
-            const u32 peers = __match_any_sync(0xffffffffu, dg);
-            const u32 before = live ? warp_cnt[w][dg] : 0u;
-            __syncwarp();
-            rank[k] = before + __popc(peers & lt);
-            if (live && (peers & lt) == 0u) warp_cnt[w][dg] = before + __popc(peers);
-            __syncwarp();
-        }
-        __syncthreads();
-        // per digit: exclusive prefix over warps, tile-level digit totals
-        {
-            const int dgt = threadIdx.x;  // RS_THREADS == RS_BINS
-            u32 run = 0;
-#pragma unroll
-            for (int ww = 0; ww < RS_WARPS; ++ww) {
-                const u32 t = warp_cnt[ww][dgt];
-                warp_cnt[ww][dgt] = run;
-                run += t;
-            }
-            u32 total;
-            const u32 start = block_excl_scan_u32(run, scan_sm, &total);
-            digit_start[dgt] = start;
-            digit_gbase[dgt] = bucket[(int64_t)dgt * tiles + tile];
-        }
-        __syncthreads();
-        const int64_t tile_base = tile * RS_TILE;
-        const int tile_n = (count - tile_base < RS_TILE) ? (int)(count - tile_base) : RS_TILE;
-        u32 pos[RS_IPT];
-#pragma unroll
-        for (int k = 0; k < RS_IPT; ++k) {
-            const int64_t i = base + k * 32 + lane;
-            if (i < count) {
-                const u32 dg = (u32)(key[k] >> shift) & 0xffu;
-                pos[k] = digit_start[dg] + warp_cnt[w][dg] + rank[k];
-                stage[pos[k]] = key[k];
-                stage_dg[pos[k]] = (uint8_t)dg;
-            }
-        }
-        __syncthreads();
-        for (int j = threadIdx.x; j < tile_n; j += RS_THREADS) {
-            const u32 dg = stage_dg[j];
-            keys_out[(int64_t)digit_gbase[dg] + (j - digit_start[dg])] = stage[j];
-        }
-        __syncthreads();
-        // payload: same permutation, staged through the same buffer
-#pragma unroll
-        for (int k = 0; k < RS_IPT; ++k) {
-            const int64_t i = base + k * 32 + lane;
-            if (i < count) stage[pos[k]] = vals_in[i];
-        }
-        __syncthreads();
-        for (int j = threadIdx.x; j < tile_n; j += RS_THREADS) {
-            const u32 dg = stage_dg[j];
-            vals_out[(int64_t)digit_gbase[dg] + (j - digit_start[dg])] = stage[j];
-        }
-        __syncthreads();
-    }
-}
 
 // ------------------------------------------------------------------ single-pass-per-digit sort
 // ("onesweep" class).  One upfront kernel builds the digit histograms of ALL passes from one read
 // of the keys; every pass is then ONE kernel that reads keys + payload once, finds each tile's
 // output offsets by decoupled look-back over per-tile digit counts (no global scan, no second
 // read), reorders the tile by digit in shared memory -- keys and payload staged together -- and
-// writes every digit run to its final place.  Stability is the legacy kernel's: inside a tile
-// (warp, round, lane) order is input order, tiles are ordered by the look-back.
+// writes every digit run to its final place.  Stability: inside a tile (warp, round, lane) order
+// is input order, tiles are ordered by the look-back.
 // Tile ids are handed out by an atomic ticket, so a tile's predecessors have always started and
 // the look-back cannot dead-lock; its spin is bounded anyway (error flag instead of a hang).
 constexpr int OS_MAXPASS = 8;
@@ -438,15 +331,10 @@ int radix_sort_check(nodal_ctx* ctx) {
     return NODAL_OK;
 }
 
-static bool use_legacy_sort() {
-    static const bool legacy = getenv("NODAL_SORT_LEGACY") != nullptr;
-    return legacy;
-}
-
 size_t radix_sort_scratch_bytes(int64_t count) {
-    const int64_t tiles = (count + OS_TILE - 1) / OS_TILE;     // OS_TILE <= RS_TILE: covers both paths
-    const size_t hist = align_up((size_t)tiles * RS_BINS * sizeof(u32), 256) + 256;
-    return hist + scan_scratch_bytes(tiles * RS_BINS) + align_up(OS_MAXPASS * RS_BINS * sizeof(u32), 256) + 1024;
+    const int64_t tiles = (count + OS_TILE - 1) / OS_TILE;
+    const size_t desc = align_up(((size_t)tiles * RS_BINS + 64) * sizeof(u32), 256);
+    return desc + align_up(OS_MAXPASS * RS_BINS * sizeof(u32), 256) + 1024;
 }
 
 // Sorts by key bits [0, bits).  Ping-pongs between (keys, vals) and (keys_alt, vals_alt);
@@ -456,34 +344,18 @@ int radix_sort_pairs(nodal_ctx* ctx, u64* keys, u64* vals, u64* keys_alt, u64* v
     NvtxRange nvtx_range("radix_sort_pairs");
     *result_in_alt = false;
     if (count <= 1 || bits <= 0) return NODAL_OK;
-    int64_t tiles = (count + RS_TILE - 1) / RS_TILE;
+    const int64_t tiles = (count + OS_TILE - 1) / OS_TILE;
     if (tiles * RS_BINS * 2 >= (int64_t)1 << 32 || count >= (int64_t)1 << 30) {
         nodal_set_error("radix_sort_pairs: too many elements");
         return NODAL_BAD_ARG;
     }
     const int passes = (bits + 7) / 8;
-    u64 *src_k = keys, *src_v = vals, *dst_k = keys_alt, *dst_v = vals_alt;
-    if (use_legacy_sort() || passes > OS_MAXPASS) {
-        u32* hist = carve<u32>(ctx, (size_t)tiles * RS_BINS);
-        if (!hist) return NODAL_CUDA_ERROR;
-        const size_t mark = ctx->arena_used;
-        const int grid = (int)std::min<int64_t>(tiles, (int64_t)ctx->num_sms * 16);
-        for (int p = 0; p < passes; ++p) {
-            const int shift = p * 8;
-            digit_histogram_kernel<<<grid, RS_THREADS, 0, st>>>(src_k, count, shift, tiles, hist);
-            KERNEL_CHECK();
-            ctx->arena_used = mark;  // scan scratch is reused by every pass
-            NODAL_TRY(scan_exclusive_u32(ctx, hist, hist, tiles * RS_BINS, nullptr, st));
-            scatter_kernel<<<grid, RS_THREADS, 0, st>>>(src_k, src_v, dst_k, dst_v, count, shift, tiles, hist);
-            KERNEL_CHECK();
-            u64* t = src_k; src_k = dst_k; dst_k = t;
-            t = src_v; src_v = dst_v; dst_v = t;
-            *result_in_alt = !*result_in_alt;
-        }
-        return NODAL_OK;
+    if (passes > OS_MAXPASS) {
+        nodal_set_error("radix_sort_pairs: keys wider than 64 bits");
+        return NODAL_BAD_ARG;
     }
+    u64 *src_k = keys, *src_v = vals, *dst_k = keys_alt, *dst_v = vals_alt;
     // tile descriptors + ticket + error word (zeroed before every pass), digit bases of all passes
-    tiles = (count + OS_TILE - 1) / OS_TILE;
     const size_t desc_words = (size_t)tiles * RS_BINS + 64;
     u32* desc = carve<u32>(ctx, desc_words);
     u32* ghist = carve<u32>(ctx, OS_MAXPASS * RS_BINS);

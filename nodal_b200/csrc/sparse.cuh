@@ -37,8 +37,6 @@ int sell_from_csr(nodal_ctx* ctx, int32_t n, int64_t nnz, const int32_t* indptr,
                   const int32_t* indices, const double* data, nodal_sell** out, cudaStream_t st,
                   const double* sc = nullptr);   // sc: optional row/column scale factors (S A S)
 void sell_free(nodal_sell* m);
-int sell_set_l2_window(nodal_ctx* ctx, const nodal_sell* m, cudaStream_t st);   // see spmv.cu
-void sell_clear_l2_window(cudaStream_t st);
 
 // y = A x on the generic CSR path
 int csr_spmv_launch(nodal_ctx* ctx, int32_t n, int64_t nnz, const int32_t* indptr,

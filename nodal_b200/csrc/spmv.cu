@@ -367,41 +367,3 @@ extern "C" int nodal_sell_spmv(nodal_ctx* ctx, const nodal_sell* m, const double
     KERNEL_CHECK();
     return NODAL_OK;
 }
-
-// ---------------------------------------------------------------- L2 residency
-// Every CG iteration streams the whole operator once.  When the operator is not much larger
-// than the 126 MB L2 (a rank of the multi-GPU path holds 1/R of it) plain LRU gets ~0 hits
-// out of a cyclic sweep; pinning a fraction of it as "persisting" keeps that fraction
-// resident from one iteration to the next.  Applied to the stream the iteration graph is
-// captured on, so every kernel node inherits the window.
-// MEASURED (r1, B200): a loss.  With the window the vector-update kernels that share the
-// graph slow down by 1.5-1.8x (2 x 2.1 M rows/rank: 25.8 -> 47.7 us; 1 GPU, 16.7 M rows:
-// 432 -> 674 us per iteration) while the SpMV gains 3 %; the set-aside takes L2 away from
-// the write-back traffic of the streaming kernels.  Kept opt-in (NODAL_L2_WINDOW=1) only.
-int sell_set_l2_window(nodal_ctx* ctx, const nodal_sell* m, cudaStream_t st) {
-    if (!m || !m->store || !getenv("NODAL_L2_WINDOW")) return NODAL_OK;
-    cudaDeviceProp prop;
-    CUDA_TRY(cudaGetDeviceProperties(&prop, ctx->device));
-    if (prop.persistingL2CacheMaxSize <= 0 || prop.accessPolicyMaxWindowSize <= 0) return NODAL_OK;
-    const size_t persist = (size_t)prop.persistingL2CacheMaxSize;
-    CUDA_TRY(cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, persist));
-    cudaStreamAttrValue attr;
-    memset(&attr, 0, sizeof(attr));
-    const size_t window = std::min<size_t>(m->store_bytes, (size_t)prop.accessPolicyMaxWindowSize);
-    attr.accessPolicyWindow.base_ptr = m->store;
-    attr.accessPolicyWindow.num_bytes = window;
-    attr.accessPolicyWindow.hitRatio = (float)std::min(1.0, 0.85 * (double)persist / (double)window);
-    attr.accessPolicyWindow.hitProp = cudaAccessPropertyPersisting;
-    attr.accessPolicyWindow.missProp = cudaAccessPropertyStreaming;
-    CUDA_TRY(cudaStreamSetAttribute(st, cudaStreamAttributeAccessPolicyWindow, &attr));
-    return NODAL_OK;
-}
-
-void sell_clear_l2_window(cudaStream_t st) {
-    if (!getenv("NODAL_L2_WINDOW")) return;
-    cudaStreamAttrValue attr;
-    memset(&attr, 0, sizeof(attr));
-    attr.accessPolicyWindow.num_bytes = 0;
-    cudaStreamSetAttribute(st, cudaStreamAttributeAccessPolicyWindow, &attr);
-    cudaCtxResetPersistingL2Cache();
-}

@@ -175,13 +175,16 @@ def test_many_port_equivalent_resistances(device, mode):
 
 # ------------------------------------------------------------------ row-partitioned form, one rank
 @pytest.mark.parametrize("N,amg", [(100, {}), (100, {"gather_below": 400}), (100, {"gather_below": 3000, "passes": 1}),
-                                   (400, {"gather_below": 5000}), (1000, {"gather_below": 20000})])
+                                   (400, {"gather_below": 5000}), (1000, {"gather_below": 20000}),
+                                   ("random", {"gather_below": 2000})])
 def test_dist_amg_single_rank(device, N, amg):
     """csrc/dist_amg.cu with a world of one rank (empty halos, no exchange) must reproduce the
-    single-GPU hierarchy: same level sizes where the levels are built the same way, same answer."""
+    single-GPU hierarchy: same level sizes where the levels are built the same way, same answer.
+    The random network's distributed levels are too dense for the member-row merge (amg_merge_pays
+    is false): their products go through the sort-based builder."""
     import copy
     from nodal_b200 import dist as ndist
-    net = copy.deepcopy(gen.grid2d(N))
+    net = copy.deepcopy(gen.random_network(20000, degree=8, seed=1) if N == "random" else gen.grid2d(N))
     net.process_component(["a1", "A", "1", "1", "g"])
     table = net.table()
     csr, rhs = device.assemble_csr(table)
@@ -201,8 +204,11 @@ def test_dist_amg_single_rank(device, N, amg):
     common = min(len(info["level_rows"]), len(i1["level_rows"]))
     assert info["level_rows"][:common] == i1["level_rows"][:common], (info, i1)
     assert abs(info["iterations"] - i1["iterations"]) <= 4
-    want = {100: GRIDS["grid2d_100"]["R_sparse"], 400: 0.7732566450916762, 1000: 0.7732422803670024}[N]
-    assert float(x[net.nodenum["1"]]) == pytest.approx(want, rel=1e-9)
+    if N == "random":       # no pinned value: the single-GPU solve is the reference
+        assert float((x - x1).abs().max()) <= 1e-9 * float(x1.abs().max())
+    else:
+        want = {100: GRIDS["grid2d_100"]["R_sparse"], 400: 0.7732566450916762, 1000: 0.7732422803670024}[N]
+        assert float(x[net.nodenum["1"]]) == pytest.approx(want, rel=1e-9)
     resid = device.spmv(csr, x) - rhs
     assert float(resid.norm() / rhs.norm()) <= 1.05e-10
     assert float((x - x1).abs().max()) <= 1e-8 * float(x1.abs().max())
